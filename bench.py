@@ -2,7 +2,7 @@
 """Headline benchmark: Kalman-filter trajectory-steps/sec on B200 (BASELINE.json metric), one JSON line.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dtype f64|f32]
-                    [--traj-per-gpu M | --traj-total M]
+                    [--traj-per-gpu M | --traj-total M] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload (config.workload): the Monte-Carlo noise sweep of BASELINE.json configs[2]/[3] - trajectories x 1,000 steps over
@@ -122,6 +122,24 @@ def algorithmic_bytes(n_local, T, S, esz):
     return (58 * T * S + (22 + 52) * n_local) * esz
 
 
+DUMP_MEMBERS = 1 << 16  # --dump-outputs: 52 summary rows x 65,536 members x 8 B = 27 MB, under the 64 MB a dump may take
+
+
+def dump_members(n: int) -> np.ndarray:
+    """Member ids whose outputs --dump-outputs writes: all of them up to DUMP_MEMBERS, else a sorted sample drawn from a fixed
+    seed, so that every run of the same shape writes the same members."""
+    if n <= DUMP_MEMBERS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_MEMBERS, replace=False))
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    os.makedirs(path, exist_ok=True)
+    for name, arr in arrays.items():
+        assert arr.dtype in (np.float32, np.float64), (name, arr.dtype)
+        np.save(os.path.join(path, name + ".npy"), arr)
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -144,7 +162,13 @@ def parse():
     ap.add_argument("--e2e-trace", action="store_true", help="add the per-batch event timeline of the host pipeline (rank 0) to the e2e object")
     ap.add_argument("--gather", default="fused", choices=["fused", "nccl"],
                     help="N > 1: all-gather of the summaries fused into the filter kernel (NVLink peer stores) or NCCL after it")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy (a fixed sample of "
+                         f"at most {DUMP_MEMBERS} members), so that two builds can be compared output for output on identical inputs")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 def job_shape(a, world, rank):
@@ -366,7 +390,8 @@ def run_reference(a):
     st = make_streams(range(S), a.T)
     n = threads * 16
     q, r = mc_noise(0, n, S)
-    fn = lambda: c_oracle.run(st, n, Q=q, R=r, n_threads=threads, want=("x_final",))  # noqa: E731
+    last = {}
+    fn = lambda: last.update(c_oracle.run(st, n, Q=q, R=r, n_threads=threads, want=("x_final",)))  # noqa: E731
     t0 = time.perf_counter()
     fn()
     first = time.perf_counter() - t0
@@ -379,6 +404,9 @@ def run_reference(a):
     for _ in range(a.steps):
         fn()
     dt = time.perf_counter() - t0
+    if a.dump_outputs:
+        m = dump_members(n)
+        dump_outputs(a.dump_outputs, {"x_final": last["x_final"][:, m], "members": m.astype(np.float64)})
     value = n * a.T * a.steps / dt
     sample = f"{n} trajectories x {a.T} steps per step over {S} base streams, Monte-Carlo Q/R"
     cpu = {"value": value, "unit": UNIT, "cores": threads, "kind": "port", "sample": sample}
@@ -506,6 +534,14 @@ def run_native(a):
     value = steps_total / (ms * 1e-3)
     status_bad = int((out["status"] != 0).sum().item())
     gathered = (peer.tensor if peer is not None else step_nccl()) if world > 1 else out["summary"]
+    if rank == 0 and a.dump_outputs:
+        # the gathered summary columns of a sample of the whole job's members; status words are per rank, so only those of
+        # rank 0's own members (ids 0 .. n_local - 1) among them
+        m = dump_members(n_total)
+        mine = m[m < n_local]
+        dump_outputs(a.dump_outputs, {"summary": gathered[:, torch.from_numpy(m).to(dev)].cpu().numpy(), "members": m.astype(np.float64),
+                                      "status": out["status"][torch.from_numpy(mine).to(dev)].cpu().numpy().astype(np.float64),
+                                      "status_members": mine.astype(np.float64)})
 
     # ---- parity of what was just timed: members of the timed batch against the C oracle (rank 0, outside the timed region).
     # First / last member, a nominal member, both sides of every shard boundary, and a few in between.

@@ -113,6 +113,14 @@ def test_parity_sample_with_ten_and_twelve_members_reads_the_noise_per_trajector
         assert bench.parity_sample(st, q, r, idx, sm)["max_rel_x"] == 0.0
 
 
+def test_dump_sample_is_fixed_and_fits_the_dump_budget():
+    assert np.array_equal(bench.dump_members(100), np.arange(100))
+    m = bench.dump_members(1 << 20)
+    assert m.size == bench.DUMP_MEMBERS and np.array_equal(m, bench.dump_members(1 << 20))
+    assert (np.diff(m) > 0).all() and 0 <= m[0] and m[-1] < 1 << 20
+    assert (52 + 3) * 8 * m.size <= 64 << 20  # FP64 summary columns + member ids + status words and their member ids
+
+
 def test_clock_sampler_survives_a_box_without_gpu_or_nvml():
     with bench.ClockSampler(0, period=0.01) as c:
         pass
@@ -120,9 +128,19 @@ def test_clock_sampler_survives_a_box_without_gpu_or_nvml():
     assert set(s) >= {"sm_mhz", "sm_max_mhz", "reasons", "samples", "how"}
 
 
-def test_bench_reference_arm_line():
-    d = _bench("--impl", "reference", "--steps", "1", "--warmup", "1", "--T", "50")
+def test_bench_reference_arm_line(tmp_path):
+    d = _bench("--impl", "reference", "--steps", "1", "--warmup", "1", "--T", "50", "--dump-outputs", str(tmp_path))
     assert d["impl"] == "reference" and d["value"] > 0 and d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["value"] == d["value"]
+    # --dump-outputs: the final states of the last timed step, as the C oracle computes them for the same members and noise
+    x, members = np.load(tmp_path / "x_final.npy"), np.load(tmp_path / "members.npy")
+    assert sorted(os.listdir(tmp_path)) == ["members.npy", "x_final.npy"] and x.dtype == np.float64 and x.shape == (12, members.size)
+    from oracle import c_oracle
+    from optistate_b200.synth import make_streams
+
+    n = int(members.max()) + 1
+    q, r = bench.mc_noise(0, n, 64)
+    want = c_oracle.run(make_streams(range(64), 50), n, Q=q, R=r, want=("x_final",))["x_final"]
+    assert np.array_equal(x, want[:, members.astype(np.int64)])
     if os.path.isfile(os.path.join(ROOT, "oracle", "_ref", "kalman_filter", "kalman_filter.py")) or os.path.isdir("/root/reference"):
         assert d["cpu_baseline"]["reference_class_steps_per_s_1core"] > 100  # the unmodified reference class, timed on this box

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 pytestmark = pytest.mark.gpu
@@ -47,3 +48,32 @@ def test_bench_strong_scaling_mode_and_full_covariance_structure():
                "--no-e2e", "--structure", "full")
     assert d["scaling"] == "strong" and d["config"]["trajectories_total"] == 4096 and d["parity_sample"]["ok"]
     assert "78" in d["config"]["covariance_structure"]
+
+
+def test_bench_dump_outputs_are_the_oracles_and_the_same_in_every_run(tmp_path):
+    """--dump-outputs writes the summaries and status words the timed path returned in its last step: the dumped columns are
+    those the C oracle computes for the listed members, and two runs with the same arguments dump identical arrays."""
+    import bench
+    from oracle import c_oracle
+    from optistate_b200.synth import make_streams
+
+    args = ("--steps", "2", "--warmup", "1", "--traj-per-gpu", "4096", "--T", "50", "--streams", "64", "--no-cpu-baseline", "--no-secondary", "--no-e2e")
+    for run in ("a", "b"):
+        d = _bench(*args, "--dump-outputs", str(tmp_path / run))
+        assert d["steps"] == 2 and d["parity_sample"]["ok"]
+    names = ("members", "status", "status_members", "summary")
+    a, b = ({k: np.load(tmp_path / run / f"{k}.npy") for k in names} for run in ("a", "b"))
+    assert sorted(os.listdir(tmp_path / "a")) == [k + ".npy" for k in names]
+    assert a["summary"].shape == (52, 4096) and a["summary"].dtype == np.float64
+    assert np.array_equal(a["members"], np.arange(4096)) and np.array_equal(a["status_members"], a["members"]) and not a["status"].any()
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k
+    # columns of members other than those bench.py's parity sample picks, against the oracle on the same streams and noise
+    st = make_streams(range(64), 50)
+    pick = np.array([1, 2, 63, 64, 65, 1000, 2047, 3001, 4094])
+    qs = np.concatenate([bench.mc_noise(int(m), 1, 64)[0] for m in pick], axis=1)
+    rs = np.concatenate([bench.mc_noise(int(m), 1, 64)[1] for m in pick], axis=1)
+    nominal = c_oracle.run(st, want=("x_steps",))["x_steps"]
+    cols = a["summary"][:, np.searchsorted(a["members"], pick)]
+    e = bench.parity_sample(st, qs, rs, (pick % 64).astype(np.int32), cols, nominal)
+    assert max(v for k, v in e.items() if k.startswith("max_rel_") and k != "max_rel_dev") < 1e-9 and e["max_rel_dev"] < 1e-7, e
