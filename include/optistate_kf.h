@@ -39,7 +39,7 @@
 extern "C" {
 #endif
 
-#define OPTISTATE_KF_ABI_VERSION 4
+#define OPTISTATE_KF_ABI_VERSION 5
 
 #define OPTI_KF_NX 12 /* states  [thx thy thz | x y z | wx wy wz | vx vy vz]   kalman_filter.py:9  */
 #define OPTI_KF_NZ 10 /* measurements [th_imu(3) z_odom w_imu(3) v_odom(3)]    kalman_filter.py:11 */
@@ -259,18 +259,17 @@ typedef struct OptiKfMpcDesc {
     const void *p;                 /* [12][N] body-frame feet, held over the horizon (kalman_filter.py:141-142)       */
     const void *contact;           /* [4][N] 0 / 1 flags stored as dtype, held over the horizon (kalman_filter.py:145-146) */
     void *forces;                  /* [5][12][N] optimal forces; stage 0 is what predict_mpc applies (kalman_filter.py:161) */
-    uint32_t *status;              /* [N] optional: OPTI_KF_MPC_ST_* | interior-point iterations << 8                  */
+    uint32_t *status;              /* [N] required: OPTI_KF_MPC_ST_* | iterations << 8; the dual active set also marks in it
+                                      the problems it hands to the interior point                                       */
     /* Optional warm start for closed loops (estimate_state_mpc solves a near-identical QP every step), in / out, both or
-     * neither: the active set (one word per stage: bit 5 leg + row, bits 24..27 legs out of swing, bit 31 valid; zeroed
-     * memory = no warm start) and the multipliers of its rows.  A set that verifies (primal and dual feasibility of the
-     * equality-constrained solve, the same test that ends the cold path) skips the interior-point phase; one that does
-     * not, or a changed contact pattern, falls back to it.  (The shared-memory interior point for three and four legs out of
-     * swing ignores it.)                                                                                              */
+     * neither: the working set (one word per stage: bit 5 leg + row, bits 24..27 legs out of swing, bit 31 valid; zeroed
+     * memory = no warm start) and the multipliers of its rows.  The dual active set enters the stored set, drops the rows
+     * whose multipliers come out negative and continues from there; a changed contact pattern starts cold.  (The interior
+     * point ignores it.)                                                                                              */
     uint32_t *warm_set;            /* [5][N]                                                                           */
     void *warm_mult;               /* [5][4][5][N] doubles                                                              */
-    int32_t warm_rounds;           /* active-set correction rounds a warm start may take before the interior point runs
-                                      (0 = default)                                                                    */
-    int32_t solver;                /* 0 = dual active set, interior point for what it gives up on (default); 1 = interior point only */
+    int32_t solver;                /* 0 = dual active set, interior point for what it gives up on (default); 1 = the interior-point
+                                      kernel only                                                                      */
     int32_t max_changes;           /* dual active set: constraints entered + dropped before a problem is handed to the interior
                                       point (0 = default 400) - a time budget for real-time callers                     */
     int32_t reserved0;

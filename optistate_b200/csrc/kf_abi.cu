@@ -498,7 +498,7 @@ int optistate_kf_mpc_forces(const OptiKfMpcDesc *d, void *cuda_stream) {
     for (int k = 0; k < 12; ++k)
         if (!(d->w_state[k] >= 0)) return OPTI_KF_E_SHAPE;
     if (d->n_problems == 0) return OPTI_KF_OK;
-    if (!d->x || !d->body_ref || !d->p || !d->contact || !d->forces) return OPTI_KF_E_NULL;
+    if (!d->x || !d->body_ref || !d->p || !d->contact || !d->forces || !d->status) return OPTI_KF_E_NULL;
     if ((d->warm_set == nullptr) != (d->warm_mult == nullptr)) return OPTI_KF_E_NULL;
     okf::MpcParams p;
     std::memset(&p, 0, sizeof p);
@@ -507,7 +507,6 @@ int optistate_kf_mpc_forces(const OptiKfMpcDesc *d, void *cuda_stream) {
     p.x = (const double *)d->x; p.body_ref = (const double *)d->body_ref; p.p = (const double *)d->p;
     p.contact = (const double *)d->contact; p.forces = (double *)d->forces; p.status = d->status;
     p.warm_set = d->warm_set; p.warm_mult = (double *)d->warm_mult;
-    p.warm_rounds = d->warm_rounds > 0 ? d->warm_rounds : 0;
     if (d->solver != 0 && d->solver != 1) return OPTI_KF_E_SHAPE;
     p.solver = d->solver;
     p.max_changes = d->max_changes > 0 ? d->max_changes : 0;

@@ -1,6 +1,5 @@
 // Batched convex force MPC (kf_mpc.cuh): launch.
 #include "kf_mpc.cuh"
-#include "kf_mpc_rows.cuh"
 #include "kf_mpc_gi.cuh"
 
 #include "kf_launch.cuh"
@@ -8,30 +7,20 @@
 namespace okf {
 
 int launch_mpc(const MpcParams &p, cudaStream_t stream) {
-    if (p.max_legs <= MPCR_MAX_LEGS) {  // a trot or less: one warp per problem
-        // dual active set first (kf_mpc_gi.cuh); the interior point (kf_mpc_rows.cuh) solves what it flags, or everything when
-        // the caller asks for it or gives no status array to carry the flags.  Both take a warm start
-        const bool gi = p.solver == 0 && p.status != nullptr;
-        MpcParams q = p;
-        if (gi) {
+    // dual active set first (kf_mpc_gi.cuh): one warp per problem for a trot or less, two warps when the batch has three or four
+    // legs out of swing somewhere; then the shared-memory interior point (kf_mpc.cuh) for what it flags - or for everything when
+    // the caller asks for the interior point
+    MpcParams q = p;
+    if (p.solver == 0) {
+        if (p.max_legs <= MPCG_MAX_LEGS) {
             const size_t smem = mpcg_smem_bytes();
             if (cudaFuncSetAttribute(kf_mpc_gi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return OPTI_KF_E_CUDA;
             kf_mpc_gi_kernel<<<(unsigned)((p.N + MPCG_WARPS - 1) / MPCG_WARPS), 32 * MPCG_WARPS, smem, stream>>>(p);
-            q.only_flagged = 1;
+        } else {
+            const size_t smem2 = mpcg2_smem_bytes(p.max_legs);
+            if (cudaFuncSetAttribute(kf_mpc_gi2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2) != cudaSuccess) return OPTI_KF_E_CUDA;
+            kf_mpc_gi2_kernel<<<(unsigned)p.N, 64, smem2, stream>>>(p);
         }
-        const size_t smem = mpcr_smem_bytes();
-        if (cudaFuncSetAttribute(kf_mpc_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return OPTI_KF_E_CUDA;
-        const unsigned blocks = (unsigned)((p.N + MPCR_WARPS - 1) / MPCR_WARPS);
-        kf_mpc_rows_kernel<<<blocks, 32 * MPCR_WARPS, smem, stream>>>(q);
-        return OPTI_KF_OK;
-    }
-    // three or four legs out of swing somewhere in the batch: the dual active set with two warps per problem (kf_mpc_gi.cuh), then
-    // the round-1 shared-memory interior point (kf_mpc.cuh) for what it flags - or for everything on request / without a status array
-    MpcParams q = p;
-    if (p.solver == 0 && p.status != nullptr) {
-        const size_t smem2 = mpcg2_smem_bytes(p.max_legs);
-        if (cudaFuncSetAttribute(kf_mpc_gi2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2) != cudaSuccess) return OPTI_KF_E_CUDA;
-        kf_mpc_gi2_kernel<<<(unsigned)p.N, 64, smem2, stream>>>(p);
         q.only_flagged = 1;
     }
     const size_t smem = mpc_smem_bytes(p.max_legs);

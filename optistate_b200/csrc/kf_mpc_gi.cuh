@@ -1,6 +1,7 @@
-// Batched force MPC, dual active-set solver (Goldfarb & Idnani 1983) for problems with at most two legs out of swing - the
-// primary path of optistate_kf_mpc_forces for a trot.  Same QP and same minimiser as kf_mpc.cuh / kf_mpc_rows.cuh (the QP is
-// strictly convex: the minimiser is unique and the method terminates at it); what changes is the work per problem:
+// Batched force MPC, dual active-set solver (Goldfarb & Idnani 1983) - the primary path of optistate_kf_mpc_forces: one warp per
+// problem for at most two legs out of swing (a trot, kf_mpc_gi_kernel), two warps for three and four (kf_mpc_gi2_kernel).  Same
+// QP and same minimiser as the interior point of kf_mpc.cuh (the QP is strictly convex: the minimiser is unique and the method
+// terminates at it); what changes is the work per problem:
 //
 //   * the interior point refactorises the n x n normal equations every iteration (~13 factorisations + ~30 triangular solves
 //     per QP, each a chain of n dependent columns).  But H is FIXED per problem and every constraint row touches one leg of one
@@ -18,15 +19,259 @@
 //     step alone, exactly as in the paper.
 //   * the loop is rolled and compact (it fits the 32 KB instruction cache); only the inversion is straight-line code, run once.
 //   * a problem the method gives up on (iteration cap, working set full, a breakdown of S^-1) is flagged and solved by the
-//     interior-point kernel (kf_mpc_rows.cuh) in a second launch that only touches flagged problems.
+//     interior-point kernel (kf_mpc_kernel, kf_mpc.cuh) in a second launch that only touches flagged problems.
 // Measured against the independent active-set solve of the test infrastructure: see tests/test_mpc_gpu.py.
 #pragma once
 
 #include <type_traits>
 
-#include "kf_mpc_rows.cuh"
+#include "kf_mpc.cuh"
 
 namespace okf {
+
+constexpr int MPCG_MAX_LEGS = 2;  // legs out of swing the one-warp kernel is instantiated for
+
+__host__ __device__ constexpr int mpcg_even(int v) { return v + (v & 1); }
+
+// Reciprocal of a positive normal number, straight-line (20-bit seed + two Newton steps: rounding-limited): the IEEE division is a
+// call into a ~70-instruction slow-path routine, and the inversion of H takes one per pivot, every constraint change several more.
+__device__ __forceinline__ double rcp2_(double a) {
+    double r;
+    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(a));
+    double e = fma(-a, r, 1.0);
+    r = fma(r, e, r);
+    e = fma(-a, r, 1.0);
+    return fma(r, e, r);
+}
+
+// The threads that work on one problem: one warp, or - for the orders 45 and 60 of three and four legs out of swing in
+// kf_mpc_gi.cuh - the two warps of a 64-thread block.  Thread t of the group owns row t / slot t / constraint block t.
+// `scr`: eight doubles of shared memory per problem (only the two-warp form touches it).
+__device__ __forceinline__ void warp_argmin(double &v, int &idx) {  // smallest (value, index); ties to the smaller index; index < 0 = none
+    // Three warp-wide integer reductions (REDUX) on an order-preserving 64-bit key instead of five rounds of three shuffles and a
+    // compare chain: the high word, the low word among the lanes that hold the smallest high word, then the index among those.
+    unsigned long long u = (unsigned long long)__double_as_longlong(v);
+    u = (u >> 63) ? ~u : (u | 0x8000000000000000ull);  // ascending as unsigned: negative values below positive ones
+    if (idx < 0) u = ~0ull;
+    const unsigned hi = (unsigned)(u >> 32), lo = (unsigned)u;
+    const unsigned mhi = __reduce_min_sync(0xffffffffu, hi);
+    const unsigned mlo = __reduce_min_sync(0xffffffffu, hi == mhi ? lo : 0xffffffffu);
+    const bool mine = idx >= 0 && hi == mhi && lo == mlo;
+    const unsigned midx = __reduce_min_sync(0xffffffffu, mine ? (unsigned)idx : 0xffffffffu);
+    if (midx == 0xffffffffu) { idx = -1; return; }  // no candidate (v is left as it is)
+    unsigned long long m = ((unsigned long long)mhi << 32) | mlo;
+    m = (m >> 63) ? (m & 0x7fffffffffffffffull) : ~m;
+    v = __longlong_as_double((long long)m);
+    idx = (int)midx;
+}
+template <int NW>
+struct MpcGroup;
+template <>
+struct MpcGroup<1> {
+    static constexpr int threads = 32;
+    static __device__ __forceinline__ int tid() { return threadIdx.x & 31; }
+    static __device__ __forceinline__ void sync() { __syncwarp(); }
+    static __device__ __forceinline__ double sum(double v, double *) { return warp_sum(v); }
+    static __device__ __forceinline__ double max(double v, double *) { return warp_max(v); }
+    static __device__ __forceinline__ void argmin(double &v, int &idx, double *) { warp_argmin(v, idx); }
+};
+template <>
+struct MpcGroup<2> {  // one problem per 64-thread block
+    static constexpr int threads = 64;
+    static __device__ __forceinline__ int tid() { return threadIdx.x; }
+    static __device__ __forceinline__ void sync() { __syncthreads(); }
+    static __device__ __forceinline__ double sum(double v, double *scr) {
+        v = warp_sum(v);
+        if ((threadIdx.x & 31) == 0) scr[threadIdx.x >> 5] = v;
+        __syncthreads();
+        v = scr[0] + scr[1];
+        __syncthreads();
+        return v;
+    }
+    static __device__ __forceinline__ double max(double v, double *scr) {
+        v = warp_max(v);
+        if ((threadIdx.x & 31) == 0) scr[threadIdx.x >> 5] = v;
+        __syncthreads();
+        v = fmax(scr[0], scr[1]);
+        __syncthreads();
+        return v;
+    }
+    static __device__ __forceinline__ void argmin(double &v, int &idx, double *scr) {
+        warp_argmin(v, idx);
+        if ((threadIdx.x & 31) == 0) {
+            scr[2 + 2 * (threadIdx.x >> 5)] = v;
+            scr[3 + 2 * (threadIdx.x >> 5)] = (double)idx;
+        }
+        __syncthreads();
+        const double v0 = scr[2], v1 = scr[4];
+        const int i0 = (int)scr[3], i1 = (int)scr[5];
+        const bool second = i1 >= 0 && (i0 < 0 || v1 < v0 || (v1 == v0 && i1 < i0));
+        v = second ? v1 : v0;
+        idx = second ? i1 : i0;
+        __syncthreads();
+    }
+};
+
+// Condensed QP, thread by row in registers: hrow <- row `lane` of 2 sum_i Su_i^T W Su_i (WITHOUT the 2 w_force of the diagonal),
+// grow <- entry `lane` of g = 2 sum_i Su_i^T W (sc_i - ref_i).  `lane` is the thread's index in its group (MpcGroup<NW>).
+// Unknown 3 (NFL i + r) + c = component c of free_leg[r] at stage i; a free_leg entry that is a swing leg is a phantom (no
+// dynamics: its row and column are zero).
+// scratch: shared memory, mpc_condense_scratch(NFL) doubles: the sensitivities Su [12][ld] of the stage state to the forces, the five
+// rotation matrices of the horizon and its 60 reference values.
+//   * the rotations (three sin / cos pairs each) are evaluated ONCE, stage i by thread i, instead of by every thread in every
+//     stage; the reference states are fetched once, coalesced, instead of one dependent global load per use;
+//   * rows 3..5 and 9..11 of Su (position and velocity sensitivities) are known in closed form - a force component c of stage j
+//     changes velocity c by dt / m from stage j on and position c by (i - j) dt^2 / m at stage i, nothing else - so their part of
+//     the Gram matrix, sum_i over the common stages of w_pos (i - j)(i - j') (dt^2 / m)^2 + w_vel (dt / m)^2 for equal components,
+//     is added once at the end, and the per-stage accumulation runs over the six attitude / body-rate rows only (pairs of columns
+//     per 16-byte load): half the FMAs and a third of the shared-memory loads of the straightforward form.
+__host__ __device__ constexpr int mpc_condense_scratch(int nfl) { return 12 * mpcg_even(15 * nfl) + 48 + 64; }
+
+template <int NFL, int NW = 1>
+__device__ __forceinline__ void mpc_condense(const MpcParams &prm, long long prob, int lane, const int (&kind_leg)[4], const int (&free_leg)[4],
+                                             double *scratch, double (&hrow)[15 * NFL], double &grow) {
+    using G = MpcGroup<NW>;
+    constexpr int n = 15 * NFL, ld = mpcg_even(n), GT = G::threads;
+    const long long N = prm.N;
+    const int row = lane < n ? lane : n - 1;
+    double *Su = scratch, *Rs = scratch + 12 * ld, *bref = Rs + 48;  // Rs [5][9] (padded), bref [5][12]
+    for (int e = lane; e < 12 * ld; e += GT) Su[e] = 0.0;
+    for (int e = lane; e < MPC_NH * 12; e += GT) bref[e] = prm.body_ref[(long long)e * N + prob];
+    grow = 0.0;
+#pragma unroll
+    for (int j = 0; j < n; ++j) hrow[j] = 0.0;
+    double sc[12], pf[12];
+#pragma unroll
+    for (int k = 0; k < 12; ++k) sc[k] = prm.x[k * N + prob];
+#pragma unroll
+    for (int k = 0; k < 12; ++k) pf[k] = prm.p[k * N + prob];
+    bool real[NFL];  // leg r of the unknowns carries a force (not a phantom)
+#pragma unroll
+    for (int r = 0; r < NFL; ++r) {
+        real[r] = false;
+#pragma unroll
+        for (int q = 0; q < 4; ++q)
+            if (q == free_leg[r]) real[r] = kind_leg[q] != 0;
+    }
+    G::sync();
+    if (lane < MPC_NH) {  // linearisation attitude of stage i: the current state for stage 0, body_ref[:, i - 1] after
+        double R[9];
+        if (lane == 0) rot_zyx(sc[0], sc[1], sc[2], R);
+        else rot_zyx(bref[(lane - 1) * 12], bref[(lane - 1) * 12 + 1], bref[(lane - 1) * 12 + 2], R);
+#pragma unroll
+        for (int k = 0; k < 9; ++k) Rs[9 * lane + k] = R[k];
+    }
+    G::sync();
+#pragma unroll 1
+    for (int i = 0; i < MPC_NH; ++i) {
+        double R[9];
+#pragma unroll
+        for (int k = 0; k < 9; ++k) R[k] = Rs[9 * i + k];
+        // Su <- (I + dt A) Su: rows 0..2 += dt R^T rows 6..8, rows 3..5 += dt rows 9..11 (rows 6..11 unchanged)
+        if (lane < n) {
+            const int c = lane;
+            const double w0 = Su[6 * ld + c], w1 = Su[7 * ld + c], w2 = Su[8 * ld + c];
+#pragma unroll
+            for (int a = 0; a < 3; ++a) Su[a * ld + c] += prm.dt * (R[0 * 3 + a] * w0 + R[1 * 3 + a] * w1 + R[2 * 3 + a] * w2);
+#pragma unroll
+            for (int a = 0; a < 3; ++a) Su[(3 + a) * ld + c] += prm.dt * Su[(9 + a) * ld + c];
+        }
+        G::sync();
+        // Su[:, 3 NFL i + 3 r + c] += dt B: rows 6..8 = Ihat^-1 skew(R p_l), rows 9..11 = I / m;  Ihat^-1 = R diag(1/I) R^T
+        if (lane < 3 * NFL) {
+            const int c = lane % 3;
+            int l = 0;
+            bool real_leg = false;
+#pragma unroll
+            for (int r = 0; r < NFL; ++r)
+                if (r == lane / 3) { l = free_leg[r]; real_leg = real[r]; }
+            double pl[3] = {0.0, 0.0, 0.0};
+#pragma unroll
+            for (int q = 0; q < 4; ++q)
+                if (q == l) { pl[0] = pf[3 * q]; pl[1] = pf[3 * q + 1]; pl[2] = pf[3 * q + 2]; }
+            double pw[3];
+#pragma unroll
+            for (int a = 0; a < 3; ++a) pw[a] = R[3 * a] * pl[0] + R[3 * a + 1] * pl[1] + R[3 * a + 2] * pl[2];
+            double sk[3];  // column c of skew(pw) = [[0,-z,y],[z,0,-x],[-y,x,0]]
+            sk[0] = c == 0 ? 0.0 : (c == 1 ? -pw[2] : pw[1]);
+            sk[1] = c == 0 ? pw[2] : (c == 1 ? 0.0 : -pw[0]);
+            sk[2] = c == 0 ? -pw[1] : (c == 1 ? pw[0] : 0.0);
+            double t3[3];
+#pragma unroll
+            for (int a = 0; a < 3; ++a) t3[a] = prm.inv_inertia[a] * (R[a] * sk[0] + R[3 + a] * sk[1] + R[6 + a] * sk[2]);
+            const int col = 3 * NFL * i + lane;
+            if (real_leg) {
+#pragma unroll
+                for (int a = 0; a < 3; ++a) Su[(6 + a) * ld + col] += prm.dt * (R[3 * a] * t3[0] + R[3 * a + 1] * t3[1] + R[3 * a + 2] * t3[2]);
+                Su[(9 + c) * ld + col] += prm.dt * prm.inv_mass;
+            }
+        }
+        // free response: sc <- (I + dt A) sc + dt g
+        {
+            const double w0 = sc[6], w1 = sc[7], w2 = sc[8];
+#pragma unroll
+            for (int a = 0; a < 3; ++a) sc[a] += prm.dt * (R[a] * w0 + R[3 + a] * w1 + R[6 + a] * w2);
+#pragma unroll
+            for (int a = 0; a < 3; ++a) sc[3 + a] += prm.dt * sc[9 + a];
+            sc[11] += prm.dt * prm.gravity;
+        }
+        G::sync();
+        // gradient: all twelve rows of this thread's column; Gram matrix: the attitude (0..2) and body-rate (6..8) rows, columns in pairs
+        double sa[6], gacc = 0.0;
+#pragma unroll
+        for (int k = 0; k < 12; ++k) {
+            const double s_k = Su[k * ld + row];
+            if (k < 3) sa[k] = prm.w_state[k] * s_k;
+            if (k >= 6 && k < 9) sa[k - 3] = prm.w_state[k] * s_k;
+            gacc = fma(s_k, prm.w_state[k] * (sc[k] - bref[i * 12 + k]), gacc);
+        }
+        grow = fma(2.0, gacc, grow);
+        const int ncol = 3 * NFL * (i + 1);  // the later columns of Su are still zero
+#pragma unroll
+        for (int b = 0; b + 1 < n; b += 2) {
+            if (b < ncol) {  // uniform; ncol is even or the odd last column is handled below
+                double a0 = 0.0, a1 = 0.0;
+#pragma unroll
+                for (int k = 0; k < 6; ++k) {
+                    const double2 v = *reinterpret_cast<const double2 *>(Su + (k < 3 ? k : k + 3) * ld + b);
+                    a0 = fma(sa[k], v.x, a0);
+                    a1 = fma(sa[k], v.y, a1);
+                }
+                hrow[b] = fma(2.0, a0, hrow[b]);
+                hrow[b + 1] = fma(2.0, a1, hrow[b + 1]);
+            }
+        }
+        if (n & 1) {
+            double a0 = 0.0;
+#pragma unroll
+            for (int k = 0; k < 6; ++k) a0 = fma(sa[k], Su[(k < 3 ? k : k + 3) * ld + n - 1], a0);
+            hrow[n - 1] = fma(2.0, a0, hrow[n - 1]);
+        }
+        G::sync();
+    }
+    // closed-form part: position and velocity rows (see the header)
+    {
+        const int jr = row / (3 * NFL), rr = (row / 3) % NFL, cr = row % 3;
+        bool real_row = false;
+#pragma unroll
+        for (int r = 0; r < NFL; ++r)
+            if (r == rr) real_row = real[r];
+        const double d2m = prm.dt * prm.dt * prm.inv_mass, d1m = prm.dt * prm.inv_mass;
+        double wp = 0.0, wv = 0.0;  // 2 w_pos (dt^2 / m)^2 and 2 w_vel (dt / m)^2 of this row's component
+#pragma unroll
+        for (int c = 0; c < 3; ++c)
+            if (c == cr) { wp = 2.0 * prm.w_state[3 + c] * d2m * d2m; wv = 2.0 * prm.w_state[9 + c] * d1m * d1m; }
+#pragma unroll
+        for (int b = 0; b < n; ++b) {
+            const int jb = b / (3 * NFL), rb = (b / 3) % NFL, cb = b % 3;  // compile-time after unrolling
+            int s1 = 0, cnt = 0;  // sum over the common stages i >= max(jr, jb) of (i - jr)(i - jb), and their number
+#pragma unroll
+            for (int i = 0; i < MPC_NH; ++i)
+                if (i >= jb && i >= jr) { s1 += (i - jr) * (i - jb); ++cnt; }
+            if (cb == cr && real_row && real[rb]) hrow[b] += wp * (double)s1 + wv * (double)cnt;
+        }
+    }
+}
 
 #ifndef OKF_MPCG_WARPS
 #define OKF_MPCG_WARPS 5
@@ -45,7 +290,7 @@ __host__ __device__ constexpr int mpcg_group(int nfl) { return nfl <= 2 ? 32 : 6
 // per-problem shared memory (doubles): H^-1 [n][n|1] (Su [12][n] while H is built) | S^-1 [slots][slots+1] | x g | strip 2 x 64, after the
 // inversion y d r (three vectors of one entry per thread) | normals [3][threads] | block and id of a slot, list of the slots in use (3 ints per thread) | scratch 8
 __host__ __device__ constexpr int mpcg_problem_doubles(int nfl) {
-    return mpcr_even((15 * nfl) * ((15 * nfl) | 1)) + mpcg_slots(nfl) * (mpcg_slots(nfl) + 1) + 2 * mpcg_group(nfl) +
+    return mpcg_even((15 * nfl) * ((15 * nfl) | 1)) + mpcg_slots(nfl) * (mpcg_slots(nfl) + 1) + 2 * mpcg_group(nfl) +
            (3 * mpcg_group(nfl) > 128 ? 3 * mpcg_group(nfl) : 128) + 3 * mpcg_group(nfl) + mpcg_group(nfl) + mpcg_group(nfl) / 2 + 8;
 }
 __host__ __device__ constexpr size_t mpcg_smem_bytes() { return (size_t)MPCG_WARPS * mpcg_problem_doubles(2) * sizeof(double); }
@@ -93,7 +338,7 @@ __device__ __forceinline__ void mpc_solve_gi(const MpcParams &prm, long long pro
     static_assert(n <= GT && SLOTS <= GT && mpc_condense_scratch(NFL) <= n * ldg && GT == mpcg_group(NFL), "layout");
     const long long N = prm.N;
     const int lane = G::tid();  // index in the group: row / slot / constraint block owned by this thread
-    double *Ginv = base, *Su = base, *P = Ginv + mpcr_even(n * ldg), *xs = P + SLOTS * LDP, *g = xs + GT, *strip = g + GT;
+    double *Ginv = base, *Su = base, *P = Ginv + mpcg_even(n * ldg), *xs = P + SLOTS * LDP, *g = xs + GT, *strip = g + GT;
     double *y = strip, *dslot = y + GT, *rslot = dslot + GT, *ncoef = strip + (3 * GT > 128 ? 3 * GT : 128);  // y, d, r reuse the strip once H is inverted
     int *sblk = reinterpret_cast<int *>(ncoef + 3 * GT), *sid = sblk + GT, *slist = sid + GT;
     double *scr = reinterpret_cast<double *>(slist + GT);
@@ -524,7 +769,7 @@ __global__ void __launch_bounds__(32 * MPCG_WARPS, MPCG_MIN_BLOCKS) kf_mpc_gi_ke
                 if (r == nfl) free_leg[r] = l;
             ++nfl;
         }
-    if (nfl > prm.max_legs || nfl > MPCR_MAX_LEGS) {  // the caller's bound on the legs out of swing is wrong for this problem: no answer
+    if (nfl > prm.max_legs || nfl > MPCG_MAX_LEGS) {  // the caller's bound on the legs out of swing is wrong for this problem: no answer
         for (int e = lane; e < MPC_N; e += 32) prm.forces[(long long)e * N + prob] = __longlong_as_double(0x7ff8000000000000LL);
         if (lane == 0) prm.status[prob] = 4u;
         if (prm.warm_set && lane < MPC_NH) prm.warm_set[(long long)lane * N + prob] = 0u;

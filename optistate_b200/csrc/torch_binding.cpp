@@ -346,11 +346,10 @@ int kf_mpc_forces(int64_t n, int64_t max_free_legs, const std::map<std::string, 
     d.contact = ck.get(tensors, "contact", 4 * n, true);
     d.forces = const_cast<void *>(ck.get(tensors, "forces", OPTI_KF_MPC_HORIZON * 12 * n, true));
     auto is = tensors.find("status");
-    if (is != tensors.end()) {
-        const at::Tensor &t = is->second;
-        TORCH_CHECK(t.is_cuda() && t.device() == ck.dev && t.scalar_type() == at::kInt && t.is_contiguous() && t.numel() == n, "optistate_b200: bad 'status'");
-        d.status = reinterpret_cast<uint32_t *>(t.data_ptr<int32_t>());
-    }
+    TORCH_CHECK(is != tensors.end(), "optistate_b200: missing tensor 'status'");
+    const at::Tensor &st = is->second;
+    TORCH_CHECK(st.is_cuda() && st.device() == ck.dev && st.scalar_type() == at::kInt && st.is_contiguous() && st.numel() == n, "optistate_b200: bad 'status'");
+    d.status = reinterpret_cast<uint32_t *>(st.data_ptr<int32_t>());
     auto iw = tensors.find("warm_set");
     if (iw != tensors.end()) {
         const at::Tensor &t = iw->second;
@@ -358,8 +357,6 @@ int kf_mpc_forces(int64_t n, int64_t max_free_legs, const std::map<std::string, 
                     "optistate_b200: bad 'warm_set'");
         d.warm_set = reinterpret_cast<uint32_t *>(t.data_ptr<int32_t>());
         d.warm_mult = const_cast<void *>(ck.get(tensors, "warm_mult", OPTI_KF_MPC_HORIZON * 4 * 5 * n, true));
-        auto wr = consts.find("warm_rounds");
-        d.warm_rounds = wr == consts.end() ? 0 : (int32_t)wr->second;
     }
     auto sv = consts.find("solver");
     d.solver = sv == consts.end() ? 0 : (int32_t)sv->second;

@@ -35,8 +35,8 @@ def mpc_forces(x, body_ref, p, contact, *, dt: float = INITIAL_PARAMS.DT_mpc, ma
     contact [4, N] (0 swing, 1 stance).  max_free_legs: bound on the legs out of swing in any problem (None = taken from
     `contact`, which costs one small reduction and a host sync; it sizes the kernel's shared memory).
     solver: "auto" - the dual active-set kernels (csrc/kf_mpc_gi.cuh: one warp per problem for at most two legs out of swing, two
-    warps for three and four), with the interior-point kernels behind them for problems they give up on; "interior_point" - the
-    interior-point kernels only.
+    warps for three and four), with the interior-point kernel (csrc/kf_mpc.cuh) behind them for problems they give up on;
+    "interior_point" - the interior-point kernel only, for every leg count (it takes no warm start).
     max_changes: cap on the constraints the dual active-set method may enter + drop per problem before it hands the problem to the
     interior point (0 = the kernel's default, 400).
     warm: a `WarmStart` (in / out) carrying the active set and multipliers from one solve to the next one of the same
@@ -64,7 +64,6 @@ def mpc_forces(x, body_ref, p, contact, *, dt: float = INITIAL_PARAMS.DT_mpc, ma
         if warm.n != n or warm.active.device != device:
             raise ValueError("warm start was set up for another batch size or device")
         tensors.update(warm_set=warm.active, warm_mult=warm.multipliers)
-        consts["warm_rounds"] = float(warm.rounds)
     with torch.cuda.device(device):
         nv.check(int(nv.ext().kf_mpc_forces(n, int(max_free_legs), consts, [float(w) for w in w_state], tensors)), "optistate_kf_mpc_forces")
     return forces, status
@@ -74,9 +73,8 @@ class WarmStart:
     """Active set and multipliers carried between consecutive solves of the same N problems (include/optistate_kf.h,
     OptiKfMpcDesc.warm_set / warm_mult).  Starts empty: the first solve is a cold one."""
 
-    def __init__(self, n: int, device=None, rounds: int = 0):
+    def __init__(self, n: int, device=None):
         nv.require_cuda()
-        self.rounds = int(rounds)  # active-set correction rounds before the interior point takes over (0 = the kernel's default)
         device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.n = int(n)
         self.active = torch.zeros((HORIZON, self.n), dtype=torch.int32, device=device)

@@ -137,11 +137,11 @@ def test_workspace_query(lib):
     assert n.value >= 10 * 10 * 256 * 8 + 256 * 4
 
 
-def test_extension_loads_and_refuses_cpu_tensors():
+def test_extension_loads_at_abi_5_and_refuses_cpu_tensors():
     from optistate_b200 import _native as nv
 
     ext = nv.ext()
-    assert ext.abi_version() == nv.ABI_VERSION == 4 and ext.MAX_PEERS == 7 and ext.launch_count() >= 0
+    assert ext.abi_version() == nv.ABI_VERSION == 5 and ext.MAX_PEERS == 7 and ext.launch_count() >= 0
     cfg = dict(dtype=nv.F64, n_traj=1, n_steps=1, n_streams=1)
     consts = dict(dt=0.01, mass=8.8, inertia0=0.05, inertia1=0.06, inertia2=0.1, gravity=-9.81)
     with pytest.raises(RuntimeError, match="CUDA tensor"):

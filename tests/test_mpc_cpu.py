@@ -5,6 +5,7 @@ import ctypes
 
 import numpy as np
 import pytest
+import torch
 
 from oracle import mpc_numpy as mpc
 from tests import mpc_cases
@@ -38,21 +39,29 @@ def test_oracle_solver_returns_kkt_points_for_every_contact_pattern():
     assert max(mpc.kkt_certificate(bad, H, g, A, b, pinned)) > 1e-7
 
 
-def test_mpc_descriptor_validation():
+P, D = ctypes.c_void_p, ctypes.c_double
+
+
+class _MpcDesc(ctypes.Structure):  # OptiKfMpcDesc (include/optistate_kf.h)
+    _fields_ = [("struct_size", ctypes.c_uint32), ("abi_version", ctypes.c_uint32), ("dtype", ctypes.c_int32), ("max_free_legs", ctypes.c_int32),
+                ("n_problems", ctypes.c_int64), ("x", P), ("body_ref", P), ("p", P), ("contact", P), ("forces", P), ("status", P),
+                ("warm_set", P), ("warm_mult", P), ("solver", ctypes.c_int32), ("max_changes", ctypes.c_int32), ("reserved0", ctypes.c_int32), ("dt", D), ("mass", D), ("inertia", D * 3), ("gravity", D), ("mu", D), ("fz_max", D), ("w_state", D * 12), ("w_force", D)]
+
+
+def _mpc_lib_and_desc():
+    """The library and a descriptor of four problems with valid constants and no pointers."""
     from optistate_b200 import _build
 
     lib = ctypes.CDLL(_build.build_all()[0])
-    P, D = ctypes.c_void_p, ctypes.c_double
-
-    class Desc(ctypes.Structure):
-        _fields_ = [("struct_size", ctypes.c_uint32), ("abi_version", ctypes.c_uint32), ("dtype", ctypes.c_int32), ("max_free_legs", ctypes.c_int32),
-                    ("n_problems", ctypes.c_int64), ("x", P), ("body_ref", P), ("p", P), ("contact", P), ("forces", P), ("status", P),
-                    ("warm_set", P), ("warm_mult", P), ("warm_rounds", ctypes.c_int32), ("solver", ctypes.c_int32), ("max_changes", ctypes.c_int32), ("reserved0", ctypes.c_int32), ("dt", D), ("mass", D), ("inertia", D * 3), ("gravity", D), ("mu", D), ("fz_max", D), ("w_state", D * 12), ("w_force", D)]
-
-    d = Desc(struct_size=ctypes.sizeof(Desc), abi_version=lib.optistate_kf_abi_version(), dtype=0, n_problems=4, dt=0.01, mass=8.8,
-             gravity=-9.81, mu=0.6, fz_max=150.0, w_force=1e-6)
+    d = _MpcDesc(struct_size=ctypes.sizeof(_MpcDesc), abi_version=lib.optistate_kf_abi_version(), dtype=0, n_problems=4, dt=0.01, mass=8.8,
+                 gravity=-9.81, mu=0.6, fz_max=150.0, w_force=1e-6)
     d.inertia = (D * 3)(0.055, 0.060, 0.105)
     d.w_state = (D * 12)(*([1.0] * 12))
+    return lib, d
+
+
+def test_mpc_descriptor_validation():
+    lib, d = _mpc_lib_and_desc()
     assert lib.optistate_kf_mpc_forces(ctypes.byref(d), None) == -1  # pointers missing
     d.dtype = 1
     assert lib.optistate_kf_mpc_forces(ctypes.byref(d), None) == -3  # FP64 only
@@ -66,6 +75,18 @@ def test_mpc_descriptor_validation():
     d.struct_size -= 8
     assert lib.optistate_kf_mpc_forces(ctypes.byref(d), None) == -2
     assert lib.optistate_kf_mpc_forces(None, None) == -1
+
+
+# Where a device is present, a descriptor that passes validation would launch kernels on the fake pointers.
+@pytest.mark.skipif(torch.cuda.is_available(), reason="runs only without a CUDA device")
+def test_mpc_forces_requires_a_status_array():
+    """The dual active set marks the problems it hands to the interior point in `status`; without it every problem would go to
+    the slower interior point, so a call without one is refused."""
+    lib, d = _mpc_lib_and_desc()
+    fake = ctypes.c_void_p(0x1000)  # never dereferenced: validation only
+    for n in ("x", "body_ref", "p", "contact", "forces", "warm_set", "warm_mult"):
+        setattr(d, n, fake)
+    assert lib.optistate_kf_mpc_forces(ctypes.byref(d), None) == -1
 
 
 def _oracle_verdict(f, x, ref, p, contact):

@@ -106,7 +106,7 @@ def test_shared_memory_bound_on_the_legs_out_of_swing():
     x, ref, p, c = mpc_cases.batch(64, seed=7)
     c[:] = np.array([1.0, 0.0, 0.0, 1.0])[:, None]  # a trot: two legs in stance
     loose, _ = mpc_forces(x, ref, p, c, max_free_legs=4)   # the shared-memory kernel (kf_mpc.cuh)
-    tight, st = mpc_forces(x, ref, p, c)              # bound taken from the contact array: 2 - the row-per-lane kernel (kf_mpc_rows.cuh)
+    tight, st = mpc_forces(x, ref, p, c)              # bound taken from the contact array: 2 - the one-warp kernel (kf_mpc_gi.cuh)
     assert float((loose - tight).abs().max()) < 1e-8 * float(tight.abs().max()) and not (st & 7).any()
     c[:, 5] = 1.0                                      # one problem with four legs in stance, but the caller promises two
     wrong, st = mpc_forces(x, ref, p, c, max_free_legs=2)
@@ -131,46 +131,6 @@ def test_trot_batch_polishes_every_problem():
         assert np.abs(u - want).max() < 1e-8 * max(1.0, np.abs(want).max()), k
         viol, stat = mpc.kkt_certificate(u, H, g, A, b, pinned)
         assert viol < 1e-7 and stat < 1e-8, (k, viol, stat)
-
-
-def test_warm_start_is_verified_and_falls_back():
-    """Closed-loop warm start (kf_mpc_rows.cuh): the active set and multipliers of one solve start the next one.  The same
-    problems again: every constrained problem is accepted without an interior-point phase and returns the same forces; nearby
-    problems (the next filter step): still the exact minimiser, whatever path each one took; a changed contact pattern: cold
-    path, same answer as a cold solve."""
-    from optistate_b200.mpc import ST_WARM, WarmStart
-
-    n = 512
-    x, ref, p, c = mpc_cases.batch(n, seed=3)
-    c[:] = np.where((np.arange(n) % 2 == 0)[None, :], np.array([1.0, 0, 0, 1])[:, None], np.array([0, 1.0, 1, 0])[:, None])
-    ip = dict(solver="interior_point")                  # kf_mpc_rows.cuh: the warm set skips the interior-point phase when it verifies
-    warm = WarmStart(n)
-    cold, st0 = mpc_forces(x, ref, p, c, warm=warm, **ip)
-    assert not (st0 & (7 | ST_WARM)).any() and int((st0 >> 8).min()) > 0            # interior point everywhere
-    again, st1 = mpc_forces(x, ref, p, c, warm=warm, **ip)
-    assert (st1 & ST_WARM).all() and not (st1 & 7).any() and int((st1 >> 8).max()) == 0
-    assert float((again - cold).abs().max()) < 1e-8 * float(cold.abs().max())
-    # the next step of a closed loop: states and references move a little
-    rng = np.random.default_rng(9)
-    x2 = x + 2e-3 * rng.standard_normal(x.shape)
-    ref2 = ref + 1e-3 * rng.standard_normal(ref.shape)
-    near, st2 = mpc_forces(x2, ref2, p, c, warm=warm, **ip)
-    plain, st2c = mpc_forces(x2, ref2, p, c, **ip)
-    assert not (st2 & 7).any() and not (st2c & 7).any()
-    assert float((st2 & ST_WARM).ne(0).double().mean()) > 0.5, float((st2 & ST_WARM).ne(0).double().mean())
-    assert float((near - plain).abs().max()) < 1e-8 * float(plain.abs().max())
-    F = near.cpu().numpy()
-    for k in range(0, n, 37):
-        H, g, _ = mpc.build_qp(x2[:, k], ref2[:, :, k].T, p[:, k])
-        A, b, pinned = mpc.constraints(c[:, k])
-        want = mpc.solve_ldp(H, g, A, b, pinned)
-        u = F[:, :, k].reshape(-1)
-        assert np.abs(u - want).max() < 1e-8 * max(1.0, np.abs(want).max()), k
-    # the gait switches legs: the stored sets belong to other legs
-    c2 = 1.0 - c
-    sw, st3 = mpc_forces(x2, ref2, p, c2, warm=warm, **ip)
-    sw_cold, _ = mpc_forces(x2, ref2, p, c2, **ip)
-    assert not (st3 & (7 | ST_WARM)).any() and float((sw - sw_cold).abs().max()) < 1e-8 * float(sw_cold.abs().max())
 
 
 def test_dual_active_set_warm_start_and_solver_agreement():

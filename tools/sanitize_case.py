@@ -31,7 +31,7 @@ trot = np.where((np.arange(n) % 2 == 0)[None, :], np.array([1.0, 0, 0, 1])[:, No
 warm = WarmStart(n)
 for _ in range(2):
     f1, s1 = mpc_forces(x, ref, p, trot, warm=warm)                      # dual active set, one warp (cold, then warm)
-f2, s2 = mpc_forces(x, ref, p, trot, solver="interior_point")            # row-per-lane interior point
+f2, s2 = mpc_forces(x, ref, p, trot, solver="interior_point")            # shared-memory interior point
 warm4 = WarmStart(n)
 for _ in range(2):
     f3, s3 = mpc_forces(x, ref, p, c, warm=warm4)                        # all contact patterns: two warps per problem
