@@ -159,8 +159,9 @@ typedef struct OptiKfDesc {
     uint32_t *status;     /* [N] */
 
     /* optional scratch (device memory owned by the caller) of at least optistate_kf_workspace_bytes():
-       lets the SEQUENTIAL path hoist the state-independent measurement formation into a pre-pass and stream
-       the per-step inputs with TMA; without it the measurement is formed inside the filter kernel */
+       lets the SEQUENTIAL path hoist the state-independent work of every base stream - the measurement formation
+       (unless z_in is given) and the leg moments of the mean model - into a pre-pass and stream the per-step inputs
+       with TMA; without it the filter kernel forms both per trajectory */
     void *workspace;
     size_t workspace_bytes;
 

@@ -145,7 +145,8 @@ def kf_batch(
     outputs: any of x_steps, x_model_steps, p_world_steps, z_steps, p_trace_steps (alias p_trace), k_gain_steps
     (k_gain), nis_steps, P_ckpt (p_checkpoints, needs ckpt_every), x_final, P_final, final (= both), K_final, summary.
     algo: "auto" | "sequential" | "joint" (see include/optistate_kf.h).  cov_model: "predict" | "mpc".
-    out: optional preallocated output tensors by canonical name.
+    out: optional preallocated output tensors by canonical name, and "workspace" (uint8 scratch of the streamed sequential
+    path); a workspace that is missing or smaller than the library asks for is replaced in `out` by one of the queried size.
     p0_is_symmetric: skips the (synchronising) symmetry test of a dense P0 when the caller knows the answer, e.g. when P0
     is the P_final of a previous sequential call.
     structure: "auto" | "full" - the sequential kernels exploit that predict()'s F_d only couples attitude with body rate
@@ -252,6 +253,8 @@ def kf_batch(
             ws = out.get("workspace") if out is not None else None
             if ws is None or ws.numel() < ws_bytes:
                 ws = torch.empty(int(ws_bytes), dtype=torch.uint8, device=device)
+                if out is not None:
+                    out["workspace"] = ws  # kept for the caller's next call with the same shapes
             tensors["workspace"] = ws
         nv.check(int(ext.kf_batch(cfg, consts, tensors)), "optistate_kf_batch")
     res = {k: tensors[k] for k in want}

@@ -9,6 +9,7 @@
 #include "kf_identify.cuh"
 #include "kf_launch.cuh"
 #include "kf_mpc_params.cuh"
+#include "kf_seq_core.cuh"
 
 namespace {
 
@@ -93,18 +94,24 @@ okf::Params<Real> make_params(const OptiKfDesc *d) {
 }
 
 template <typename Real>
-void launch_measure(long long T, long long S, const Real *imu, const Real *p, const Real *dp, const Real *contact, Real *z,
-                    Real *odom, uint32_t *status, cudaStream_t stream);
+void launch_measure(long long T, long long S, const Real *imu, const Real *p, const Real *dp, const Real *contact, const Real *f, Real *z,
+                    Real *mom, Real *odom, uint32_t *status, cudaStream_t stream);
 
 inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
-// bytes of scratch the streamed SEQUENTIAL path wants: z [T][10][S] + per-stream status [S]
-size_t seq_workspace_bytes(const OptiKfDesc *d) {
-    if (d->phases != OPTI_KF_PHASE_ALL) return 0;
-    const size_t esz = d->dtype == OPTI_KF_F64 ? 8 : 4;
-    const size_t z_bytes = ((size_t)d->n_steps * okf::NZ * (size_t)d->n_streams * esz + 255) & ~(size_t)255;
-    return z_bytes + (((size_t)d->n_streams * sizeof(uint32_t) + 255) & ~(size_t)255);
-}
+// Scratch of the streamed SEQUENTIAL path, each part padded to 256 bytes: z [T][10][S] (PHASE_ALL only), the leg moments of the
+// mean model M [T][12][S], and the per-stream status [S] (PHASE_ALL only).  Byte offsets; z starts at 0.
+struct SeqWorkspace {
+    size_t mom, status, total;
+    explicit SeqWorkspace(const OptiKfDesc *d) {
+        const auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+        const size_t esz = d->dtype == OPTI_KF_F64 ? 8 : 4, ts = (size_t)d->n_steps * (size_t)d->n_streams;
+        const bool all = d->phases == OPTI_KF_PHASE_ALL;
+        mom = all ? up(ts * okf::NZ * esz) : 0;
+        status = mom + up(ts * okf::NM * esz);
+        total = status + (all ? up((size_t)d->n_streams * sizeof(uint32_t)) : 0);
+    }
+};
 
 // The streamed kernel needs every warp (32 consecutive trajectories) to read one aligned tile of 32 consecutive
 // streams, 16-byte aligned arrays and row counts that fit the 32-bit tensor-map coordinates.
@@ -170,24 +177,27 @@ int launch(const OptiKfDesc *d, int algo, cudaStream_t stream) {
         p.stream_status = d->status;
     }
     if (algo == OPTI_KF_ALGO_SEQUENTIAL) {
-        bool streamed = tma_layout_ok(d);
-        if (streamed && d->phases == OPTI_KF_PHASE_ALL) {
-            // hoist the state-independent measurement formation into a pre-pass over the S base streams
-            const size_t need = seq_workspace_bytes(d);
-            if (d->workspace && d->workspace_bytes >= need && aligned16(d->workspace)) {
-                const size_t esz = sizeof(Real);
-                const size_t z_bytes = ((size_t)d->n_steps * okf::NZ * (size_t)d->n_streams * esz + 255) & ~(size_t)255;
-                Real *z = (Real *)d->workspace;
-                uint32_t *sst = (uint32_t *)((unsigned char *)d->workspace + z_bytes);
-                if (cudaMemsetAsync(sst, 0, (size_t)d->n_streams * sizeof(uint32_t), stream) != cudaSuccess) return OPTI_KF_E_CUDA;
-                launch_measure<Real>(d->n_steps, d->n_streams, p.imu, p.p, p.dp, p.contact, z, nullptr, sst, stream);
-                p.z_in = z;
-                p.stream_status = sst;
+        bool streamed = tma_layout_ok(d) && (d->phases == OPTI_KF_PHASE_ALL || aligned16(p.z_in));
+        if (streamed) {
+            // hoist the state-independent work into a pre-pass over the S base streams: the leg moments of the mean model
+            // and, unless the caller supplies z, the measurements
+            const SeqWorkspace ws(d);
+            if (d->workspace && d->workspace_bytes >= ws.total && aligned16(d->workspace)) {
+                unsigned char *base = (unsigned char *)d->workspace;
+                Real *z = nullptr;
+                uint32_t *sst = nullptr;
+                if (d->phases == OPTI_KF_PHASE_ALL) {
+                    z = (Real *)base;
+                    sst = (uint32_t *)(base + ws.status);
+                    if (cudaMemsetAsync(sst, 0, (size_t)d->n_streams * sizeof(uint32_t), stream) != cudaSuccess) return OPTI_KF_E_CUDA;
+                    p.z_in = z;
+                    p.stream_status = sst;
+                }
+                p.mom = (Real *)(base + ws.mom);
+                launch_measure<Real>(d->n_steps, d->n_streams, p.imu, p.p, p.dp, p.contact, p.f, z, (Real *)p.mom, nullptr, sst, stream);
             } else {
                 streamed = false;
             }
-        } else if (streamed && !aligned16(p.z_in)) {
-            streamed = false;
         }
         if (streamed) {
             const int rc = launch_streamed<Real>(d, p, stream);
@@ -208,42 +218,57 @@ int launch(const OptiKfDesc *d, int algo, cudaStream_t stream) {
     return cudaGetLastError() == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
 }
 
-// ---- batched get_odom + set_measurements ---------------------------------------------------------------------
+// ---- batched get_odom + set_measurements, and the leg moments of the mean model (leg_moments, kf_seq_core.cuh) ----------
+// z / odom / status: the measurement (imu, dp and contact are read only then); mom: the moments of p and f
 template <typename Real>
 __global__ void __launch_bounds__(256) kf_measure_kernel(long long T, long long S, const Real *__restrict__ imu,
                                                          const Real *__restrict__ p, const Real *__restrict__ dp,
-                                                         const Real *__restrict__ contact, Real *__restrict__ z,
+                                                         const Real *__restrict__ contact, const Real *__restrict__ f,
+                                                         Real *__restrict__ z, Real *__restrict__ mom,
                                                          Real *__restrict__ odom, uint32_t *__restrict__ status) {
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;  // (t, s) flattened, s fastest
     if (idx >= T * S) return;
     const long long t = idx / S, s = idx % S;
-    Real im[6], pp[12], dd[12], cc[4], zz[okf::NZ];
+    Real pp[12];
 #pragma unroll
-    for (int c = 0; c < 6; ++c) im[c] = imu[(t * 6 + c) * S + s];
+    for (int c = 0; c < 12; ++c) pp[c] = p[(t * 12 + c) * S + s];
+    if (z || odom || status) {
+        Real im[6], dd[12], cc[4], zz[okf::NZ];
 #pragma unroll
-    for (int c = 0; c < 12; ++c) { pp[c] = p[(t * 12 + c) * S + s]; dd[c] = dp[(t * 12 + c) * S + s]; }
+        for (int c = 0; c < 6; ++c) im[c] = imu[(t * 6 + c) * S + s];
 #pragma unroll
-    for (int c = 0; c < 4; ++c) cc[c] = contact[(t * 4 + c) * S + s];
-    const bool all_swing = okf::form_measurement(im, pp, dd, cc, zz);
-    if (z) {
+        for (int c = 0; c < 12; ++c) dd[c] = dp[(t * 12 + c) * S + s];
 #pragma unroll
-        for (int c = 0; c < okf::NZ; ++c) z[(t * okf::NZ + c) * S + s] = zz[c];
+        for (int c = 0; c < 4; ++c) cc[c] = contact[(t * 4 + c) * S + s];
+        const bool all_swing = okf::form_measurement(im, pp, dd, cc, zz);
+        if (z) {
+#pragma unroll
+            for (int c = 0; c < okf::NZ; ++c) z[(t * okf::NZ + c) * S + s] = zz[c];
+        }
+        if (odom) {
+            odom[(t * 4 + 0) * S + s] = zz[3];
+            odom[(t * 4 + 1) * S + s] = zz[7];
+            odom[(t * 4 + 2) * S + s] = zz[8];
+            odom[(t * 4 + 3) * S + s] = zz[9];
+        }
+        if (status && all_swing) atomicOr(status + s, (uint32_t)OPTI_KF_ST_ALL_SWING);
     }
-    if (odom) {
-        odom[(t * 4 + 0) * S + s] = zz[3];
-        odom[(t * 4 + 1) * S + s] = zz[7];
-        odom[(t * 4 + 2) * S + s] = zz[8];
-        odom[(t * 4 + 3) * S + s] = zz[9];
+    if (mom) {
+        Real ff[12], M[okf::NM];
+#pragma unroll
+        for (int c = 0; c < 12; ++c) ff[c] = f[(t * 12 + c) * S + s];
+        okf::leg_moments(pp, ff, M);
+#pragma unroll
+        for (int c = 0; c < okf::NM; ++c) mom[(t * okf::NM + c) * S + s] = M[c];
     }
-    if (status && all_swing) atomicOr(status + s, (uint32_t)OPTI_KF_ST_ALL_SWING);
 }
 
 template <typename Real>
-void launch_measure(long long T, long long S, const Real *imu, const Real *p, const Real *dp, const Real *contact, Real *z,
-                    Real *odom, uint32_t *status, cudaStream_t stream) {
+void launch_measure(long long T, long long S, const Real *imu, const Real *p, const Real *dp, const Real *contact, const Real *f, Real *z,
+                    Real *mom, Real *odom, uint32_t *status, cudaStream_t stream) {
     const long long total = T * S;
     if (total == 0) return;
-    kf_measure_kernel<Real><<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(T, S, imu, p, dp, contact, z, odom, status);
+    kf_measure_kernel<Real><<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(T, S, imu, p, dp, contact, f, z, mom, odom, status);
     g_launches.fetch_add(1, std::memory_order_relaxed);
 }
 
@@ -328,7 +353,7 @@ int optistate_kf_workspace_bytes(const OptiKfDesc *desc, size_t *bytes_out) {
     if (!bytes_out) return OPTI_KF_E_NULL;
     const int algo = resolve(desc);
     if (algo < 0) return algo;
-    *bytes_out = (algo == OPTI_KF_ALGO_SEQUENTIAL && tma_layout_ok(desc)) ? seq_workspace_bytes(desc) : 0;
+    *bytes_out = (algo == OPTI_KF_ALGO_SEQUENTIAL && tma_layout_ok(desc)) ? SeqWorkspace(desc).total : 0;
     return OPTI_KF_OK;
 }
 
@@ -363,10 +388,10 @@ int optistate_kf_measure(const OptiKfMeasureDesc *d, void *cuda_stream) {
     cudaGetLastError();
     if (d->dtype == OPTI_KF_F64)
         launch_measure<double>(d->n_steps, d->n_streams, (const double *)d->imu, (const double *)d->p, (const double *)d->dp,
-                               (const double *)d->contact, (double *)d->z, (double *)d->odom, d->status, stream);
+                               (const double *)d->contact, nullptr, (double *)d->z, nullptr, (double *)d->odom, d->status, stream);
     else
         launch_measure<float>(d->n_steps, d->n_streams, (const float *)d->imu, (const float *)d->p, (const float *)d->dp,
-                              (const float *)d->contact, (float *)d->z, (float *)d->odom, d->status, stream);
+                              (const float *)d->contact, nullptr, (float *)d->z, nullptr, (float *)d->odom, d->status, stream);
     return cudaGetLastError() == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
 }
 

@@ -16,9 +16,9 @@ constexpr size_t kAlign = 256;
 inline size_t up(size_t b) { return (b + kAlign - 1) & ~(kAlign - 1); }
 
 // workspace layout (bytes): z [T][10][N] | P ping-pong 2 x [144][N] | forces of the horizon [5][12][N] | warm set [5][N] u32 |
-// warm multipliers [100][N] | MPC status scratch [N] u32
+// warm multipliers [100][N] | MPC status scratch [N] u32 | the filter step's workspace (leg moments [12][N])
 struct Layout {
-    size_t z, p0, p1, fh, wset, wmult, mst, total;
+    size_t z, p0, p1, fh, wset, wmult, mst, fws, total;
     Layout(int64_t N, int64_t T) {
         size_t o = 0;
         z = o; o += up((size_t)T * 10 * N * 8);
@@ -28,6 +28,7 @@ struct Layout {
         wset = o; o += up((size_t)OPTI_KF_MPC_HORIZON * N * 4);
         wmult = o; o += up((size_t)OPTI_KF_MPC_HORIZON * 4 * 5 * N * 8);
         mst = o; o += up((size_t)N * 4);
+        fws = o; o += up((size_t)12 * N * 8);
         total = o;
     }
 };
@@ -99,6 +100,7 @@ int optistate_kf_closed_loop(const OptiKfClosedLoopDesc *d, void *cuda_stream) {
     f.q_kind = d->q_kind; f.r_kind = d->r_kind; f.Q = d->Q; f.R = d->R;
     f.status = d->status;
     f.flags = d->status ? OPTI_KF_FLAG_STATUS_ACCUMULATE : 0;
+    f.workspace = ws + L.fws; f.workspace_bytes = L.total - L.fws;
 
     const double *x_cur = (const double *)d->x0;
     int x_per = d->x0_per_traj;

@@ -23,6 +23,7 @@ struct Params {
     int block;  // 1: P has the decoupled group structure (OPTI_KF_FLAG_*; kBlock kernels, kf_seq_core.cuh)
     Real dt, dt_over_m, dt_g, inv_inertia[3];
     const Real *imu, *p, *dp, *contact, *f, *z_in, *body_ref, *truth, *nominal;
+    const Real *mom;  // [T][12][S] leg moments of the mean model from the measurement pre-pass (streamed kernel only)
     const int32_t *stream_index;
     const Real *x0; long long x0_ld; int x0_inc;
     const Real *P0; int p0_kind;

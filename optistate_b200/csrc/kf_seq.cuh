@@ -77,7 +77,12 @@ __global__ void __launch_bounds__(128) kf_seq_kernel(const __grid_constant__ Par
             if (form_measurement(imu, pf, dp, contact, z)) status[0] |= OPTI_KF_ST_ALL_SWING;
         }
 
-        propagate_mean_with_R<1>(prm, x, pf, ff, Rm, any_trunc, prm.p_world_steps, (t * 12) * N + i, N);
+        if (prm.p_world_steps) store_world_feet<1>(pf, Rm, prm.p_world_steps, (t * 12) * N + i, N);
+        {
+            Real M[NM];
+            leg_moments(pf, ff, M);
+            propagate_mean_from_moments<1>(prm, x, M, Rm, any_trunc);
+        }
         if (prm.x_model_steps) {
 #pragma unroll
             for (int c = 0; c < NX; ++c) st_stream(prm.x_model_steps + (t * NX + c) * N + i, x[c]);

@@ -260,31 +260,51 @@ __device__ __forceinline__ bool may_truncate(const Real (&R)[9]) {
     return m >= (sizeof(S) == 8 ? 0x3ff00000 : 0x3f7ffff0);  // |entry| >= 1 (double) / >= 1 - 2^-20 (float)
 }
 
-// Mean model with the rotation of the prior attitude supplied by the caller (see propagate_mean in kf_common.cuh).
-// Feet and forces are read leg by leg through `pin` / `fin` (channel stride STRIDE: 32 for a warp's shared-memory tile,
-// 1 for a per-thread array) so that at most one leg is live in registers; `pw_out` (optional) receives the feet rotated
-// into the world frame (the reference's in-place mutation of p, force_controller.py:274-277).
+// Leg moments of the mean model: C[3m + k] = sum_l p_l[m] f_l[k] (rows 0-8) and fs[k] = sum_l f_l[k] (rows 9-11).  They depend
+// on the stream and the step only, so the measurement pre-pass forms them once for every member of a stream; the direct-load
+// kernel forms them in-thread with this same function, which keeps the two kernels bit-identical.  Explicit mul_rn / fma_: the
+// result does not depend on contraction, and double, float and F2 run the same sequence.
+constexpr int NM = 12;
+template <typename Real>
+__device__ __forceinline__ void leg_moments(const Real (&p)[12], const Real (&f)[12], Real (&M)[NM]) {
+#pragma unroll
+    for (int m = 0; m < 3; ++m)
+#pragma unroll
+        for (int k = 0; k < 3; ++k)
+            M[3 * m + k] = fma_(p[9 + m], f[9 + k], fma_(p[6 + m], f[6 + k], fma_(p[3 + m], f[3 + k], mul_rn(p[m], f[k]))));
+#pragma unroll
+    for (int k = 0; k < 3; ++k) M[9 + k] = ((f[k] + f[3 + k]) + f[6 + k]) + f[9 + k];
+}
+
+// Feet rotated into the world frame (the reference's in-place mutation of p, force_controller.py:274-277), stored to `pw_out`;
+// `pin` reads the feet with channel stride STRIDE (32 for a warp's shared-memory tile, 1 for a per-thread array).
 template <int STRIDE, typename Real, typename Scalar>
-__device__ __forceinline__ void propagate_mean_with_R(const Params<Scalar> &prm, Real (&x)[NX], const Real *pin, const Real *fin,
-                                                      const Real (&R)[9], bool any_trunc, Scalar *pw_out, long long pw_idx, long long pw_stride) {
-    constexpr int L = Lanes<Real>::n;
-    Real tau[3] = {Real(0), Real(0), Real(0)}, fs[3] = {Real(0), Real(0), Real(0)};
+__device__ __forceinline__ void store_world_feet(const Real *pin, const Real (&R)[9], Scalar *pw_out, long long pw_idx, long long pw_stride) {
 #pragma unroll
     for (int l = 0; l < 4; ++l) {
         const Real a = pin[(3 * l) * STRIDE], b = pin[(3 * l + 1) * STRIDE], c = pin[(3 * l + 2) * STRIDE];
-        const Real pw0 = fma_(R[2], c, fma_(R[1], b, R[0] * a));
-        const Real pw1 = fma_(R[5], c, fma_(R[4], b, R[3] * a));
-        const Real pw2 = fma_(R[8], c, fma_(R[7], b, R[6] * a));
-        if (pw_out) {
-            st_traj(pw_out, pw_idx + (3 * l) * pw_stride, pw0);
-            st_traj(pw_out, pw_idx + (3 * l + 1) * pw_stride, pw1);
-            st_traj(pw_out, pw_idx + (3 * l + 2) * pw_stride, pw2);
-        }
-        const Real f0 = fin[(3 * l) * STRIDE], f1 = fin[(3 * l + 1) * STRIDE], f2 = fin[(3 * l + 2) * STRIDE];
-        tau[0] += fnma_(pw2, f1, pw1 * f2);
-        tau[1] += fnma_(pw0, f2, pw2 * f0);
-        tau[2] += fnma_(pw1, f0, pw0 * f1);
-        fs[0] += f0; fs[1] += f1; fs[2] += f2;
+        st_traj(pw_out, pw_idx + (3 * l) * pw_stride, fma_(R[2], c, fma_(R[1], b, R[0] * a)));
+        st_traj(pw_out, pw_idx + (3 * l + 1) * pw_stride, fma_(R[5], c, fma_(R[4], b, R[3] * a)));
+        st_traj(pw_out, pw_idx + (3 * l + 2) * pw_stride, fma_(R[8], c, fma_(R[7], b, R[6] * a)));
+    }
+}
+
+// Mean model with the rotation of the prior attitude supplied by the caller (see propagate_mean in kf_common.cuh), from the
+// leg moments (leg_moments; read through `min` with channel stride STRIDE).  The torque sum_l (R p_l) x f_l is regrouped
+// exactly as tau_i = eps_ijk (R C)_jk, an identity for any 3x3 R: per member 18 FP64 operations instead of 84 for the four
+// legs.  It rounds differently from the leg-by-leg order of propagate_mean (the last bits of the state).
+template <int STRIDE, typename Real, typename Scalar>
+__device__ __forceinline__ void propagate_mean_from_moments(const Params<Scalar> &prm, Real (&x)[NX], const Real *min, const Real (&R)[9],
+                                                            bool any_trunc) {
+    constexpr int L = Lanes<Real>::n;
+    const auto C = [&](int k) { return min[k * STRIDE]; };
+    // tau_i = sum_m R[j][m] C[m][k] - R[k][m] C[m][j]  for (i, j, k) a cyclic permutation of (0, 1, 2)
+    Real tau[3];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+        const int j = (i + 1) % 3, k = (i + 2) % 3;
+        tau[i] = fnma_(R[3 * k + 2], C(6 + j), fnma_(R[3 * k + 1], C(3 + j), fnma_(R[3 * k], C(j),
+                 fma_(R[3 * j + 2], C(6 + k), fma_(R[3 * j + 1], C(3 + k), mul_rn(R[3 * j], C(k)))))));
     }
     Real u[3];
 #pragma unroll
@@ -312,7 +332,7 @@ __device__ __forceinline__ void propagate_mean_with_R(const Params<Scalar> &prm,
         xn[i] = x[i] + dth[i];
         xn[3 + i] = fma_(dt, x[9 + i], x[3 + i]);
         xn[6 + i] = fma_(dt, fma_(R[3 * i + 2], u[2], fma_(R[3 * i + 1], u[1], R[3 * i] * u[0])), x[6 + i]);
-        xn[9 + i] = fma_(Real(prm.dt_over_m), fs[i], x[9 + i]);
+        xn[9 + i] = fma_(Real(prm.dt_over_m), min[(9 + i) * STRIDE], x[9 + i]);  // fs
     }
     xn[11] += Real(prm.dt_g);
 #pragma unroll

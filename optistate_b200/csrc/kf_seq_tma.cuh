@@ -3,18 +3,19 @@
 //
 //   * 32 consecutive trajectories (one warp) read 32 consecutive base streams, so the inputs of one step are
 //     [C] x 32 tiles of the [T*C][S] arrays, delivered by 2-D tensor-map copies (cp.async.bulk.tensor, SASS UTMALDG)
-//     per array - p, f, z, label streams - that complete on an mbarrier (complete_tx).  No per-thread address
+//     per array - leg moments, z, label streams - that complete on an mbarrier (complete_tx).  No per-thread address
 //     arithmetic, no LDG in the recursion, no registers tied up by loads in flight, no block-wide barrier.
 //   * The WARPS OF A BLOCK SHARE ONE TILE: they filter different members (trajectory i, i + S, i + 2 S, ...) of the same 32
-//     streams, so one copy feeds all of them and a block of four needs 15 KB of input tiles instead of 59 KB.
+//     streams, so one copy feeds all of them and a block of four needs 12 KB of FP64 input tiles instead of 47 KB.
 //     That is what decides occupancy: with a tile per warp the decoupled-group kernels (168 registers, three blocks per
 //     SM by registers) were held to two blocks by 108 KB of shared memory; with the shared tile three blocks fit
 //     (ncu: launch__occupancy_limit_shared_mem).  The warp that is LAST to finish reading a group (a shared-memory
 //     counter) issues the refill, so nobody waits on a designated producer.
 //   * Three channel groups, each single-buffered and refilled for step t+1 the moment the block has consumed
 //     step t's copy, so the copy has most of a filter step (several microseconds) to land:
-//         G0 = p[12] f[12]      read at the top of the step (mean model)        -> refilled right away
-//              (+ the 3 reference body angles of the predict_mpc covariance model in the kMpc instantiations)
+//         G0 = M[12]            read at the top of the step (mean model)        -> refilled right away
+//              (+ the feet p[12] in the kOut == 2 instantiations, which write p_world_steps, and the 3 reference body
+//              angles of the predict_mpc covariance model in the kMpc instantiations)
 //         G1 = z[10]            read one by one as the measurements are folded  -> refilled before the last fold
 //         G2 = truth / nominal  label streams of the summary, read inside the last fold -> refilled after it
 //   * Inputs are consumed straight from shared memory (conflict-free: consecutive threads, consecutive words);
@@ -26,8 +27,8 @@
 //     costs an instruction-fetch bubble at its target, ~10 % of a lone warp's time before they were compiled out.
 //   * Instantiated for double, float and F2 (kf_arith.cuh): F2 packs TWO FP32 trajectories into one thread and runs
 //     the recursion on FFMA2 / FADD2 / FMUL2, halving the issue slots per trajectory-step; its tiles are [C] x 64.
-//   * z comes from the measurement pre-pass (optistate_kf_measure): it is state-independent and, with shared
-//     base streams, identical for every Monte-Carlo member of a stream.
+//   * z and the leg moments M of the mean model (leg_moments, kf_seq_core.cuh) come from the measurement pre-pass: they are
+//     state-independent and, with shared base streams, identical for every Monte-Carlo member of a stream.
 #pragma once
 
 #include <cuda.h>  // CUtensorMap (types only; the encoder is fetched through cudaGetDriverEntryPoint)
@@ -46,8 +47,11 @@ template <bool kBlock>
 __host__ __device__ constexpr int tma_warps() { return kBlock ? OKF_BLK_WARPS : 4; }
 template <bool kBlock>
 __host__ __device__ constexpr int tma_threads() { return 32 * tma_warps<kBlock>(); }
-constexpr int TMA_CH_G0 = 24, TMA_CH_G1 = 10;
+constexpr int TMA_CH_G1 = 10;
 constexpr int TMA_CH_REF = 3;  // reference body angles of the predict_mpc covariance model (kMpc kernels), part of group G0
+// rows of group G0: the leg moments M, the feet (kOut == 2: p_world_steps) and the reference body angles (kMpc)
+template <int kOut, bool kMpc>
+__host__ __device__ constexpr int tma_g0_rows() { return NM + (kOut == 2 ? 12 : 0) + (kMpc ? TMA_CH_REF : 0); }
 constexpr int TMA_NOISE_ROWS = 22;  // q[12] r[10]
 constexpr int TMA_NOISE_ROWS_OUT = 32;  // ... and 1 / r[10] in the instantiations with per-step outputs (K_gain every step)
 template <int kW>
@@ -81,7 +85,7 @@ __device__ __forceinline__ void bulk_g2s(void *dst, const void *src, uint32_t by
 
 // tensor maps of the per-step input arrays, each viewed as a [T*C][S] matrix with a [C][32] box
 struct alignas(64) TmaMaps {
-    CUtensorMap p, f, z, lab0, lab1, body_ref;
+    CUtensorMap mom, p, z, lab0, lab1, body_ref;
 };
 
 __device__ __forceinline__ void tma_tile_g2s(void *dst, const CUtensorMap *map, int col, int row, uint64_t *bar) {
@@ -93,27 +97,27 @@ __device__ __forceinline__ void tma_tile_g2s(void *dst, const CUtensorMap *map, 
 
 template <typename Real, int kThreads, int kNoiseRows = TMA_NOISE_ROWS, int kStages = 1>
 struct TmaSmem {
-    // dynamic shared memory: [mbarriers + counters 128 B][G0 [24][32] | G1 [10][32] | G2 [12*n_lab][32] | ref [ref_rows][32]] (kStages tile
-    //                        sets per block)  [noise [22 | 32][128]][acc [25][128] (8-byte sums; double and F2 kernels only)]   (elements: Real)
-    static __host__ __device__ constexpr size_t warp_rows(int n_lab, int ref_rows) { return TMA_CH_G0 + TMA_CH_G1 + 12 * n_lab + ref_rows; }
-    static __host__ __device__ constexpr size_t warp_bytes(int n_lab, int ref_rows) { return warp_rows(n_lab, ref_rows) * 32 * sizeof(Real); }
+    // dynamic shared memory: [mbarriers + counters 128 B][G0 [g0_rows][32] | G1 [10][32] | G2 [12*n_lab][32]] (kStages tile sets per
+    //                        block)  [noise [22 | 32][128]][acc [25][128] (8-byte sums; double and F2 kernels only)]   (elements: Real)
+    static __host__ __device__ constexpr size_t warp_rows(int n_lab, int g0_rows) { return g0_rows + TMA_CH_G1 + 12 * n_lab; }
+    static __host__ __device__ constexpr size_t warp_bytes(int n_lab, int g0_rows) { return warp_rows(n_lab, g0_rows) * 32 * sizeof(Real); }
     static __host__ __device__ constexpr size_t off_in() { return 128; }
-    static __host__ __device__ constexpr size_t off_noise(int n_lab, int ref_rows) { return off_in() + kStages * warp_bytes(n_lab, ref_rows); }
-    static __host__ __device__ constexpr size_t off_acc(int n_lab, int ref_rows) { return off_noise(n_lab, ref_rows) + (size_t)kNoiseRows * kThreads * sizeof(Real); }
-    static __host__ __device__ constexpr size_t total(int n_lab, int ref_rows, bool acc_in_smem) {
-        return off_acc(n_lab, ref_rows) + (acc_in_smem ? (size_t)TMA_ACC_ROWS * kThreads * 8 : 0);
+    static __host__ __device__ constexpr size_t off_noise(int n_lab, int g0_rows) { return off_in() + kStages * warp_bytes(n_lab, g0_rows); }
+    static __host__ __device__ constexpr size_t off_acc(int n_lab, int g0_rows) { return off_noise(n_lab, g0_rows) + (size_t)kNoiseRows * kThreads * sizeof(Real); }
+    static __host__ __device__ constexpr size_t total(int n_lab, int g0_rows, bool acc_in_smem) {
+        return off_acc(n_lab, g0_rows) + (acc_in_smem ? (size_t)TMA_ACC_ROWS * kThreads * 8 : 0);
     }
 };
 
 // One elected thread (`lane` == 0 of the warp that is entitled to refill): arm the group's mbarrier with the byte count, then
-// issue the tile copies of step t.
-template <bool kMpc, typename Real>
-__device__ __forceinline__ void issue_g0(const TmaMaps &m, long long t, int s_warp, Real *g0w, Real *refw, uint64_t *bar, int lane) {
+// issue the tile copies of step t.  G0 = M [12] | p [12] (kOut == 2) | body_ref [3] (kMpc), rows of the block's tile.
+template <int kOut, bool kMpc, typename Real>
+__device__ __forceinline__ void issue_g0(const TmaMaps &m, long long t, int s_warp, Real *g0w, uint64_t *bar, int lane) {
     if (lane == 0) {
-        mbar_expect_tx(bar, (uint32_t)((TMA_CH_G0 + (kMpc ? TMA_CH_REF : 0)) * 32 * sizeof(Real)));
-        tma_tile_g2s(g0w, &m.p, s_warp, (int)(t * 12), bar);
-        tma_tile_g2s(g0w + 12 * 32, &m.f, s_warp, (int)(t * 12), bar);
-        if constexpr (kMpc) tma_tile_g2s(refw, &m.body_ref, s_warp, (int)(t * 12), bar);  // rows 0..2 of the step's 12
+        mbar_expect_tx(bar, (uint32_t)(tma_g0_rows<kOut, kMpc>() * 32 * sizeof(Real)));
+        tma_tile_g2s(g0w, &m.mom, s_warp, (int)(t * NM), bar);
+        if constexpr (kOut == 2) tma_tile_g2s(g0w + NM * 32, &m.p, s_warp, (int)(t * 12), bar);
+        if constexpr (kMpc) tma_tile_g2s(g0w + (tma_g0_rows<kOut, kMpc>() - TMA_CH_REF) * 32, &m.body_ref, s_warp, (int)(t * 12), bar);  // rows 0..2 of the step's 12
     }
 }
 template <typename Real>
@@ -196,15 +200,14 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
 
     uint64_t *bars = reinterpret_cast<uint64_t *>(smem_raw);  // full[G0], full[G1], full[G2]
     int *consumed = reinterpret_cast<int *>(smem_raw + 64);   // warps that have finished reading the current copy of G0, G1, G2
-    constexpr int kRefRows = kMpc ? TMA_CH_REF : 0;
+    constexpr int kG0Rows = tma_g0_rows<kOut, kMpc>();
     Real *g0w = reinterpret_cast<Real *>(smem_raw + Smem::off_in());
-    Real *g1w = g0w + TMA_CH_G0 * 32, *g2w = g1w + TMA_CH_G1 * 32;  // the block's [C][32] tiles (of Real)
-    Real *refw = g2w + 12 * n_lab * 32;                              // reference body angles (kMpc), fetched with G0
-    Real *noise = reinterpret_cast<Real *>(smem_raw + Smem::off_noise(n_lab, kRefRows));
-    AccT *acc_s = reinterpret_cast<AccT *>(smem_raw + Smem::off_acc(n_lab, kRefRows)) + tid;
+    Real *g1w = g0w + kG0Rows * 32, *g2w = g1w + TMA_CH_G1 * 32;  // the block's [C][32] tiles (of Real)
+    Real *noise = reinterpret_cast<Real *>(smem_raw + Smem::off_noise(n_lab, kG0Rows));
+    AccT *acc_s = reinterpret_cast<AccT *>(smem_raw + Smem::off_acc(n_lab, kG0Rows)) + tid;
 
     if (grp_j * TMA_WARPS * S + tile_k * TW >= N) return;  // the whole block lies beyond the last trajectory (fewer trajectories than streams)
-    const int tile_elems = (int)Smem::warp_rows(n_lab, kRefRows) * 32;  // elements of one tile set
+    const int tile_elems = (int)Smem::warp_rows(n_lab, kG0Rows) * 32;  // elements of one tile set
     if (tid == 0) {
 #pragma unroll
         for (int b = 0; b < 3 * kStages; ++b) mbar_init(&bars[b], 1);  // full[G0], full[G1], full[G2] of every tile set
@@ -217,7 +220,7 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
 #pragma unroll
         for (int sg = 0; sg < kStages; ++sg) {
             if (sg < prm.T) {
-                issue_g0<kMpc>(maps, sg, s_warp, g0w + sg * tile_elems, refw + sg * tile_elems, &bars[3 * sg], lane);
+                issue_g0<kOut, kMpc>(maps, sg, s_warp, g0w + sg * tile_elems, &bars[3 * sg], lane);
                 issue_g1(maps, sg, s_warp, g1w + sg * tile_elems, &bars[3 * sg + 1], lane);
                 if (n_lab) issue_g2(maps, sg, s_warp, n_lab, g2w + sg * tile_elems, &bars[3 * sg + 2], lane);
             }
@@ -294,7 +297,7 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
         }
     }
 
-    // label tiles of this lane; a label stream that was not given reads the (always valid) feet tile and is ignored
+    // label tiles of this lane; a label stream that was not given reads the (always valid) moments tile and is ignored
     const Real *lab_truth = (kSummary && prm.truth) ? g2w + lane : g0w + lane;
     const Real *lab_nominal = (kSummary && prm.nominal) ? g2w + (prm.truth ? 12 * 32 : 0) + lane : g0w + lane;
     // labels and running sums are fetched six at a time BEFORE they are used, so the shared-memory latency of one batch
@@ -335,24 +338,27 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
         const uint32_t par = kStages == 2 ? (uint32_t)((t >> 1) & 1) : (uint32_t)(t & 1);
         const bool more = t + kStages < prm.T;
         uint64_t *bar = bars + (kStages == 2 ? 3 * (int)(t & 1) : 0);
-        Real *g0 = g0w + stg, *g1 = g1w + stg, *g2 = g2w + stg, *rf = refw + stg;
+        Real *g0 = g0w + stg, *g1 = g1w + stg, *g2 = g2w + stg;
 
-        // ---- G0: feet and forces -> mean model --------------------------------------------------------------
+        // ---- G0: leg moments -> mean model ------------------------------------------------------------------
         mbar_wait(&bar[0], par);
-        propagate_mean_with_R<32>(prm, x, g0 + lane, g0 + 12 * 32 + lane, Rm, any_trunc,
-                              (kOut == 2 && active) ? prm.p_world_steps : nullptr, (t * 12) * N + i, N);
+        if constexpr (kOut == 2) {
+            if (active && prm.p_world_steps) store_world_feet<32>(g0 + NM * 32 + lane, Rm, prm.p_world_steps, (t * 12) * N + i, N);
+        }
+        propagate_mean_from_moments<32>(prm, x, g0 + lane, Rm, any_trunc);
         Real E[kMpc ? 9 : 1];  // D[a][6 + k] = exp(dt Rb^T[a][k]) - 1 of the predict_mpc transition (kalman_filter.py:153-157)
         if constexpr (kMpc) {
             Real Rb[9];
-            rot_zyx(rf[lane], rf[32 + lane], rf[64 + lane], Rb);
+            const Real *rf = g0 + (kG0Rows - TMA_CH_REF) * 32 + lane;
+            rot_zyx(rf[0], rf[32], rf[64], Rb);
 #pragma unroll
             for (int a = 0; a < 3; ++a)
 #pragma unroll
                 for (int k = 0; k < 3; ++k) E[3 * a + k] = exp_minus_one(Real(prm.dt) * Rb[3 * k + a]);
         }
-        {  // this warp has consumed the step's feet and forces: the last one refills G0 for step t + 1
+        {  // this warp has consumed the step's moments: the last one refills G0 for step t + 1
             const int elect = last_reader(0);
-            if (more) issue_g0<kMpc>(maps, t + kStages, s_warp, g0, rf, &bar[0], elect);
+            if (more) issue_g0<kOut, kMpc>(maps, t + kStages, s_warp, g0, &bar[0], elect);
         }
         if constexpr (kOut == 2) {
             if (active && prm.x_model_steps) {

@@ -48,14 +48,14 @@ int launch_seq_tma_k(const Params<typename Lanes<Real>::scalar> &p, cudaStream_t
     TmaMaps maps;
     std::memset(&maps, 0, sizeof maps);
     const int bw = 32 * L;
-    bool ok = make_map(&maps.p, p.p, p.T, 12, p.S, bw, 12) && make_map(&maps.f, p.f, p.T, 12, p.S, bw, 12) &&
-              make_map(&maps.z, p.z_in, p.T, 10, p.S, bw, 10);
+    bool ok = make_map(&maps.mom, p.mom, p.T, NM, p.S, bw, NM) && make_map(&maps.z, p.z_in, p.T, 10, p.S, bw, 10);
+    if (ok && kOut == 2) ok = make_map(&maps.p, p.p, p.T, 12, p.S, bw, 12);
     if (ok && kMpc) ok = make_map(&maps.body_ref, p.body_ref, p.T, 12, p.S, bw, 3);
     if (ok && n_lab >= 1) ok = make_map(&maps.lab0, p.truth ? p.truth : p.nominal, p.T, 12, p.S, bw, 12);
     if (ok && n_lab >= 2) ok = make_map(&maps.lab1, p.nominal, p.T, 12, p.S, bw, 12);
     if (!ok) return 1;
     constexpr int kWarps = kW ? kW : tma_warps<kBlock>(), kThreads = 32 * kWarps;
-    const size_t smem = TmaSmem<Real, kThreads, tma_noise_rows<kOut>(), tma_stages<kW>()>::total(n_lab, kMpc ? TMA_CH_REF : 0, kW == 1 ? false : tma_acc_in_smem<Real, kSummary, kBlock>());
+    const size_t smem = TmaSmem<Real, kThreads, tma_noise_rows<kOut>(), tma_stages<kW>()>::total(n_lab, tma_g0_rows<kOut, kMpc>(), kW == 1 ? false : tma_acc_in_smem<Real, kSummary, kBlock>());
     auto kern = kf_seq_tma_kernel<Real, kSummary, kOut, kMpc, kBlock, kW>;
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return OPTI_KF_E_CUDA;
     // one block per (stream tile, group of kWarps members): see the index mapping at the top of the kernel

@@ -55,7 +55,6 @@ class KfHostPipeline:
         self.n_traj, self.n_steps, self.n_streams, self.dtype = n_traj, n_steps, n_streams, dtype
         self.labels, self.stream_offset, self.n_slots = tuple(labels), int(stream_offset), n_slots
         self.structure = structure
-        esz = 8 if dtype == torch.float64 else 4
         names = ["imu", "p", "dp", "contact", "f", *self.labels]
         self.group, self.world, self.rank = shared_streams_group, 1, 0
         if shared_streams_group is not None:
@@ -73,8 +72,8 @@ class KfHostPipeline:
             dev["Q"] = torch.empty((12, n_traj), dtype=dtype, device=self.device)
             dev["R"] = torch.empty((10, n_traj), dtype=dtype, device=self.device)
             out = {"summary": torch.empty((nv.SUMMARY_ROWS, n_traj), dtype=dtype, device=self.device),
-                   "status": torch.zeros(n_traj, dtype=torch.int32, device=self.device),
-                   "workspace": torch.empty(n_steps * 10 * n_streams * esz + 4 * n_streams + 4096, dtype=torch.uint8, device=self.device)}
+                   "status": torch.zeros(n_traj, dtype=torch.int32, device=self.device)}
+            # "workspace" is added by the slot's first kf_batch call, at the size the library asks for
             host = torch.empty((nv.SUMMARY_ROWS, n_traj), dtype=dtype).pin_memory()
             self.slots.append({"dev": dev, "flat": flat, "out": out, "host": host, "ev_in": torch.cuda.Event(), "ev_k": torch.cuda.Event(),
                                "ev_out": torch.cuda.Event(), "busy": False})
