@@ -14,6 +14,9 @@
  *                           kalman_filter.py:153-161) make.
  *   optistate_kf_measure    replaces get_odom + set_measurements (kalman_filter.py:79-117) for S streams x T steps.
  *   optistate_fma_peak      measures the FP64 / FP32 FMA issue peak of the device (roofline denominator).
+ *   optistate_kf_smooth     runs optistate_kf_batch and then the fixed-interval Rauch-Tung-Striebel smoother backwards over
+ *                           its per-step estimates (optistate_kf_smooth_storage_bytes sizes its scratch).  The reference
+ *                           has no smoother: this entry point has no reference counterpart.
  *
  * Conventions
  *   - plain C, no torch / C++ types; every pointer is a NON-OWNING DEVICE pointer unless stated otherwise;
@@ -99,8 +102,10 @@ enum {
     OPTI_KF_ST_ALL_SWING = 4,  /* a step had sum(contact) == 0 (reference raises ValueError, kalman_filter.py:97-103);
                                   the odometry part of z is set to 0 for that step                              */
     OPTI_KF_ST_ASYMMETRIC = 8, /* JOINT: S was visibly asymmetric: pivoted inverse instead of the Cholesky solve */
-    OPTI_KF_ST_SINGULAR = 16   /* JOINT: the pivoted inverse of S met a zero pivot - where the reference's np.linalg.inv raises
+    OPTI_KF_ST_SINGULAR = 16,  /* JOINT: the pivoted inverse of S met a zero pivot - where the reference's np.linalg.inv raises
                                   LinAlgError (kalman_filter.py:168); an indefinite but regular S does not set it       */
+    OPTI_KF_ST_SMOOTH_NOT_PD = 32 /* optistate_kf_smooth: a pivot of a prior covariance P-_{t+1} was <= 0 or not finite; the
+                                     backward recursion carries on with that pivot                                    */
 };
 
 /* error codes */
@@ -311,6 +316,26 @@ typedef struct OptiKfClosedLoopDesc {
 } OptiKfClosedLoopDesc;
 size_t optistate_kf_closed_loop_workspace_bytes(int64_t n_traj, int64_t n_steps);
 int optistate_kf_closed_loop(const OptiKfClosedLoopDesc *desc, void *cuda_stream);
+
+/* ---- fixed-interval Rauch-Tung-Striebel smoother (offline: every measurement of the recording is known).  Runs the forward
+ * pass exactly as optistate_kf_batch runs `filter` (its outputs, summary, status and workspace included), keeping the packed
+ * posterior covariance of every step in `storage`, then a backward kernel, one thread per trajectory:
+ *     G_t = P+_t F_{t+1}^T (P-_{t+1})^-1,  xs_t = x+_t + G_t (xs_{t+1} - x-_{t+1}),  Ps_t = P+_t + G_t (Ps_{t+1} - P-_{t+1}) G_t^T
+ * from xs_{T-1} = x+_{T-1}, Ps_{T-1} = P+_{T-1}, with F_{t+1} the covariance transition of the filter's own predict (F[0:3,6:9] =
+ * R(x+_t)^T).  SEQUENTIAL algo, predict() covariance model, diagonal Q and R, and a P0 without cross-group entries only (see the
+ * flags above): anything else returns OPTI_KF_E_UNSUPPORTED.  status[i] gains OPTI_KF_ST_SMOOTH_NOT_PD. ---- */
+typedef struct OptiKfSmoothDesc {
+    uint32_t struct_size;       /* sizeof(OptiKfSmoothDesc) */
+    uint32_t abi_version;       /* OPTISTATE_KF_ABI_VERSION */
+    const OptiKfDesc *filter;   /* the forward pass (host pointer to its descriptor) */
+    void *x_smooth;             /* [T][12][N] required: smoothed state */
+    void *var_smooth;           /* [T][12][N] optional: diagonal of the smoothed covariance */
+    void *storage;              /* device scratch of optistate_kf_smooth_storage_bytes(filter): packed P+ [T][30][N], plus x+ and x-
+                                   [T][12][N] each unless filter->x_steps / filter->x_model_steps are given (they are read there) */
+    size_t storage_bytes;
+} OptiKfSmoothDesc;
+int optistate_kf_smooth_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out);
+int optistate_kf_smooth(const OptiKfSmoothDesc *desc, void *cuda_stream);
 
 /* Runs the filter; dtype taken from the descriptor. */
 int optistate_kf_batch(const OptiKfDesc *desc, void *cuda_stream);

@@ -3,7 +3,8 @@
     from optistate_b200 import Kalman_Filter, kf_batch
 
 `Kalman_Filter` is the drop-in for the reference class (same constructor / predict / update surface);
-`kf_batch` filters thousands to millions of independent trajectories in one kernel launch.
+`kf_batch` filters thousands to millions of independent trajectories in one kernel launch;
+`kf_smooth` adds the fixed-interval (Rauch-Tung-Striebel) smoother for offline recordings.
 Both call the CUDA library liboptistate_kf.so (C ABI: include/optistate_kf.h) through a thin PyTorch C++
 extension.  There is no CPU fallback: without the built extension and a CUDA device the calls raise.
 """
@@ -12,7 +13,7 @@ from .settings import INITIAL_PARAMS  # noqa: F401
 
 def __getattr__(name):
     # torch and the native extension are imported on first use so that `import optistate_b200` stays cheap
-    if name in ("kf_batch", "kf_measure", "fma_peak", "KfBatchResult", "SUMMARY_FIELDS"):
+    if name in ("kf_batch", "kf_smooth", "kf_measure", "fma_peak", "KfBatchResult", "SUMMARY_FIELDS"):
         from . import batch
 
         return getattr(batch, name)

@@ -14,7 +14,7 @@ ALGO_AUTO, ALGO_JOINT, ALGO_SEQUENTIAL = 0, 1, 2
 COV_PREDICT, COV_MPC = 0, 1
 PHASE_MEASURE, PHASE_PREDICT, PHASE_UPDATE, PHASE_ALL = 1, 2, 4, 7
 MAT_NONE, MAT_DIAG, MAT_DIAG_PER, MAT_DENSE, MAT_DENSE_PER = 0, 1, 2, 3, 4
-ST_NOT_PD, ST_NONFINITE, ST_ALL_SWING, ST_ASYMMETRIC, ST_SINGULAR = 1, 2, 4, 8, 16
+ST_NOT_PD, ST_NONFINITE, ST_ALL_SWING, ST_ASYMMETRIC, ST_SINGULAR, ST_SMOOTH_NOT_PD = 1, 2, 4, 8, 16, 32
 FLAG_P0_DECOUPLED, FLAG_FULL_COVARIANCE, FLAG_SCALAR_FP32 = 1, 2, 4
 ABI_VERSION = 5
 SUMMARY_ROWS = 52

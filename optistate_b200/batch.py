@@ -160,6 +160,55 @@ def kf_batch(
     stores); `result.summary` is the local column block, `summary_peers.tensor` the gathered array once
     `summary_peers.wait()` has run.
     """
+    call = _filter_call(imu, p, dp, contact, f, x0, P0, Q, R, n_traj=n_traj, dtype=dtype, stream_index=stream_index,
+                        stream_offset=stream_offset, outputs=outputs, ckpt_every=ckpt_every, truth=truth, nominal=nominal,
+                        body_ref=body_ref, z=z, algo=algo, cov_model=cov_model, q_kind=q_kind, r_kind=r_kind, p0_kind=p0_kind, dt=dt,
+                        mass=mass, inertia=inertia, gravity=gravity, device=device, out=out, summary_peers=summary_peers,
+                        p0_is_symmetric=p0_is_symmetric, structure=structure, packed=packed)
+    with torch.cuda.device(call.device):
+        _attach_workspace(call, out)
+        nv.check(int(call.ext.kf_batch(call.cfg, call.consts, call.tensors)), "optistate_kf_batch")
+    return call.result(summary_peers)
+
+
+@dataclass
+class _FilterCall:
+    """The prepared arguments of one filter run (kf_batch, and the forward pass of kf_smooth)."""
+    ext: object
+    device: torch.device
+    cfg: dict
+    consts: dict
+    tensors: Dict[str, torch.Tensor]
+    want: list
+    status: torch.Tensor
+    n_traj: int
+    n_steps: int
+
+    def result(self, summary_peers=None, extra=()) -> KfBatchResult:
+        res = {k: self.tensors[k] for k in (*self.want, *extra)}
+        if summary_peers is not None and "summary" in res:
+            res["summary"] = summary_peers.local
+        return KfBatchResult(algo=_ALGO_NAMES[self.cfg["algo"]], n_traj=self.n_traj, n_steps=self.n_steps, tensors=res, status=self.status)
+
+
+def _attach_workspace(call: _FilterCall, out):
+    """Scratch for the streamed SEQUENTIAL path (measurement pre-pass + TMA-fed kernel); 0 bytes when unused."""
+    ws_bytes = call.ext.kf_batch(dict(call.cfg, query_workspace=1), call.consts, call.tensors)
+    if ws_bytes < 0:
+        nv.check(int(ws_bytes), "optistate_kf_workspace_bytes")
+    if ws_bytes > 0:
+        ws = out.get("workspace") if out is not None else None
+        if ws is None or ws.numel() < ws_bytes:
+            ws = torch.empty(int(ws_bytes), dtype=torch.uint8, device=call.device)
+            if out is not None:
+                out["workspace"] = ws  # kept for the caller's next call with the same shapes
+        call.tensors["workspace"] = ws
+
+
+def _filter_call(imu, p, dp, contact, f, x0, P0, Q, R, *, n_traj, dtype, stream_index, stream_offset, outputs, ckpt_every, truth,
+                 nominal, body_ref, z, algo, cov_model, q_kind, r_kind, p0_kind, dt, mass, inertia, gravity, device, out, summary_peers,
+                 p0_is_symmetric, structure, packed) -> _FilterCall:
+    """kf_batch's argument handling: inputs to the device, noise kinds, output tensors, the resolved algo."""
     nv.require_cuda()
     ext = nv.ext()
     device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
@@ -244,23 +293,73 @@ def kf_batch(
     inertia = np.diag(INITIAL_PARAMS.INERTIA_ROT) if inertia is None else np.asarray(inertia, float).reshape(3)
     consts = dict(dt=float(dt), mass=float(mass), inertia0=float(inertia[0]), inertia1=float(inertia[1]),
                   inertia2=float(inertia[2]), gravity=float(gravity))
-    with torch.cuda.device(device):
-        # scratch for the streamed SEQUENTIAL path (measurement pre-pass + TMA-fed kernel); 0 bytes when unused
-        ws_bytes = ext.kf_batch(dict(cfg, query_workspace=1), consts, tensors)
-        if ws_bytes < 0:
-            nv.check(int(ws_bytes), "optistate_kf_workspace_bytes")
-        if ws_bytes > 0:
-            ws = out.get("workspace") if out is not None else None
-            if ws is None or ws.numel() < ws_bytes:
-                ws = torch.empty(int(ws_bytes), dtype=torch.uint8, device=device)
-                if out is not None:
-                    out["workspace"] = ws  # kept for the caller's next call with the same shapes
-            tensors["workspace"] = ws
-        nv.check(int(ext.kf_batch(cfg, consts, tensors)), "optistate_kf_batch")
-    res = {k: tensors[k] for k in want}
-    if summary_peers is not None and "summary" in res:
-        res["summary"] = summary_peers.local
-    return KfBatchResult(algo=_ALGO_NAMES[cfg["algo"]], n_traj=N, n_steps=T, tensors=res, status=status)
+    return _FilterCall(ext=ext, device=device, cfg=cfg, consts=consts, tensors=tensors, want=want, status=status, n_traj=N, n_steps=T)
+
+
+_SMOOTH_OUTPUTS = ("x_smooth", "var_smooth")
+
+
+def kf_smooth(
+    imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *,
+    n_traj: Optional[int] = None, dtype: torch.dtype = torch.float64, stream_index=None, stream_offset: int = 0,
+    outputs: Iterable[str] = ("x_smooth",), ckpt_every: int = 0, truth=None, nominal=None, body_ref=None, z=None,
+    algo: str = "auto", cov_model: str = "predict", q_kind=None, r_kind=None, p0_kind=None,
+    dt: float = INITIAL_PARAMS.DT_mpc, mass: float = INITIAL_PARAMS.ROBOT_MASS, inertia=None,
+    gravity: float = INITIAL_PARAMS.GRAVITY, device=None, out: Optional[Dict[str, torch.Tensor]] = None,
+    summary_peers=None, p0_is_symmetric: Optional[bool] = None, structure: str = "auto", packed: bool = True,
+) -> KfBatchResult:
+    """Fixed-interval Rauch-Tung-Striebel smoother: runs the filter exactly as kf_batch runs it with the same arguments, then a
+    backward kernel that conditions every step's estimate on ALL measurements of the recording (offline use).
+
+    outputs: x_smooth [T,12,N] (smoothed state, the default), var_smooth [T,12,N] (diagonal of the smoothed covariance), and any
+    kf_batch output - those come from the same forward pass.  out: as for kf_batch, plus "smooth_storage" (uint8 scratch of
+    optistate_kf_smooth_storage_bytes: the packed posterior covariance of every step, 240 B per trajectory-step in FP64, and the
+    filter's x_steps / x_model_steps when they are not outputs), replaced in `out` when missing or too small.
+    Supported: the sequential algo with the predict() covariance model, diagonal Q and R and a P0 without entries across the
+    groups {th, w}, {x, vx}, {y, vy}, {z, vz}; anything else raises ValueError.  status gains OPTI_KF_ST_SMOOTH_NOT_PD (32).
+    """
+    if cov_model != "predict":
+        raise ValueError("kf_smooth supports the predict() covariance model only (predict_mpc makes F_d dense)")
+    if structure != "auto":
+        raise ValueError("kf_smooth needs the decoupled-group form of P; structure='full' keeps cross-group entries")
+    if algo == "joint":
+        raise ValueError("kf_smooth runs on the sequential filter; algo='joint' is not supported")
+    outputs = list(outputs)
+    smooth_want = [o for o in outputs if o in _SMOOTH_OUTPUTS]
+    if "x_smooth" not in smooth_want:
+        smooth_want.insert(0, "x_smooth")
+    call = _filter_call(imu, p, dp, contact, f, x0, P0, Q, R, n_traj=n_traj, dtype=dtype, stream_index=stream_index,
+                        stream_offset=stream_offset, outputs=[o for o in outputs if o not in _SMOOTH_OUTPUTS], ckpt_every=ckpt_every,
+                        truth=truth, nominal=nominal, body_ref=body_ref, z=z, algo="sequential" if algo == "auto" else algo,
+                        cov_model=cov_model, q_kind=q_kind, r_kind=r_kind, p0_kind=p0_kind, dt=dt, mass=mass, inertia=inertia,
+                        gravity=gravity, device=device, out=out, summary_peers=summary_peers, p0_is_symmetric=p0_is_symmetric,
+                        structure=structure, packed=packed)
+    cfg = call.cfg
+    if cfg["q_kind"] not in (nv.MAT_DIAG, nv.MAT_DIAG_PER) or cfg["r_kind"] not in (nv.MAT_DIAG, nv.MAT_DIAG_PER):
+        raise ValueError("kf_smooth needs diagonal Q and R (dense noise couples the decoupled groups)")
+    if cfg["p0_kind"] in (nv.MAT_DENSE, nv.MAT_DENSE_PER) and not cfg["flags"] & nv.FLAG_P0_DECOUPLED:
+        raise ValueError("kf_smooth needs a P0 without entries across the groups {th, w}, {x, vx}, {y, vy}, {z, vz}")
+    T, N = call.n_steps, call.n_traj
+    for o in smooth_want:
+        shape = (T, 12, N)
+        if out is not None and o in out:
+            if tuple(out[o].shape) != shape or out[o].dtype != dtype:
+                raise ValueError(f"out['{o}'] must be {shape} {dtype}")
+            call.tensors[o] = out[o]
+        else:
+            call.tensors[o] = torch.empty(shape, dtype=dtype, device=call.device)
+    with torch.cuda.device(call.device):
+        _attach_workspace(call, out)
+        st_bytes = call.ext.kf_smooth(dict(cfg, query_storage=1), call.consts, call.tensors)
+        nv.check(int(min(st_bytes, 0)), "optistate_kf_smooth_storage_bytes")
+        st = out.get("smooth_storage") if out is not None else None
+        if st is None or st.numel() < st_bytes:
+            st = torch.empty(max(int(st_bytes), 1), dtype=torch.uint8, device=call.device)
+            if out is not None:
+                out["smooth_storage"] = st  # kept for the caller's next call with the same shapes
+        call.tensors["smooth_storage"] = st
+        nv.check(int(call.ext.kf_smooth(cfg, call.consts, call.tensors)), "optistate_kf_smooth")
+    return call.result(summary_peers, extra=smooth_want)
 
 
 def kf_measure(imu, p, dp, contact, *, dtype: torch.dtype = torch.float64, device=None, want_odom: bool = False):

@@ -10,6 +10,7 @@
 #include "kf_launch.cuh"
 #include "kf_mpc_params.cuh"
 #include "kf_seq_core.cuh"
+#include "kf_smooth.cuh"
 
 namespace {
 
@@ -166,10 +167,12 @@ int launch_streamed<float>(const OptiKfDesc *d, const okf::Params<float> &p, cud
     return packed_pair_ok(d) ? launch_streamed_t<okf::F2>(d, p, stream) : launch_streamed_t<float>(d, p, stream);
 }
 
+// P_steps: the smoother's packed per-step posterior covariance [T][30][N] (optistate_kf_smooth only; decoupled form)
 template <typename Real>
-int launch(const OptiKfDesc *d, int algo, cudaStream_t stream) {
+int launch(const OptiKfDesc *d, int algo, cudaStream_t stream, void *P_steps = nullptr) {
     if (d->n_traj == 0) return OPTI_KF_OK;
     okf::Params<Real> p = make_params<Real>(d);
+    p.P_steps = (Real *)P_steps;
     cudaGetLastError();
     if ((d->flags & OPTI_KF_FLAG_STATUS_ACCUMULATE) && d->status) {
         // the kernels OR stream_status[stream of i] into what they write: with one stream per trajectory that is the old status
@@ -313,6 +316,56 @@ int fma_peak(long long fma_per_thread, double *flops_out, double *seconds_out, c
     return OPTI_KF_OK;
 }
 
+// ---- fixed-interval smoother ------------------------------------------------------------------------------------
+// What the backward kernel can take: the decoupled-group form of the SEQUENTIAL filter (kf_smooth.cuh).
+int smooth_check(const OptiKfDesc *d) {
+    const int rc = validate(d);
+    if (rc != OPTI_KF_OK) return rc;
+    if (d->cov_model != OPTI_KF_COV_PREDICT || (d->flags & OPTI_KF_FLAG_FULL_COVARIANCE)) return OPTI_KF_E_UNSUPPORTED;
+    if (!is_diag_kind(d->q_kind) || !is_diag_kind(d->r_kind)) return OPTI_KF_E_UNSUPPORTED;
+    const bool p0_groups = d->p0_kind == OPTI_KF_MAT_NONE || is_diag_kind(d->p0_kind) || (d->flags & OPTI_KF_FLAG_P0_DECOUPLED);
+    if (!p0_groups) return OPTI_KF_E_UNSUPPORTED;
+    const int algo = resolve(d);
+    if (algo < 0) return algo;
+    return algo == OPTI_KF_ALGO_SEQUENTIAL ? OPTI_KF_OK : OPTI_KF_E_UNSUPPORTED;
+}
+
+// Scratch of the smoother, each part padded to 256 bytes: packed P+ [T][30][N] at 0, then x+ and x- [T][12][N] unless the
+// filter descriptor has x_steps / x_model_steps (the smoother reads those).  Byte offsets.
+struct SmoothStorage {
+    size_t x_post, x_prior, total;
+    explicit SmoothStorage(const OptiKfDesc *d) {
+        const auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+        const size_t esz = d->dtype == OPTI_KF_F64 ? 8 : 4, tn = (size_t)d->n_steps * (size_t)d->n_traj;
+        x_post = up(tn * okf::NPB * esz);
+        x_prior = x_post + (d->x_steps ? 0 : up(tn * okf::NX * esz));
+        total = x_prior + (d->x_model_steps ? 0 : up(tn * okf::NX * esz));
+    }
+};
+
+template <typename Real>
+int smooth(const OptiKfSmoothDesc *s, cudaStream_t stream) {
+    const OptiKfDesc *f = s->filter;
+    const SmoothStorage ss(f);
+    unsigned char *base = (unsigned char *)s->storage;
+    OptiKfDesc fw = *f;  // the forward pass, with x+ / x- in the storage where the caller did not ask for them
+    if (!fw.x_steps && base) fw.x_steps = base + ss.x_post;
+    if (!fw.x_model_steps && base) fw.x_model_steps = base + ss.x_prior;
+    int rc = launch<Real>(&fw, OPTI_KF_ALGO_SEQUENTIAL, stream, base);
+    if (rc != OPTI_KF_OK) return rc;
+    if (f->n_traj == 0 || f->n_steps == 0) return OPTI_KF_OK;
+    okf::SmoothParams<Real> p;
+    std::memset(&p, 0, sizeof p);
+    p.N = f->n_traj; p.T = f->n_steps; p.dt = (Real)f->dt;
+    p.Q = (const Real *)f->Q; p.q_kind = f->q_kind;
+    p.x_post = (const Real *)fw.x_steps; p.x_prior = (const Real *)fw.x_model_steps; p.P_post = (const Real *)base;
+    p.x_smooth = (Real *)s->x_smooth; p.var_smooth = (Real *)s->var_smooth; p.status = f->status;
+    rc = okf::launch_rts<Real>(p, stream);
+    if (rc < 0) return rc;
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return cudaGetLastError() == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
+}
+
 template <typename Real>
 int identify_noise(const OptiKfIdentifyDesc *d, cudaStream_t stream) {
     okf::Params<Real> p;
@@ -355,6 +408,29 @@ int optistate_kf_workspace_bytes(const OptiKfDesc *desc, size_t *bytes_out) {
     if (algo < 0) return algo;
     *bytes_out = (algo == OPTI_KF_ALGO_SEQUENTIAL && tma_layout_ok(desc)) ? SeqWorkspace(desc).total : 0;
     return OPTI_KF_OK;
+}
+
+int optistate_kf_smooth_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out) {
+    const int rc = smooth_check(filter);
+    if (rc != OPTI_KF_OK) return rc;
+    if (!bytes_out) return OPTI_KF_E_NULL;
+    *bytes_out = SmoothStorage(filter).total;
+    return OPTI_KF_OK;
+}
+
+int optistate_kf_smooth(const OptiKfSmoothDesc *desc, void *cuda_stream) {
+    if (!desc) return OPTI_KF_E_NULL;
+    if (desc->struct_size != sizeof(OptiKfSmoothDesc) || desc->abi_version != OPTISTATE_KF_ABI_VERSION) return OPTI_KF_E_VERSION;
+    if (!desc->filter) return OPTI_KF_E_NULL;
+    const int rc = smooth_check(desc->filter);
+    if (rc != OPTI_KF_OK) return rc;
+    const OptiKfDesc *f = desc->filter;
+    const bool steps = f->n_traj > 0 && f->n_steps > 0;  // empty batches carry empty (NULL) arrays
+    if (steps && !desc->x_smooth) return OPTI_KF_E_NULL;
+    if (desc->storage_bytes < SmoothStorage(f).total) return OPTI_KF_E_SHAPE;
+    if (steps && !desc->storage) return OPTI_KF_E_NULL;
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    return f->dtype == OPTI_KF_F64 ? smooth<double>(desc, stream) : smooth<float>(desc, stream);
 }
 
 int optistate_kf_batch(const OptiKfDesc *desc, void *cuda_stream) {

@@ -39,6 +39,9 @@ struct Params {
     long long summary_ld;
     int n_summary_peers;
     Real *summary_peers[OPTI_KF_MAX_PEERS];
+    // [T][30][N] posterior covariance of every step, decoupled-group entries only (pk_slot, kf_seq_core.cuh); set by the
+    // smoother's forward pass alone.  Last, so that every other field keeps its constant-bank offset.
+    Real *P_steps;
 };
 
 // One summary value of trajectory i (or of the pair i, i+1 for the packed FP32 type): local copy plus every peer copy.

@@ -36,6 +36,37 @@ __host__ __device__ constexpr int grp(int i) { return (i < 3 || (i >= 6 && i < 9
 template <bool kBlock>
 __host__ __device__ constexpr bool cpl(int i, int j) { return !kBlock || grp(i) == grp(j); }
 
+// Packed per-step posterior covariance of the decoupled form (Params.P_steps, read by the smoother, kf_smooth.cuh): the 30
+// entries (a, b) with b <= a and cpl<true>(a, b), in tri(a, b) order.  pk_slot is the one map the store and the load use.
+constexpr int NPB = 30;
+// Closed form (straight arithmetic, so it folds to a constant in the unrolled loops that use it): rows 0-2 hold 1, 2, 3 entries,
+// rows 3-5 one (the diagonal), rows 6-8 4, 5, 6 (the attitude columns and their own), rows 9-11 two (position, diagonal).
+__host__ __device__ constexpr int pk_row_start(int a) {
+    return a < 3 ? a * (a + 1) / 2 : a < 6 ? 3 + a : a < 9 ? 9 + 4 * (a - 6) + (a - 6) * (a - 7) / 2 : 24 + 2 * (a - 9);
+}
+__host__ __device__ constexpr int pk_slot(int a, int b) {
+    return pk_row_start(a) + (grp(a) == 0 ? (b < 3 ? b : b - 3) : (b == a && a >= 9 ? 1 : 0));
+}
+// the same map by enumeration, checked against the closed form at compile time
+__host__ __device__ constexpr bool pk_slot_ok() {
+    int n = 0;
+    for (int i = 0; i < 12; ++i)
+        for (int j = 0; j <= i; ++j)
+            if (cpl<true>(i, j) && pk_slot(i, j) != n++) return false;
+    return n == NPB;
+}
+static_assert(pk_slot_ok(), "pk_slot enumerates the 30 coupled entries in tri order");
+
+// P's coupled entries of step t to dst[t][pk_slot][N] (Scalar = the array type, Real = double | float | F2)
+template <typename Real, typename Scalar>
+__device__ __forceinline__ void store_packed_P(Scalar *dst, long long t, long long N, long long i, const Real (&P)[NP]) {
+#pragma unroll
+    for (int a = 0; a < NX; ++a)
+#pragma unroll
+        for (int b = 0; b <= a; ++b)
+            if (cpl<true>(a, b)) st_traj(dst, (t * NPB + pk_slot(a, b)) * N + i, P[tri(a, b)]);
+}
+
 // P <- F_d P F_d^T + diag(q), F_d = I + dt N, N[a,c] = R^T, N[b,d] = I   (blocks a=0..2 b=3..5 c=6..8 d=9..11)
 // Written with explicit fma_ so that double, float and the packed F2 type run the same operation sequence.
 template <bool kBlock = false, typename Real, typename Scalar>

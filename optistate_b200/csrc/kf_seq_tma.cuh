@@ -138,7 +138,7 @@ __device__ __forceinline__ void issue_g2(const TmaMaps &m, long long t, int s_wa
 
 // kOut: which per-step outputs the instantiation can write.  0 = none; 1 = the estimates (x_steps, p_trace_steps,
 // k_gain_steps, nis_steps - what the reference driver records every step); 2 = also the rarely wanted ones
-// (x_model_steps, p_world_steps, z_steps, P_ckpt).  Blocks of outputs that are not wanted are compiled out instead of being
+// (x_model_steps, p_world_steps, z_steps, P_ckpt, and the smoother's P_steps).  Blocks of outputs that are not wanted are compiled out instead of being
 // jumped over every step: the taken branches across them cost the lone warp of a scheduler ~10 % of its time in
 // instruction-fetch bubbles (ncu: stall_no_inst / stall_branch_resolving at the branch targets of the 35 KB loop body).
 // kBlock: the decoupled-group form of the covariance recursion (kf_seq_core.cuh): 30 live scalars of P instead of 78, which
@@ -436,6 +436,9 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
                         for (int a = 0; a < NX; ++a)
 #pragma unroll
                             for (int b = 0; b < NX; ++b) st_traj(prm.P_ckpt, base + (long long)(a * NX + b) * N, cpl<kBlock>(a, b) ? P[tri(a, b)] : Real(0));
+                    }
+                    if constexpr (kBlock) {
+                        if (prm.P_steps) store_packed_P(prm.P_steps, t, N, i, P);
                     }
                 }
             }

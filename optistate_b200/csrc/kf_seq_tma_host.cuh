@@ -70,7 +70,7 @@ int launch_seq_tma_k(const Params<typename Lanes<Real>::scalar> &p, cudaStream_t
 // (see kf_seq_tma.cuh); kBlock is chosen by the caller from Params.block and never combines with the predict_mpc model
 template <typename Real, bool kSummary, bool kBlock>
 int launch_seq_tma(const Params<typename Lanes<Real>::scalar> &p, cudaStream_t stream) {
-    const bool rare = p.x_model_steps || p.p_world_steps || p.z_steps || p.P_ckpt;
+    const bool rare = p.x_model_steps || p.p_world_steps || p.z_steps || p.P_ckpt || p.P_steps;
     const bool estimates = p.x_steps || p.p_trace_steps || p.k_gain_steps || p.nis_steps;
     const int out = rare ? 2 : (estimates ? 1 : 0);
     const bool mpc = p.cov_model == OPTI_KF_COV_MPC;
@@ -97,7 +97,7 @@ int launch_seq_tma(const Params<typename Lanes<Real>::scalar> &p, cudaStream_t s
 // kf_seq_tma_lone_*.cu for double and float.
 template <typename Real, bool kSummary>
 int launch_seq_tma_lone(const Params<typename Lanes<Real>::scalar> &p, cudaStream_t stream) {
-    const bool rare = p.x_model_steps || p.p_world_steps || p.z_steps || p.P_ckpt;
+    const bool rare = p.x_model_steps || p.p_world_steps || p.z_steps || p.P_ckpt || p.P_steps;
     const bool estimates = p.x_steps || p.p_trace_steps || p.k_gain_steps || p.nis_steps;
     if (rare) return launch_seq_tma_k<Real, kSummary, 2, false, true, 1>(p, stream);
     if (estimates) return launch_seq_tma_k<Real, kSummary, 1, false, true, 1>(p, stream);

@@ -51,9 +51,10 @@ int64_t mat_numel(int kind, int64_t n, int64_t N) {
     }
 }
 
-// cfg: integer settings; consts: dt, mass, inertia0..2, gravity; tensors: named device arrays (see optistate_kf.h)
-int64_t kf_batch(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
-    OptiKfDesc d;
+// The filter descriptor of kf_batch and kf_smooth.  cfg: integer settings; consts: dt, mass, inertia0..2, gravity; tensors: named
+// device arrays (see optistate_kf.h).  Returns the device of the tensors (the caller makes it current).
+c10::Device filter_desc(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors,
+                        OptiKfDesc &d) {
     std::memset(&d, 0, sizeof d);
     d.struct_size = sizeof d;
     d.abi_version = OPTISTATE_KF_ABI_VERSION;
@@ -82,7 +83,6 @@ int64_t kf_batch(const std::map<std::string, int64_t> &cfg, const std::map<std::
     auto x0 = tensors.find("x0");
     TORCH_CHECK(x0 != tensors.end() && x0->second.is_cuda(), "optistate_b200: 'x0' must be a CUDA tensor (there is no CPU path)");
     const Checker ck{d.dtype == OPTI_KF_F64 ? at::kDouble : at::kFloat, x0->second.device()};
-    const c10::cuda::CUDAGuard guard(ck.dev);
     const int64_t N = d.n_traj, T = d.n_steps, S = d.n_streams;
     const bool m = d.phases & OPTI_KF_PHASE_MEASURE, p = d.phases & OPTI_KF_PHASE_PREDICT, u = d.phases & OPTI_KF_PHASE_UPDATE;
     d.imu = ck.get(tensors, "imu", T * 6 * S, m);
@@ -154,12 +154,48 @@ int64_t kf_batch(const std::map<std::string, int64_t> &cfg, const std::map<std::
             d.workspace_bytes = (size_t)t.numel();
         }
     }
+    return ck.dev;
+}
+
+int64_t kf_batch(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
+    OptiKfDesc d;
+    const c10::cuda::CUDAGuard guard(filter_desc(cfg, consts, tensors, d));
     if (geti(cfg, "query_workspace", 0)) {
         size_t bytes = 0;
         const int rc = optistate_kf_workspace_bytes(&d, &bytes);
         return rc < 0 ? rc : (int64_t)bytes;
     }
     return optistate_kf_batch(&d, at::cuda::getCurrentCUDAStream().stream());
+}
+
+// Fixed-interval smoother: the filter's tensors as for kf_batch, plus x_smooth [T][12][N], optional var_smooth [T][12][N] and
+// smooth_storage (uint8, optistate_kf_smooth_storage_bytes; cfg query_storage = 1 returns that size instead of running).
+int64_t kf_smooth(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
+    OptiKfDesc d;
+    const c10::Device dev = filter_desc(cfg, consts, tensors, d);
+    const c10::cuda::CUDAGuard guard(dev);
+    if (geti(cfg, "query_storage", 0)) {
+        size_t bytes = 0;
+        const int rc = optistate_kf_smooth_storage_bytes(&d, &bytes);
+        return rc < 0 ? rc : (int64_t)bytes;
+    }
+    const Checker ck{d.dtype == OPTI_KF_F64 ? at::kDouble : at::kFloat, dev};
+    const int64_t N = d.n_traj, T = d.n_steps;
+    OptiKfSmoothDesc s;
+    std::memset(&s, 0, sizeof s);
+    s.struct_size = sizeof s;
+    s.abi_version = OPTISTATE_KF_ABI_VERSION;
+    s.filter = &d;
+    s.x_smooth = const_cast<void *>(ck.get(tensors, "x_smooth", T * 12 * N, true));
+    s.var_smooth = const_cast<void *>(ck.get(tensors, "var_smooth", T * 12 * N, false));
+    auto is = tensors.find("smooth_storage");
+    TORCH_CHECK(is != tensors.end(), "optistate_b200: missing tensor 'smooth_storage'");
+    const at::Tensor &t = is->second;
+    TORCH_CHECK(t.is_cuda() && t.device() == dev && t.scalar_type() == at::kByte && t.is_contiguous(),
+                "optistate_b200: 'smooth_storage' must be a contiguous uint8 CUDA tensor");
+    s.storage = t.data_ptr();
+    s.storage_bytes = (size_t)t.numel();
+    return optistate_kf_smooth(&s, at::cuda::getCurrentCUDAStream().stream());
 }
 
 int kf_resolve_algo(const std::map<std::string, int64_t> &cfg) {
@@ -570,6 +606,7 @@ int64_t kf_class_step(int64_t ops, int64_t cov_model, const std::vector<double> 
 PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
     m.doc() = "PyTorch loader of liboptistate_kf.so (C ABI in include/optistate_kf.h)";
     m.def("kf_batch", &kf_batch);
+    m.def("kf_smooth", &kf_smooth);
     m.def("kf_measure", &kf_measure);
     m.def("kf_class_step", &kf_class_step);
     m.def("kf_resolve_algo", &kf_resolve_algo);
