@@ -215,8 +215,8 @@ __device__ __forceinline__ void cov_predict_mpc_sym(Real (&P)[NP], const Real (&
 }
 
 // Measurement J folded in with the reciprocal of its pivot already available (`inv` = 1 / (P_kk + r_J)).  The entry
-// that becomes the NEXT pivot is updated first and its reciprocal started at once, so that chain (MUFU + Newton
-// steps) runs underneath the 65 remaining independent FMAs of this rank-1 update.  `mid` runs after the state update.
+// that becomes the NEXT pivot is updated first and its reciprocal started at once, so that chain (MUFU + its
+// refinement) runs underneath the 65 remaining independent FMAs of this rank-1 update.  `mid` runs after the state update.
 template <int J, bool kBlock = false, typename Real, int L, typename Mid>
 __device__ __forceinline__ void fold_pipelined(Real (&P)[NP], Real (&x)[NX], Real zj, Real rj, Real r_next, Real inv, Real &inv_next,
                                                Real &nis, uint32_t (&status)[L], Mid mid) {
@@ -257,7 +257,7 @@ __device__ __forceinline__ void fold_pipelined(Real (&P)[NP], Real (&x)[NX], Rea
 }
 
 // K_gain of the reference (np.trace of the 12x10 gain): K = P'[:, sel] R^-1  =>  K[j][j] = P'[j][sel(j)] / r_j.  The ten
-// reciprocals are the straight-line rcp_ (<= 2 ulp), not IEEE divisions: each division carries a branch to a slow path, and
+// reciprocals are the straight-line rcp_ (kf_arith.cuh), not IEEE divisions: each division carries a branch to a slow path, and
 // ten of those in a row cost a lone warp ~4,000 cycles per step (measured on the 1,024 x 10 k case with k_gain_steps on).
 template <bool kBlock = false, typename Real>
 __device__ __forceinline__ Real gain_trace(const Real (&P)[NP], const Real *r, int stride) {
@@ -321,27 +321,38 @@ __device__ __forceinline__ void store_world_feet(const Real *pin, const Real (&R
 }
 
 // Mean model with the rotation of the prior attitude supplied by the caller (see propagate_mean in kf_common.cuh), from the
-// leg moments (leg_moments; read through `min` with channel stride STRIDE).  The torque sum_l (R p_l) x f_l is regrouped
-// exactly as tau_i = eps_ijk (R C)_jk, an identity for any 3x3 R: per member 18 FP64 operations instead of 84 for the four
-// legs.  It rounds differently from the leg-by-leg order of propagate_mean (the last bits of the state).
+// leg moments (leg_moments; read through `min` with channel stride STRIDE).  The rate rows need the torque
+// tau = sum_l (R p_l) x f_l only in the body frame, as R^T tau.  For a rotation (R a) x (R b) = R (a x b), so
+// R^T tau = sum_l p_l x (R^T f_l), i.e. (R^T tau)_i = eps_ijk (C R)_jk: 18 FP64 operations per member instead of 84 for the four
+// legs, and w' = w + R (dt I^-1 R^T tau) adds 12.  Unlike the regrouping into moments, this step holds only because R is
+// orthogonal, which rot_zyx's R is to rounding.  The result rounds differently from propagate_mean's leg-by-leg order (the
+// last bits of the state).
 template <int STRIDE, typename Real, typename Scalar>
 __device__ __forceinline__ void propagate_mean_from_moments(const Params<Scalar> &prm, Real (&x)[NX], const Real *min, const Real (&R)[9],
                                                             bool any_trunc) {
     constexpr int L = Lanes<Real>::n;
     const auto C = [&](int k) { return min[k * STRIDE]; };
-    // tau_i = sum_m R[j][m] C[m][k] - R[k][m] C[m][j]  for (i, j, k) a cyclic permutation of (0, 1, 2)
-    Real tau[3];
+    // u_i = dt I_i^-1 (sum_m C[j][m] R[m][k] - C[k][m] R[m][j])  for (i, j, k) a cyclic permutation of (0, 1, 2)
+    Real u[3];
 #pragma unroll
     for (int i = 0; i < 3; ++i) {
         const int j = (i + 1) % 3, k = (i + 2) % 3;
-        tau[i] = fnma_(R[3 * k + 2], C(6 + j), fnma_(R[3 * k + 1], C(3 + j), fnma_(R[3 * k], C(j),
-                 fma_(R[3 * j + 2], C(6 + k), fma_(R[3 * j + 1], C(3 + k), mul_rn(R[3 * j], C(k)))))));
+        u[i] = mul_rn(fnma_(C(3 * k + 2), R[6 + j], fnma_(C(3 * k + 1), R[3 + j], fnma_(C(3 * k), R[j],
+                      fma_(C(3 * j + 2), R[6 + k], fma_(C(3 * j + 1), R[3 + k], mul_rn(C(3 * j), R[k])))))),
+                      Real(prm.dt * prm.inv_inertia[i]));
     }
-    Real u[3];
+    const Real dt = Real(prm.dt);
+    Real xn[NX];
 #pragma unroll
-    for (int k = 0; k < 3; ++k) u[k] = fma_(R[6 + k], tau[2], fma_(R[3 + k], tau[1], R[k] * tau[0])) * Real(prm.inv_inertia[k]);
-    Real dth[3] = {Real(0), Real(0), Real(0)};
+    for (int i = 0; i < 3; ++i) {
+        xn[i] = x[i];  // the attitude moves only on the trunc path below: the common path adds no zero increment
+        xn[3 + i] = fma_(dt, x[9 + i], x[3 + i]);
+        xn[6 + i] = fma_(R[3 * i + 2], u[2], fma_(R[3 * i + 1], u[1], fma_(R[3 * i], u[0], x[6 + i])));
+        xn[9 + i] = fma_(Real(prm.dt_over_m), min[(9 + i) * STRIDE], x[9 + i]);  // fs
+    }
+    xn[11] += Real(prm.dt_g);
     if (any_trunc) {  // rare: an entry of R is exactly +-1 (axis-aligned attitude); exact per-lane decision in trunc_rt
+        Real dth[3];
 #pragma unroll
         for (int ln = 0; ln < L; ++ln) {
             Scalar Rs[9], Ts[9], ang[3];
@@ -355,17 +366,9 @@ __device__ __forceinline__ void propagate_mean_from_moments(const Params<Scalar>
             for (int i = 0; i < 3; ++i)
                 lane_set(dth[i], ln, prm.dt * (Ts[3 * i] * lane_get(x[6], ln) + Ts[3 * i + 1] * lane_get(x[7], ln) + Ts[3 * i + 2] * lane_get(x[8], ln)));
         }
-    }
-    const Real dt = Real(prm.dt);
-    Real xn[NX];
 #pragma unroll
-    for (int i = 0; i < 3; ++i) {
-        xn[i] = x[i] + dth[i];
-        xn[3 + i] = fma_(dt, x[9 + i], x[3 + i]);
-        xn[6 + i] = fma_(dt, fma_(R[3 * i + 2], u[2], fma_(R[3 * i + 1], u[1], R[3 * i] * u[0])), x[6 + i]);
-        xn[9 + i] = fma_(Real(prm.dt_over_m), min[(9 + i) * STRIDE], x[9 + i]);  // fs
+        for (int i = 0; i < 3; ++i) xn[i] = add_rn(x[i], dth[i]);  // dth rounded before the sum, as in propagate_mean
     }
-    xn[11] += Real(prm.dt_g);
 #pragma unroll
     for (int i = 0; i < NX; ++i) x[i] = xn[i];
 }

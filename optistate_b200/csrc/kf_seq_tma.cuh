@@ -13,7 +13,7 @@
 //     counter) issues the refill, so nobody waits on a designated producer.
 //   * Three channel groups, each single-buffered and refilled for step t+1 the moment the block has consumed
 //     step t's copy, so the copy has most of a filter step (several microseconds) to land:
-//         G0 = M[12]            read at the top of the step (mean model)        -> refilled right away
+//         G0 = M[12]            read at the top of the step (mean model)        -> refilled after the covariance predict (kBlock), else right away
 //              (+ the feet p[12] in the kOut == 2 instantiations, which write p_world_steps, and the 3 reference body
 //              angles of the predict_mpc covariance model in the kMpc instantiations)
 //         G1 = z[10]            read one by one as the measurements are folded  -> refilled before the last fold
@@ -356,10 +356,21 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
 #pragma unroll
                 for (int k = 0; k < 3; ++k) E[3 * a + k] = exp_minus_one(Real(prm.dt) * Rb[3 * k + a]);
         }
-        {  // this warp has consumed the step's moments: the last one refills G0 for step t + 1
+        Real nis = Real(0), inv, inv_n;
+        const auto first_pivot = [&] {
+            const Real s = P[tri(0, 0)] + r[0];
+            note_bad_pivot(s, status, OPTI_KF_ST_NOT_PD);
+            inv = rcp_(s);
+        };
+        const auto refill_g0 = [&] {  // this warp has consumed the step's moments: the last one refills G0 for step t + 1
             const int elect = last_reader(0);
             if (more) issue_g0<kOut, kMpc>(maps, t + kStages, s_warp, g0, &bar[0], elect);
-        }
+        };
+        // kBlock: the first pivot's reciprocal and the G0 refill come after the predict, so that the mean model's dependent chain,
+        // the predict's independent FMAs and the reciprocal form one basic block the scheduler can interleave (the copy still has
+        // the whole update phase to land).  The full-covariance kernels keep the refill here and the reciprocal after the G1 wait:
+        // with 78 live covariance entries the longer live ranges spill.
+        if constexpr (!kBlock) refill_g0();
         if constexpr (kOut == 2) {
             if (active && prm.x_model_steps) {
 #pragma unroll
@@ -369,6 +380,10 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
 
         if constexpr (kMpc) cov_predict_mpc_sym(P, E, e1_mpc, q, nt);
         else cov_predict_sym<kBlock>(P, Rm, prm.dt, q, nt);
+        if constexpr (kBlock) {
+            first_pivot();
+            refill_g0();
+        }
 
         // ---- G1: measurements, folded in one at a time ---------------------------------------------------------
         mbar_wait(&bar[1], par);
@@ -382,12 +397,7 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
                 for (int c = 0; c < NZ; ++c) st_traj(prm.z_steps, (t * NZ + c) * N + i, z[c * 32]);
             }
         }
-        Real nis = Real(0), inv, inv_n;
-        {
-            const Real s = P[tri(0, 0)] + r[0];
-            note_bad_pivot(s, status, OPTI_KF_ST_NOT_PD);
-            inv = rcp_(s);
-        }
+        if constexpr (!kBlock) first_pivot();
         auto nothing = [] {};
         fold_pipelined<0, kBlock>(P, x, z[0 * 32], r[0 * nt], r[1 * nt], inv, inv_n, nis, status, nothing); inv = inv_n;
         fold_pipelined<1, kBlock>(P, x, z[1 * 32], r[1 * nt], r[2 * nt], inv, inv_n, nis, status, nothing); inv = inv_n;

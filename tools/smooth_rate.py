@@ -28,7 +28,7 @@ FP64_PEAK = 37.2e12
 
 # ---- exact operation count of one backward step of kf_rts_kernel (kf_smooth.cuh); FMA = 2 flops, rint / compares not counted
 SINCOS = {"f64": 1 + 4 * 2 + 1 + 5 * 2 + 1 + 2 + 5 * 2 + 1 + 1 + 2 + 1, "f32": 1 + 3 * 2 + 1 + 2 * 2 + 1 + 2 + 2 * 2 + 1 + 1 + 2 + 1}
-RCP = {"f64": 6 * 2, "f32": 2 * 2}  # Newton steps after the hardware seed
+RCP = {"f64": 3 * 2, "f32": 2 * 2}  # the FMAs that refine the hardware seed (rcp_, kf_arith.cuh)
 ROT_PRODUCTS = 21  # rot_zyx: products and sums of the multiplied-out R
 
 
