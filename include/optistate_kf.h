@@ -337,6 +337,30 @@ typedef struct OptiKfSmoothDesc {
 int optistate_kf_smooth_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out);
 int optistate_kf_smooth(const OptiKfSmoothDesc *desc, void *cuda_stream);
 
+/* ---- E-step of expectation-maximisation for diagonal Q and R, from the sensor streams alone.  Runs the forward pass exactly as
+ * optistate_kf_smooth does, then the smoother's backward kernel with one more step, t = -1, for the model
+ *     x_{-1} ~ N(x0, P0),  x_{t+1} = x-_{t+1} + F_{t+1} (x_t - x+_t) + w_t,  w_t ~ N(0, Q)  (t = -1 .. T-2, x+_{-1} = x0),
+ *     z_t = H x_t + v_t,  v_t ~ N(0, R)  (t = 0 .. T-1),
+ * whose smoother for t >= 0 is optistate_kf_smooth's.  Per trajectory, stats[row][i] holds
+ *     rows 0-11   Sw_c = sum_t E[w_{t,c}^2 | Z]
+ *     rows 12-21  Sv_k = sum_t E[v_{t,k}^2 | Z]
+ *     row 22      the prediction-error log-likelihood sum_t log N(z_t; H x-_t, H P-_t H^T + R) of the filter that ran
+ * so that the M-step is q = Sw / T, r = Sv / T (pooled: the sums over trajectories over N T).  Accepts exactly what
+ * optistate_kf_smooth accepts, with the same return codes.  P0 absent means P0 = Q, as for the filter. ---- */
+#define OPTI_KF_EM_STATS_ROWS 23  /* 0-11 Sw, 12-21 Sv, 22 log-likelihood */
+typedef struct OptiKfNoiseEmDesc {
+    uint32_t struct_size;       /* sizeof(OptiKfNoiseEmDesc) */
+    uint32_t abi_version;       /* OPTISTATE_KF_ABI_VERSION */
+    const OptiKfDesc *filter;   /* forward pass, run exactly as optistate_kf_batch runs it */
+    void *stats;                /* [23][N] required */
+    void *x_smooth, *var_smooth;  /* [T][12][N] optional here */
+    void *storage;              /* device scratch of optistate_kf_noise_em_storage_bytes(filter): the smoother's storage, plus the
+                                   measurements z [T][10][S] when the filter forms them (OPTI_KF_PHASE_MEASURE) */
+    size_t storage_bytes;
+} OptiKfNoiseEmDesc;
+int optistate_kf_noise_em_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out);
+int optistate_kf_noise_em_stats(const OptiKfNoiseEmDesc *desc, void *cuda_stream);
+
 /* Runs the filter; dtype taken from the descriptor. */
 int optistate_kf_batch(const OptiKfDesc *desc, void *cuda_stream);
 /* Same, asserting the scalar type (the two names a binding would import). */

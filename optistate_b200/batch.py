@@ -318,28 +318,39 @@ def kf_smooth(
     Supported: the sequential algo with the predict() covariance model, diagonal Q and R and a P0 without entries across the
     groups {th, w}, {x, vx}, {y, vy}, {z, vz}; anything else raises ValueError.  status gains OPTI_KF_ST_SMOOTH_NOT_PD (32).
     """
-    if cov_model != "predict":
-        raise ValueError("kf_smooth supports the predict() covariance model only (predict_mpc makes F_d dense)")
-    if structure != "auto":
-        raise ValueError("kf_smooth needs the decoupled-group form of P; structure='full' keeps cross-group entries")
-    if algo == "joint":
-        raise ValueError("kf_smooth runs on the sequential filter; algo='joint' is not supported")
+    call, smooth_want = _backward_call("kf_smooth", imu, p, dp, contact, f, x0, P0, Q, R, outputs, True, dict(
+        n_traj=n_traj, dtype=dtype, stream_index=stream_index, stream_offset=stream_offset, ckpt_every=ckpt_every, truth=truth,
+        nominal=nominal, body_ref=body_ref, z=z, algo=algo, cov_model=cov_model, q_kind=q_kind, r_kind=r_kind, p0_kind=p0_kind, dt=dt,
+        mass=mass, inertia=inertia, gravity=gravity, device=device, out=out, summary_peers=summary_peers,
+        p0_is_symmetric=p0_is_symmetric, structure=structure, packed=packed))
+    with torch.cuda.device(call.device):
+        _attach_workspace(call, out)
+        _attach_storage(call, out, call.ext.kf_smooth, "smooth_storage", "optistate_kf_smooth_storage_bytes")
+        nv.check(int(call.ext.kf_smooth(call.cfg, call.consts, call.tensors)), "optistate_kf_smooth")
+    return call.result(summary_peers, extra=smooth_want)
+
+
+def _backward_call(who, imu, p, dp, contact, f, x0, P0, Q, R, outputs, need_x_smooth, kw):
+    """The forward pass of kf_smooth / kf_noise_stats (_filter_call) with what the backward kernel refuses refused here, and the
+    smoothed outputs allocated: returns (call, smoothed output names)."""
+    if kw["cov_model"] != "predict":
+        raise ValueError(f"{who} supports the predict() covariance model only (predict_mpc makes F_d dense)")
+    if kw["structure"] != "auto":
+        raise ValueError(f"{who} needs the decoupled-group form of P; structure='full' keeps cross-group entries")
+    if kw["algo"] == "joint":
+        raise ValueError(f"{who} runs on the sequential filter; algo='joint' is not supported")
     outputs = list(outputs)
     smooth_want = [o for o in outputs if o in _SMOOTH_OUTPUTS]
-    if "x_smooth" not in smooth_want:
+    if need_x_smooth and "x_smooth" not in smooth_want:
         smooth_want.insert(0, "x_smooth")
-    call = _filter_call(imu, p, dp, contact, f, x0, P0, Q, R, n_traj=n_traj, dtype=dtype, stream_index=stream_index,
-                        stream_offset=stream_offset, outputs=[o for o in outputs if o not in _SMOOTH_OUTPUTS], ckpt_every=ckpt_every,
-                        truth=truth, nominal=nominal, body_ref=body_ref, z=z, algo="sequential" if algo == "auto" else algo,
-                        cov_model=cov_model, q_kind=q_kind, r_kind=r_kind, p0_kind=p0_kind, dt=dt, mass=mass, inertia=inertia,
-                        gravity=gravity, device=device, out=out, summary_peers=summary_peers, p0_is_symmetric=p0_is_symmetric,
-                        structure=structure, packed=packed)
+    kw = dict(kw, algo="sequential" if kw["algo"] == "auto" else kw["algo"])
+    call = _filter_call(imu, p, dp, contact, f, x0, P0, Q, R, outputs=[o for o in outputs if o not in _SMOOTH_OUTPUTS], **kw)
     cfg = call.cfg
     if cfg["q_kind"] not in (nv.MAT_DIAG, nv.MAT_DIAG_PER) or cfg["r_kind"] not in (nv.MAT_DIAG, nv.MAT_DIAG_PER):
-        raise ValueError("kf_smooth needs diagonal Q and R (dense noise couples the decoupled groups)")
+        raise ValueError(f"{who} needs diagonal Q and R (dense noise couples the decoupled groups)")
     if cfg["p0_kind"] in (nv.MAT_DENSE, nv.MAT_DENSE_PER) and not cfg["flags"] & nv.FLAG_P0_DECOUPLED:
-        raise ValueError("kf_smooth needs a P0 without entries across the groups {th, w}, {x, vx}, {y, vy}, {z, vz}")
-    T, N = call.n_steps, call.n_traj
+        raise ValueError(f"{who} needs a P0 without entries across the groups {{th, w}}, {{x, vx}}, {{y, vy}}, {{z, vz}}")
+    T, N, out, dtype = call.n_steps, call.n_traj, kw["out"], kw["dtype"]
     for o in smooth_want:
         shape = (T, 12, N)
         if out is not None and o in out:
@@ -348,18 +359,148 @@ def kf_smooth(
             call.tensors[o] = out[o]
         else:
             call.tensors[o] = torch.empty(shape, dtype=dtype, device=call.device)
+    return call, smooth_want
+
+
+def _attach_storage(call: _FilterCall, out, entry, key, what):
+    """The backward pass's device scratch (size from the library), reused from / kept in `out[key]`."""
+    st_bytes = entry(dict(call.cfg, query_storage=1), call.consts, call.tensors)
+    nv.check(int(min(st_bytes, 0)), what)
+    st = out.get(key) if out is not None else None
+    if st is None or st.numel() < st_bytes:
+        st = torch.empty(max(int(st_bytes), 1), dtype=torch.uint8, device=call.device)
+        if out is not None:
+            out[key] = st  # kept for the caller's next call with the same shapes
+    call.tensors[key] = st
+
+
+EM_STATS_ROWS = 23
+EM_FIELDS = {"Sw": slice(0, 12), "Sv": slice(12, 22), "loglik": 22}
+
+
+def kf_noise_stats(
+    imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *,
+    n_traj: Optional[int] = None, dtype: torch.dtype = torch.float64, stream_index=None, stream_offset: int = 0,
+    outputs: Iterable[str] = (), ckpt_every: int = 0, truth=None, nominal=None, body_ref=None, z=None,
+    algo: str = "auto", cov_model: str = "predict", q_kind=None, r_kind=None, p0_kind=None,
+    dt: float = INITIAL_PARAMS.DT_mpc, mass: float = INITIAL_PARAMS.ROBOT_MASS, inertia=None,
+    gravity: float = INITIAL_PARAMS.GRAVITY, device=None, out: Optional[Dict[str, torch.Tensor]] = None,
+    summary_peers=None, p0_is_symmetric: Optional[bool] = None, structure: str = "auto", packed: bool = True,
+) -> KfBatchResult:
+    """E-step of expectation-maximisation for diagonal Q and R (DESIGN.md section 0): runs the filter and the smoother's backward
+    kernel exactly as kf_smooth does with the same arguments, and returns `noise_stats` [23, N] per trajectory:
+        rows 0-11   Sw = sum_t E[w_t^2 | Z]   over the T transitions t = -1 .. T-2 (x_{-1} ~ N(x0, P0), P0 = Q when None)
+        rows 12-21  Sv = sum_t E[v_t^2 | Z]   over the T measurements
+        row 22      the prediction-error log-likelihood sum_t log N(z_t; H x-_t, H P-_t H^T + R) of the filter that ran
+    The M-step is Q = diag(Sw) / T, R = diag(Sv) / T (kf_noise_em).  outputs: x_smooth, var_smooth and any kf_batch output, all
+    optional.  out: as for kf_smooth, with "noise_stats" and "em_storage" (uint8 scratch of optistate_kf_noise_em_storage_bytes).
+    Refuses what kf_smooth refuses, with the same ValueErrors.
+    """
+    call, smooth_want = _backward_call("kf_noise_stats", imu, p, dp, contact, f, x0, P0, Q, R, outputs, False, dict(
+        n_traj=n_traj, dtype=dtype, stream_index=stream_index, stream_offset=stream_offset, ckpt_every=ckpt_every, truth=truth,
+        nominal=nominal, body_ref=body_ref, z=z, algo=algo, cov_model=cov_model, q_kind=q_kind, r_kind=r_kind, p0_kind=p0_kind, dt=dt,
+        mass=mass, inertia=inertia, gravity=gravity, device=device, out=out, summary_peers=summary_peers,
+        p0_is_symmetric=p0_is_symmetric, structure=structure, packed=packed))
+    shape = (EM_STATS_ROWS, call.n_traj)
+    if out is not None and "noise_stats" in out:
+        if tuple(out["noise_stats"].shape) != shape or out["noise_stats"].dtype != dtype:
+            raise ValueError(f"out['noise_stats'] must be {shape} {dtype}")
+        call.tensors["noise_stats"] = out["noise_stats"]
+    else:
+        call.tensors["noise_stats"] = torch.empty(shape, dtype=dtype, device=call.device)
     with torch.cuda.device(call.device):
         _attach_workspace(call, out)
-        st_bytes = call.ext.kf_smooth(dict(cfg, query_storage=1), call.consts, call.tensors)
-        nv.check(int(min(st_bytes, 0)), "optistate_kf_smooth_storage_bytes")
-        st = out.get("smooth_storage") if out is not None else None
-        if st is None or st.numel() < st_bytes:
-            st = torch.empty(max(int(st_bytes), 1), dtype=torch.uint8, device=call.device)
-            if out is not None:
-                out["smooth_storage"] = st  # kept for the caller's next call with the same shapes
-        call.tensors["smooth_storage"] = st
-        nv.check(int(call.ext.kf_smooth(cfg, call.consts, call.tensors)), "optistate_kf_smooth")
-    return call.result(summary_peers, extra=smooth_want)
+        _attach_storage(call, out, call.ext.kf_noise_em_stats, "em_storage", "optistate_kf_noise_em_storage_bytes")
+        nv.check(int(call.ext.kf_noise_em_stats(call.cfg, call.consts, call.tensors)), "optistate_kf_noise_em_stats")
+    return call.result(summary_peers, extra=("noise_stats", *smooth_want))
+
+
+@dataclass
+class KfNoiseEmResult:
+    """Result of kf_noise_em.  Q [12, N] / R [10, N] (or [12] / [10] with shared=True) are the estimates after the last M-step;
+    loglik[k] is the log-likelihood of every trajectory under the k-th iterate (the E-step of iteration k), so the last row
+    belongs to the iterate before Q, R.  status: the OR of the filter's status words over all iterations."""
+    Q: torch.Tensor
+    R: torch.Tensor
+    loglik: torch.Tensor
+    iterations: int
+    converged: bool
+    status: torch.Tensor
+
+
+def kf_noise_em(
+    imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *, iters: int = 50, tol: Optional[float] = None,
+    shared: bool = False, n_traj: Optional[int] = None, dtype: torch.dtype = torch.float64, stream_index=None,
+    stream_offset: int = 0, z=None, dt: float = INITIAL_PARAMS.DT_mpc, mass: float = INITIAL_PARAMS.ROBOT_MASS, inertia=None,
+    gravity: float = INITIAL_PARAMS.GRAVITY, device=None, out: Optional[Dict[str, torch.Tensor]] = None,
+) -> KfNoiseEmResult:
+    """Maximum-likelihood diagonal Q and R from the sensor streams alone, by expectation-maximisation: each iteration runs
+    kf_noise_stats (filter, smoother, E-step) with the current Q, R and sets Q = Sw / T, R = Sv / T - per trajectory, or with
+    shared=True pooled over all trajectories (sums over N T).  The M-step runs as torch ops on the device.
+
+    Q, R: the start, diagonal ([12] / [10], [12, N] / [10, N], or a diagonal matrix; default settings.py's).  P0 stays what the
+    caller passes for every iteration; None holds it at the starting Q.  The filter is re-linearised each iteration (F and x-
+    follow the new estimates), so the log-likelihood is not guaranteed to rise, though it does on typical recordings.
+    Known limitation (DESIGN.md section 0): q of x and y is unobservable and stays at its start, and the estimates describe the
+    affine model the filter runs, whose attitude rows use R^T rather than the mean model's trunc(R^T).
+    tol: stop once the largest relative increase of the log-likelihood (per trajectory; pooled with shared=True) falls below
+    it - one host synchronisation per iteration, only when tol is given.  Storage and workspace are reused across iterations.
+    """
+    if iters < 1:
+        raise ValueError("iters must be >= 1")
+    nv.require_cuda()
+    out = {} if out is None else out  # storage and workspace of the first E-step, reused by the others
+    device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    base = z if z is not None else imu
+    T, S = int(base.shape[0]), int(base.shape[2]) if base.ndim == 3 else 1
+    N = int(S if n_traj is None else n_traj)
+
+    def diag_start(a, default, n):
+        t = _as_device(default if a is None else a, dtype, device)
+        if t.shape == (n, n):
+            if not _is_diagonal(t):
+                raise ValueError("kf_noise_em estimates diagonal noise: Q and R must be diagonal")
+            t = torch.diagonal(t)
+        if t.shape == (n,):
+            return t.clone() if shared else t[:, None].expand(n, N).contiguous()
+        if t.shape != (n, N):
+            raise ValueError(f"kf_noise_em: a noise start of shape {tuple(t.shape)} is not [{n}], [{n}, {n}] or [{n}, {N}]")
+        if shared:
+            raise ValueError("kf_noise_em: shared=True needs a shared start ([n] or a diagonal matrix)")
+        return t.clone()
+
+    q = diag_start(Q, INITIAL_PARAMS.Q, 12)
+    r = diag_start(R, INITIAL_PARAMS.R, 10)
+    kind = nv.MAT_DIAG if shared else nv.MAT_DIAG_PER
+    p0, p0_kind = (q.clone(), kind) if P0 is None else (P0, None)
+    status = torch.zeros(N, dtype=torch.int32, device=device)
+    lls, converged, prev = [], False, None
+    for it in range(iters):
+        res = kf_noise_stats(imu, p, dp, contact, f, x0, p0, q, r, n_traj=N, dtype=dtype, stream_index=stream_index,
+                    stream_offset=stream_offset, z=z, q_kind=kind, r_kind=kind, p0_kind=p0_kind, dt=dt, mass=mass, inertia=inertia,
+                    gravity=gravity, device=device, out=out)
+        st = res.noise_stats
+        status |= res.status
+        ll = st[EM_STATS_ROWS - 1].clone()
+        lls.append(ll)
+        if shared:
+            q = st[0:12].sum(dim=1) / (N * T)
+            r = st[12:22].sum(dim=1) / (N * T)
+        else:
+            q = st[0:12] / T
+            r = st[12:22] / T
+        if tol is not None and prev is not None:
+            if shared:
+                a, b = prev.sum(), ll.sum()
+                rel = (b - a) / a.abs()
+            else:
+                rel = ((ll - prev) / prev.abs()).max()
+            if float(rel) < tol:
+                converged = True
+                break
+        prev = ll
+    loglik = torch.stack(lls) if lls else torch.empty((0, N), dtype=dtype, device=device)
+    return KfNoiseEmResult(Q=q, R=r, loglik=loglik, iterations=len(lls), converged=converged, status=status)
 
 
 def kf_measure(imu, p, dp, contact, *, dtype: torch.dtype = torch.float64, device=None, want_odom: bool = False):

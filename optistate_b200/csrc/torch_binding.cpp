@@ -198,6 +198,37 @@ int64_t kf_smooth(const std::map<std::string, int64_t> &cfg, const std::map<std:
     return optistate_kf_smooth(&s, at::cuda::getCurrentCUDAStream().stream());
 }
 
+// E-step of EM: the filter's tensors as for kf_batch, plus stats [23][N], optional x_smooth / var_smooth [T][12][N] and em_storage
+// (uint8, optistate_kf_noise_em_storage_bytes; cfg query_storage = 1 returns that size instead of running).
+int64_t kf_noise_em_stats(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
+    OptiKfDesc d;
+    const c10::Device dev = filter_desc(cfg, consts, tensors, d);
+    const c10::cuda::CUDAGuard guard(dev);
+    if (geti(cfg, "query_storage", 0)) {
+        size_t bytes = 0;
+        const int rc = optistate_kf_noise_em_storage_bytes(&d, &bytes);
+        return rc < 0 ? rc : (int64_t)bytes;
+    }
+    const Checker ck{d.dtype == OPTI_KF_F64 ? at::kDouble : at::kFloat, dev};
+    const int64_t N = d.n_traj, T = d.n_steps;
+    OptiKfNoiseEmDesc s;
+    std::memset(&s, 0, sizeof s);
+    s.struct_size = sizeof s;
+    s.abi_version = OPTISTATE_KF_ABI_VERSION;
+    s.filter = &d;
+    s.stats = const_cast<void *>(ck.get(tensors, "noise_stats", OPTI_KF_EM_STATS_ROWS * N, true));
+    s.x_smooth = const_cast<void *>(ck.get(tensors, "x_smooth", T * 12 * N, false));
+    s.var_smooth = const_cast<void *>(ck.get(tensors, "var_smooth", T * 12 * N, false));
+    auto is = tensors.find("em_storage");
+    TORCH_CHECK(is != tensors.end(), "optistate_b200: missing tensor 'em_storage'");
+    const at::Tensor &t = is->second;
+    TORCH_CHECK(t.is_cuda() && t.device() == dev && t.scalar_type() == at::kByte && t.is_contiguous(),
+                "optistate_b200: 'em_storage' must be a contiguous uint8 CUDA tensor");
+    s.storage = t.data_ptr();
+    s.storage_bytes = (size_t)t.numel();
+    return optistate_kf_noise_em_stats(&s, at::cuda::getCurrentCUDAStream().stream());
+}
+
 int kf_resolve_algo(const std::map<std::string, int64_t> &cfg) {
     // shape-free query: only kinds / phases / model matter, pointers are faked as non-null
     OptiKfDesc d;
@@ -607,6 +638,7 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
     m.doc() = "PyTorch loader of liboptistate_kf.so (C ABI in include/optistate_kf.h)";
     m.def("kf_batch", &kf_batch);
     m.def("kf_smooth", &kf_smooth);
+    m.def("kf_noise_em_stats", &kf_noise_em_stats);
     m.def("kf_measure", &kf_measure);
     m.def("kf_class_step", &kf_class_step);
     m.def("kf_resolve_algo", &kf_resolve_algo);
