@@ -17,6 +17,7 @@
  *   optistate_kf_smooth     runs optistate_kf_batch and then the fixed-interval Rauch-Tung-Striebel smoother backwards over
  *                           its per-step estimates (optistate_kf_smooth_storage_bytes sizes its scratch).  The reference
  *                           has no smoother: this entry point has no reference counterpart.
+ *   optistate_kf_smooth_full the same on the full covariance (predict_mpc model, coupled P0).
  *
  * Conventions
  *   - plain C, no torch / C++ types; every pointer is a NON-OWNING DEVICE pointer unless stated otherwise;
@@ -336,6 +337,17 @@ typedef struct OptiKfSmoothDesc {
 } OptiKfSmoothDesc;
 int optistate_kf_smooth_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out);
 int optistate_kf_smooth(const OptiKfSmoothDesc *desc, void *cuda_stream);
+
+/* ---- the same smoother on the FULL covariance: the predict_mpc covariance model (cov_model = OPTI_KF_COV_MPC, whose
+ * F_d = 1 1^T + D makes P dense), OPTI_KF_FLAG_FULL_COVARIANCE and dense (symmetric) P0 kinds are taken besides everything
+ * optistate_kf_smooth takes.  The forward pass always runs the full-covariance kernels and keeps all 78 entries of P+_t in
+ * tri order, so `storage` (optistate_kf_smooth_full_storage_bytes) holds P+ [T][78][N] plus x+ and x- as above; the outputs of
+ * the forward pass equal optistate_kf_batch's.  The backward kernel recomputes P-_{t+1} with the covariance model the filter
+ * ran (predict_mpc: from body_ref rows 0-2 of step t + 1).  Whatever the SEQUENTIAL filter cannot run (dense Q or R, algo =
+ * JOINT) returns OPTI_KF_E_UNSUPPORTED; AUTO runs SEQUENTIAL, so a dense P0 must be symmetric.  status[i] gains
+ * OPTI_KF_ST_SMOOTH_NOT_PD. ---- */
+int optistate_kf_smooth_full_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out);
+int optistate_kf_smooth_full(const OptiKfSmoothDesc *desc, void *cuda_stream);
 
 /* ---- E-step of expectation-maximisation for diagonal Q and R, from the sensor streams alone.  Runs the forward pass exactly as
  * optistate_kf_smooth does, then the smoother's backward kernel with one more step, t = -1, for the model

@@ -330,12 +330,13 @@ def kf_smooth(
     return call.result(summary_peers, extra=smooth_want)
 
 
-def _backward_call(who, imu, p, dp, contact, f, x0, P0, Q, R, outputs, need_x_smooth, kw):
-    """The forward pass of kf_smooth / kf_noise_stats (_filter_call) with what the backward kernel refuses refused here, and the
-    smoothed outputs allocated: returns (call, smoothed output names)."""
-    if kw["cov_model"] != "predict":
+def _backward_call(who, imu, p, dp, contact, f, x0, P0, Q, R, outputs, need_x_smooth, kw, full=False):
+    """The forward pass of kf_smooth / kf_noise_stats / kf_smooth_full (_filter_call) with what the backward kernel refuses refused
+    here, and the smoothed outputs allocated: returns (call, smoothed output names).  full: the dense backward kernel, which takes
+    either covariance model and any symmetric P0 (a non-symmetric one is refused by _filter_call for algo='sequential')."""
+    if not full and kw["cov_model"] != "predict":
         raise ValueError(f"{who} supports the predict() covariance model only (predict_mpc makes F_d dense)")
-    if kw["structure"] != "auto":
+    if not full and kw["structure"] != "auto":
         raise ValueError(f"{who} needs the decoupled-group form of P; structure='full' keeps cross-group entries")
     if kw["algo"] == "joint":
         raise ValueError(f"{who} runs on the sequential filter; algo='joint' is not supported")
@@ -347,8 +348,9 @@ def _backward_call(who, imu, p, dp, contact, f, x0, P0, Q, R, outputs, need_x_sm
     call = _filter_call(imu, p, dp, contact, f, x0, P0, Q, R, outputs=[o for o in outputs if o not in _SMOOTH_OUTPUTS], **kw)
     cfg = call.cfg
     if cfg["q_kind"] not in (nv.MAT_DIAG, nv.MAT_DIAG_PER) or cfg["r_kind"] not in (nv.MAT_DIAG, nv.MAT_DIAG_PER):
-        raise ValueError(f"{who} needs diagonal Q and R (dense noise couples the decoupled groups)")
-    if cfg["p0_kind"] in (nv.MAT_DENSE, nv.MAT_DENSE_PER) and not cfg["flags"] & nv.FLAG_P0_DECOUPLED:
+        raise ValueError(f"{who} needs diagonal Q and R " + ("(the sequential filter takes no dense noise)" if full else
+                                                               "(dense noise couples the decoupled groups)"))
+    if not full and cfg["p0_kind"] in (nv.MAT_DENSE, nv.MAT_DENSE_PER) and not cfg["flags"] & nv.FLAG_P0_DECOUPLED:
         raise ValueError(f"{who} needs a P0 without entries across the groups {{th, w}}, {{x, vx}}, {{y, vy}}, {{z, vz}}")
     T, N, out, dtype = call.n_steps, call.n_traj, kw["out"], kw["dtype"]
     for o in smooth_want:
@@ -360,6 +362,42 @@ def _backward_call(who, imu, p, dp, contact, f, x0, P0, Q, R, outputs, need_x_sm
         else:
             call.tensors[o] = torch.empty(shape, dtype=dtype, device=call.device)
     return call, smooth_want
+
+
+def kf_smooth_full(
+    imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *,
+    n_traj: Optional[int] = None, dtype: torch.dtype = torch.float64, stream_index=None, stream_offset: int = 0,
+    outputs: Iterable[str] = ("x_smooth",), ckpt_every: int = 0, truth=None, nominal=None, body_ref=None, z=None,
+    algo: str = "auto", cov_model: str = "predict", q_kind=None, r_kind=None, p0_kind=None,
+    dt: float = INITIAL_PARAMS.DT_mpc, mass: float = INITIAL_PARAMS.ROBOT_MASS, inertia=None,
+    gravity: float = INITIAL_PARAMS.GRAVITY, device=None, out: Optional[Dict[str, torch.Tensor]] = None,
+    summary_peers=None, p0_is_symmetric: Optional[bool] = None, structure: str = "auto", packed: bool = True,
+) -> KfBatchResult:
+    """The fixed-interval smoother of kf_smooth on the FULL 12x12 covariance (DESIGN.md section 0.2): for the predict_mpc
+    covariance model (cov_model="mpc", whose element-wise F_d = exp(dt F) makes P dense) and for a P0 with entries across the
+    groups, which kf_smooth refuses.  Arguments, outputs (x_smooth, var_smooth and any kf_batch output) and out["smooth_storage"]
+    as for kf_smooth; the storage holds all 78 entries of P+ per step (624 B per trajectory-step in FP64).  The forward pass runs
+    the sequential filter's full-covariance kernels, whose outputs equal kf_batch's with the same arguments.
+
+    The closed loop's output, smoothed offline:
+
+        xs, fs, *_ = estimate_state_mpc_batch(...)
+        res = kf_smooth_full(imu, p, dp, contact, fs, x0, P0, Q, R, cov_model="mpc", body_ref=body_ref[:, 0], n_traj=N)
+
+    Raises ValueError for algo="joint", dense Q or R, and a non-symmetric P0.  FP64 is the dtype for real data: under the
+    predict_mpc model with identified noise P- reaches condition numbers near 1e8, which FP32 cannot resolve.
+    status gains OPTI_KF_ST_SMOOTH_NOT_PD (32).
+    """
+    call, smooth_want = _backward_call("kf_smooth_full", imu, p, dp, contact, f, x0, P0, Q, R, outputs, True, dict(
+        n_traj=n_traj, dtype=dtype, stream_index=stream_index, stream_offset=stream_offset, ckpt_every=ckpt_every, truth=truth,
+        nominal=nominal, body_ref=body_ref, z=z, algo=algo, cov_model=cov_model, q_kind=q_kind, r_kind=r_kind, p0_kind=p0_kind, dt=dt,
+        mass=mass, inertia=inertia, gravity=gravity, device=device, out=out, summary_peers=summary_peers,
+        p0_is_symmetric=p0_is_symmetric, structure=structure, packed=packed), full=True)
+    with torch.cuda.device(call.device):
+        _attach_workspace(call, out)
+        _attach_storage(call, out, call.ext.kf_smooth_full, "smooth_storage", "optistate_kf_smooth_full_storage_bytes")
+        nv.check(int(call.ext.kf_smooth_full(call.cfg, call.consts, call.tensors)), "optistate_kf_smooth_full")
+    return call.result(summary_peers, extra=smooth_want)
 
 
 def _attach_storage(call: _FilterCall, out, entry, key, what):

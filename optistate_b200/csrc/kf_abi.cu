@@ -11,6 +11,7 @@
 #include "kf_mpc_params.cuh"
 #include "kf_seq_core.cuh"
 #include "kf_smooth.cuh"
+#include "kf_smooth_full.cuh"
 
 namespace {
 
@@ -167,7 +168,8 @@ int launch_streamed<float>(const OptiKfDesc *d, const okf::Params<float> &p, cud
     return packed_pair_ok(d) ? launch_streamed_t<okf::F2>(d, p, stream) : launch_streamed_t<float>(d, p, stream);
 }
 
-// P_steps: the smoother's packed per-step posterior covariance [T][30][N] (optistate_kf_smooth only; decoupled form)
+// P_steps: the smoothers' per-step posterior covariance, [T][30][N] from the decoupled kernels (optistate_kf_smooth) or [T][78][N]
+// from the full ones (optistate_kf_smooth_full)
 template <typename Real>
 int launch(const OptiKfDesc *d, int algo, cudaStream_t stream, void *P_steps = nullptr) {
     if (d->n_traj == 0) return OPTI_KF_OK;
@@ -330,14 +332,15 @@ int smooth_check(const OptiKfDesc *d) {
     return algo == OPTI_KF_ALGO_SEQUENTIAL ? OPTI_KF_OK : OPTI_KF_E_UNSUPPORTED;
 }
 
-// Scratch of the smoother, each part padded to 256 bytes: packed P+ [T][30][N] at 0, then x+ and x- [T][12][N] unless the
-// filter descriptor has x_steps / x_model_steps (the smoother reads those).  Byte offsets.
+// Scratch of the smoother, each part padded to 256 bytes: P+ [T][np][N] at 0 (np = 30 packed decoupled entries, or all 78 for
+// optistate_kf_smooth_full), then x+ and x- [T][12][N] unless the filter descriptor has x_steps / x_model_steps (the smoother
+// reads those).  Byte offsets.
 struct SmoothStorage {
     size_t x_post, x_prior, total;
-    explicit SmoothStorage(const OptiKfDesc *d) {
+    explicit SmoothStorage(const OptiKfDesc *d, int np = okf::NPB) {
         const auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
         const size_t esz = d->dtype == OPTI_KF_F64 ? 8 : 4, tn = (size_t)d->n_steps * (size_t)d->n_traj;
-        x_post = up(tn * okf::NPB * esz);
+        x_post = up(tn * (size_t)np * esz);
         x_prior = x_post + (d->x_steps ? 0 : up(tn * okf::NX * esz));
         total = x_prior + (d->x_model_steps ? 0 : up(tn * okf::NX * esz));
     }
@@ -361,6 +364,41 @@ int smooth(const OptiKfSmoothDesc *s, cudaStream_t stream) {
     p.x_post = (const Real *)fw.x_steps; p.x_prior = (const Real *)fw.x_model_steps; p.P_post = (const Real *)base;
     p.x_smooth = (Real *)s->x_smooth; p.var_smooth = (Real *)s->var_smooth; p.status = f->status;
     rc = okf::launch_rts<Real>(p, stream);
+    if (rc < 0) return rc;
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return cudaGetLastError() == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
+}
+
+// What the full-covariance smoother can take: whatever the SEQUENTIAL filter runs (AUTO means SEQUENTIAL here, as the symmetric
+// P0 this entry requires permits), in either covariance model and with any P0 kind.
+int smooth_full_check(const OptiKfDesc *d) {
+    const int rc = validate(d);
+    if (rc != OPTI_KF_OK) return rc;
+    return d->algo != OPTI_KF_ALGO_JOINT && sequential_ok(d) ? OPTI_KF_OK : OPTI_KF_E_UNSUPPORTED;
+}
+
+// The forward pass always runs the full-covariance kernels, so P+ is [T][78][N] whatever the caller's flags (on decoupled inputs
+// they are bit-identical to the kBlock ones, kf_seq_core.cuh).
+template <typename Real>
+int smooth_full(const OptiKfSmoothDesc *s, cudaStream_t stream) {
+    const OptiKfDesc *f = s->filter;
+    const SmoothStorage ss(f, okf::NP);
+    unsigned char *base = (unsigned char *)s->storage;
+    OptiKfDesc fw = *f;
+    fw.flags |= OPTI_KF_FLAG_FULL_COVARIANCE;
+    if (!fw.x_steps && base) fw.x_steps = base + ss.x_post;
+    if (!fw.x_model_steps && base) fw.x_model_steps = base + ss.x_prior;
+    int rc = launch<Real>(&fw, OPTI_KF_ALGO_SEQUENTIAL, stream, base);
+    if (rc != OPTI_KF_OK) return rc;
+    if (f->n_traj == 0 || f->n_steps == 0) return OPTI_KF_OK;
+    okf::SmoothFullParams<Real> p;
+    std::memset(&p, 0, sizeof p);
+    p.N = f->n_traj; p.T = f->n_steps; p.dt = (Real)f->dt; p.cov_model = f->cov_model;
+    p.Q = (const Real *)f->Q; p.q_kind = f->q_kind;
+    p.x_post = (const Real *)fw.x_steps; p.x_prior = (const Real *)fw.x_model_steps; p.P_post = (const Real *)base;
+    p.body_ref = (const Real *)f->body_ref; p.S = f->n_streams; p.stream_offset = f->stream_offset; p.stream_index = f->stream_index;
+    p.x_smooth = (Real *)s->x_smooth; p.var_smooth = (Real *)s->var_smooth; p.status = f->status;
+    rc = okf::launch_rts_full<Real>(p, stream);
     if (rc < 0) return rc;
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError() == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
@@ -479,6 +517,29 @@ int optistate_kf_smooth(const OptiKfSmoothDesc *desc, void *cuda_stream) {
     if (steps && !desc->storage) return OPTI_KF_E_NULL;
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     return f->dtype == OPTI_KF_F64 ? smooth<double>(desc, stream) : smooth<float>(desc, stream);
+}
+
+int optistate_kf_smooth_full_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out) {
+    const int rc = smooth_full_check(filter);
+    if (rc != OPTI_KF_OK) return rc;
+    if (!bytes_out) return OPTI_KF_E_NULL;
+    *bytes_out = SmoothStorage(filter, okf::NP).total;
+    return OPTI_KF_OK;
+}
+
+int optistate_kf_smooth_full(const OptiKfSmoothDesc *desc, void *cuda_stream) {
+    if (!desc) return OPTI_KF_E_NULL;
+    if (desc->struct_size != sizeof(OptiKfSmoothDesc) || desc->abi_version != OPTISTATE_KF_ABI_VERSION) return OPTI_KF_E_VERSION;
+    if (!desc->filter) return OPTI_KF_E_NULL;
+    const int rc = smooth_full_check(desc->filter);
+    if (rc != OPTI_KF_OK) return rc;
+    const OptiKfDesc *f = desc->filter;
+    const bool steps = f->n_traj > 0 && f->n_steps > 0;
+    if (steps && !desc->x_smooth) return OPTI_KF_E_NULL;
+    if (desc->storage_bytes < SmoothStorage(f, okf::NP).total) return OPTI_KF_E_SHAPE;
+    if (steps && !desc->storage) return OPTI_KF_E_NULL;
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    return f->dtype == OPTI_KF_F64 ? smooth_full<double>(desc, stream) : smooth_full<float>(desc, stream);
 }
 
 int optistate_kf_noise_em_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out) {

@@ -39,8 +39,9 @@ struct Params {
     long long summary_ld;
     int n_summary_peers;
     Real *summary_peers[OPTI_KF_MAX_PEERS];
-    // [T][30][N] posterior covariance of every step, decoupled-group entries only (pk_slot, kf_seq_core.cuh); set by the
-    // smoother's forward pass alone.  Last, so that every other field keeps its constant-bank offset.
+    // posterior covariance of every step: [T][30][N] decoupled-group entries (pk_slot) in the kBlock kernels, [T][78][N] in tri
+    // order in the full ones (kf_seq_core.cuh); set by the smoothers' forward passes alone.  Last, so that every other field
+    // keeps its constant-bank offset.
     Real *P_steps;
 };
 

@@ -158,8 +158,9 @@ __global__ void __launch_bounds__(128) kf_seq_kernel(const __grid_constant__ Par
 #pragma unroll
                 for (int b = 0; b < NX; ++b) dst[(long long)(a * NX + b) * N] = cpl<kBlock>(a, b) ? P[tri(a, b)] : Real(0);
         }
-        if constexpr (kBlock) {
-            if (prm.P_steps) store_packed_P(prm.P_steps, t, N, i, P);
+        if (prm.P_steps) {
+            if constexpr (kBlock) store_packed_P(prm.P_steps, t, N, i, P);
+            else store_full_P(prm.P_steps, t, N, i, P);
         }
     }
 

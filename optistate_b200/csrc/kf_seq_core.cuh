@@ -67,6 +67,14 @@ __device__ __forceinline__ void store_packed_P(Scalar *dst, long long t, long lo
             if (cpl<true>(a, b)) st_traj(dst, (t * NPB + pk_slot(a, b)) * N + i, P[tri(a, b)]);
 }
 
+// All 78 entries of P of step t to dst[t][tri(a, b)][N]: Params.P_steps of the full-covariance kernels, read by the dense
+// smoother (kf_smooth_full.cuh).  Which of the two layouts a kernel writes follows from its kBlock.
+template <typename Real, typename Scalar>
+__device__ __forceinline__ void store_full_P(Scalar *dst, long long t, long long N, long long i, const Real (&P)[NP]) {
+#pragma unroll
+    for (int k = 0; k < NP; ++k) st_traj(dst, (t * NP + k) * N + i, P[k]);
+}
+
 // P <- F_d P F_d^T + diag(q), F_d = I + dt N, N[a,c] = R^T, N[b,d] = I   (blocks a=0..2 b=3..5 c=6..8 d=9..11)
 // Written with explicit fma_ so that double, float and the packed F2 type run the same operation sequence.
 template <bool kBlock = false, typename Real, typename Scalar>

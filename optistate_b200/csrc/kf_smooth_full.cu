@@ -1,0 +1,21 @@
+// Backward kernel of the full-covariance smoother (kf_smooth_full.cuh): instantiations and launch.
+#include "kf_smooth_full.cuh"
+
+namespace okf {
+
+template <typename Real>
+int launch_rts_full(const SmoothFullParams<Real> &p, cudaStream_t stream) {
+    if (p.N == 0 || p.T == 0) return OPTI_KF_OK;
+    const long long blocks = (p.N + RTSF_TRAJ - 1) / RTSF_TRAJ;
+    if (blocks > 0x7fffffffLL) return OPTI_KF_E_SHAPE;
+    const size_t smem = (size_t)RTSF_SMEM_ROWS * RTSF_TRAJ * sizeof(Real);  // 111 KB (FP64): two blocks per SM, 55.5 KB (FP32)
+    const auto kern = p.cov_model == OPTI_KF_COV_MPC ? kf_rts_full_kernel<Real, true> : kf_rts_full_kernel<Real, false>;
+    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return OPTI_KF_E_CUDA;
+    kern<<<(unsigned)blocks, RTSF_THREADS, smem, stream>>>(p);
+    return OPTI_KF_OK;
+}
+
+template int launch_rts_full<double>(const SmoothFullParams<double> &, cudaStream_t);
+template int launch_rts_full<float>(const SmoothFullParams<float> &, cudaStream_t);
+
+}  // namespace okf

@@ -169,14 +169,18 @@ int64_t kf_batch(const std::map<std::string, int64_t> &cfg, const std::map<std::
 }
 
 // Fixed-interval smoother: the filter's tensors as for kf_batch, plus x_smooth [T][12][N], optional var_smooth [T][12][N] and
-// smooth_storage (uint8, optistate_kf_smooth_storage_bytes; cfg query_storage = 1 returns that size instead of running).
-int64_t kf_smooth(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
+// smooth_storage (uint8, the entry's storage query; cfg query_storage = 1 returns that size instead of running).  kf_smooth and
+// kf_smooth_full differ only in the two entry points.
+using SmoothStorageFn = int (*)(const OptiKfDesc *, size_t *);
+using SmoothFn = int (*)(const OptiKfSmoothDesc *, void *);
+int64_t run_smooth(SmoothStorageFn storage_bytes, SmoothFn smooth, const std::map<std::string, int64_t> &cfg,
+                   const std::map<std::string, double> &consts, const TensorMap &tensors) {
     OptiKfDesc d;
     const c10::Device dev = filter_desc(cfg, consts, tensors, d);
     const c10::cuda::CUDAGuard guard(dev);
     if (geti(cfg, "query_storage", 0)) {
         size_t bytes = 0;
-        const int rc = optistate_kf_smooth_storage_bytes(&d, &bytes);
+        const int rc = storage_bytes(&d, &bytes);
         return rc < 0 ? rc : (int64_t)bytes;
     }
     const Checker ck{d.dtype == OPTI_KF_F64 ? at::kDouble : at::kFloat, dev};
@@ -195,7 +199,16 @@ int64_t kf_smooth(const std::map<std::string, int64_t> &cfg, const std::map<std:
                 "optistate_b200: 'smooth_storage' must be a contiguous uint8 CUDA tensor");
     s.storage = t.data_ptr();
     s.storage_bytes = (size_t)t.numel();
-    return optistate_kf_smooth(&s, at::cuda::getCurrentCUDAStream().stream());
+    return smooth(&s, at::cuda::getCurrentCUDAStream().stream());
+}
+
+int64_t kf_smooth(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
+    return run_smooth(optistate_kf_smooth_storage_bytes, optistate_kf_smooth, cfg, consts, tensors);
+}
+
+// The full-covariance smoother (optistate_kf_smooth_full): arguments as for kf_smooth.
+int64_t kf_smooth_full(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
+    return run_smooth(optistate_kf_smooth_full_storage_bytes, optistate_kf_smooth_full, cfg, consts, tensors);
 }
 
 // E-step of EM: the filter's tensors as for kf_batch, plus stats [23][N], optional x_smooth / var_smooth [T][12][N] and em_storage
@@ -638,6 +651,7 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
     m.doc() = "PyTorch loader of liboptistate_kf.so (C ABI in include/optistate_kf.h)";
     m.def("kf_batch", &kf_batch);
     m.def("kf_smooth", &kf_smooth);
+    m.def("kf_smooth_full", &kf_smooth_full);
     m.def("kf_noise_em_stats", &kf_noise_em_stats);
     m.def("kf_measure", &kf_measure);
     m.def("kf_class_step", &kf_class_step);
