@@ -18,6 +18,8 @@
  *                           its per-step estimates (optistate_kf_smooth_storage_bytes sizes its scratch).  The reference
  *                           has no smoother: this entry point has no reference counterpart.
  *   optistate_kf_smooth_full the same on the full covariance (predict_mpc model, coupled P0).
+ *   optistate_kf_noise_em_stats / optistate_kf_noise_em_full_stats
+ *                           the E-step of expectation-maximisation for diagonal Q and R on either smoother.
  *
  * Conventions
  *   - plain C, no torch / C++ types; every pointer is a NON-OWNING DEVICE pointer unless stated otherwise;
@@ -372,6 +374,16 @@ typedef struct OptiKfNoiseEmDesc {
 } OptiKfNoiseEmDesc;
 int optistate_kf_noise_em_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out);
 int optistate_kf_noise_em_stats(const OptiKfNoiseEmDesc *desc, void *cuda_stream);
+
+/* ---- the same E-step on the FULL covariance: the model above with F_{t+1} the transition of either covariance model (predict_mpc:
+ * F_d = 1 1^T + D from body_ref rows 0-2 of step t + 1, and of step 0 for the transition out of x_{-1}), and x_{-1} ~ N(x0, P0) with
+ * any P0 kind, coupled or dense (symmetric).  Runs the forward pass exactly as optistate_kf_smooth_full does, then its backward
+ * kernel with one more step, t = -1; the rows of `stats` mean what they mean above, and the innovation covariance of the
+ * log-likelihood is the dense 10x10 H P-_t H^T + R.  Takes OptiKfNoiseEmDesc unchanged; `storage`
+ * (optistate_kf_noise_em_full_storage_bytes) is optistate_kf_smooth_full's, plus z [T][10][S] when the filter forms the
+ * measurements.  Accepts exactly what optistate_kf_smooth_full accepts, with the same return codes. ---- */
+int optistate_kf_noise_em_full_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out);
+int optistate_kf_noise_em_full_stats(const OptiKfNoiseEmDesc *desc, void *cuda_stream);
 
 /* Runs the filter; dtype taken from the descriptor. */
 int optistate_kf_batch(const OptiKfDesc *desc, void *cuda_stream);

@@ -331,7 +331,7 @@ def kf_smooth(
 
 
 def _backward_call(who, imu, p, dp, contact, f, x0, P0, Q, R, outputs, need_x_smooth, kw, full=False):
-    """The forward pass of kf_smooth / kf_noise_stats / kf_smooth_full (_filter_call) with what the backward kernel refuses refused
+    """The forward pass of kf_smooth / kf_noise_stats / kf_smooth_full / kf_noise_stats_full (_filter_call) with what the backward kernel refuses refused
     here, and the smoothed outputs allocated: returns (call, smoothed output names).  full: the dense backward kernel, which takes
     either covariance model and any symmetric P0 (a non-symmetric one is refused by _filter_call for algo='sequential')."""
     if not full and kw["cov_model"] != "predict":
@@ -439,6 +439,35 @@ def kf_noise_stats(
         nominal=nominal, body_ref=body_ref, z=z, algo=algo, cov_model=cov_model, q_kind=q_kind, r_kind=r_kind, p0_kind=p0_kind, dt=dt,
         mass=mass, inertia=inertia, gravity=gravity, device=device, out=out, summary_peers=summary_peers,
         p0_is_symmetric=p0_is_symmetric, structure=structure, packed=packed))
+    return _noise_stats_run(call, smooth_want, out, dtype, summary_peers, "kf_noise_em_stats", "optistate_kf_noise_em_stats")
+
+
+def kf_noise_stats_full(
+    imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *,
+    n_traj: Optional[int] = None, dtype: torch.dtype = torch.float64, stream_index=None, stream_offset: int = 0,
+    outputs: Iterable[str] = (), ckpt_every: int = 0, truth=None, nominal=None, body_ref=None, z=None,
+    algo: str = "auto", cov_model: str = "predict", q_kind=None, r_kind=None, p0_kind=None,
+    dt: float = INITIAL_PARAMS.DT_mpc, mass: float = INITIAL_PARAMS.ROBOT_MASS, inertia=None,
+    gravity: float = INITIAL_PARAMS.GRAVITY, device=None, out: Optional[Dict[str, torch.Tensor]] = None,
+    summary_peers=None, p0_is_symmetric: Optional[bool] = None, structure: str = "auto", packed: bool = True,
+) -> KfBatchResult:
+    """The E-step of kf_noise_stats on the FULL covariance (DESIGN.md section 0.3): the forward pass and backward kernel of
+    kf_smooth_full, so the predict_mpc covariance model (cov_model="mpc", with body_ref) and a coupled or dense symmetric P0 are
+    taken.  Returns `noise_stats` [23, N] with the rows of kf_noise_stats (the innovation covariance of the log-likelihood is the
+    dense H P- H^T + R), and x_smooth / var_smooth or any kf_batch output when asked for.  out: as for kf_smooth_full, with
+    "noise_stats" and "em_storage" (optistate_kf_noise_em_full_storage_bytes).  Refuses what kf_smooth_full refuses: algo="joint",
+    dense Q or R and a non-symmetric P0 raise ValueError.
+    """
+    call, smooth_want = _backward_call("kf_noise_stats_full", imu, p, dp, contact, f, x0, P0, Q, R, outputs, False, dict(
+        n_traj=n_traj, dtype=dtype, stream_index=stream_index, stream_offset=stream_offset, ckpt_every=ckpt_every, truth=truth,
+        nominal=nominal, body_ref=body_ref, z=z, algo=algo, cov_model=cov_model, q_kind=q_kind, r_kind=r_kind, p0_kind=p0_kind, dt=dt,
+        mass=mass, inertia=inertia, gravity=gravity, device=device, out=out, summary_peers=summary_peers,
+        p0_is_symmetric=p0_is_symmetric, structure=structure, packed=packed), full=True)
+    return _noise_stats_run(call, smooth_want, out, dtype, summary_peers, "kf_noise_em_full_stats", "optistate_kf_noise_em_full_stats")
+
+
+def _noise_stats_run(call, smooth_want, out, dtype, summary_peers, entry, what):
+    """The stats output and the E-step's storage attached to `call`, then the library's entry `what` (binding `entry`)."""
     shape = (EM_STATS_ROWS, call.n_traj)
     if out is not None and "noise_stats" in out:
         if tuple(out["noise_stats"].shape) != shape or out["noise_stats"].dtype != dtype:
@@ -448,8 +477,9 @@ def kf_noise_stats(
         call.tensors["noise_stats"] = torch.empty(shape, dtype=dtype, device=call.device)
     with torch.cuda.device(call.device):
         _attach_workspace(call, out)
-        _attach_storage(call, out, call.ext.kf_noise_em_stats, "em_storage", "optistate_kf_noise_em_storage_bytes")
-        nv.check(int(call.ext.kf_noise_em_stats(call.cfg, call.consts, call.tensors)), "optistate_kf_noise_em_stats")
+        fn = getattr(call.ext, entry)
+        _attach_storage(call, out, fn, "em_storage", what.replace("_stats", "_storage_bytes"))
+        nv.check(int(fn(call.cfg, call.consts, call.tensors)), what)
     return call.result(summary_peers, extra=("noise_stats", *smooth_want))
 
 
@@ -484,6 +514,40 @@ def kf_noise_em(
     tol: stop once the largest relative increase of the log-likelihood (per trajectory; pooled with shared=True) falls below
     it - one host synchronisation per iteration, only when tol is given.  Storage and workspace are reused across iterations.
     """
+    return _noise_em("kf_noise_em", kf_noise_stats, {}, imu, p, dp, contact, f, x0, P0, Q, R, iters, tol, shared, n_traj, dtype,
+                     stream_index, stream_offset, z, dt, mass, inertia, gravity, device, out)
+
+
+def kf_noise_em_full(
+    imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *, iters: int = 50, tol: Optional[float] = None,
+    shared: bool = False, n_traj: Optional[int] = None, dtype: torch.dtype = torch.float64, stream_index=None,
+    stream_offset: int = 0, z=None, cov_model: str = "predict", body_ref=None, dt: float = INITIAL_PARAMS.DT_mpc,
+    mass: float = INITIAL_PARAMS.ROBOT_MASS, inertia=None, gravity: float = INITIAL_PARAMS.GRAVITY, device=None,
+    out: Optional[Dict[str, torch.Tensor]] = None,
+) -> KfNoiseEmResult:
+    """kf_noise_em on the FULL covariance (DESIGN.md section 0.3): each iteration runs kf_noise_stats_full, so the filter may be
+    the predict_mpc covariance model the reference's conversion driver runs (cov_model="mpc", body_ref [T, 12, S]: its rows 0-2 are
+    the reference body angles of every step), and P0 may be coupled or dense (symmetric).  Arguments, M-step, tol and result as
+    for kf_noise_em; P0 is held at the caller's value (or at the starting Q) across iterations.
+
+    Q and R of the closed loop's filter, from the sensor streams alone:
+
+        xs, fs, *_ = estimate_state_mpc_batch(imu, p, dp, contact, ref)
+        em = kf_noise_em_full(imu, p, dp, contact, fs, cov_model="mpc", body_ref=ref[:, 0], n_traj=N, shared=True)
+
+    The forces fs are inputs here and stay fixed across iterations: with a new Q and R the closed loop would compute other forces,
+    and EM does not re-run it.  The estimate is the noise of the affine model the filter runs (DESIGN.md section 0.1's caveat), and
+    under predict_mpc that model is further from the mean model: F_d = 1 1^T + D is not the mean model's Jacobian, so Q absorbs
+    the difference and is not the process noise of the robot.  FP64 is the dtype for real data (kf_smooth_full).
+    """
+    return _noise_em("kf_noise_em_full", kf_noise_stats_full, dict(cov_model=cov_model, body_ref=body_ref), imu, p, dp, contact, f,
+                     x0, P0, Q, R, iters, tol, shared, n_traj, dtype, stream_index, stream_offset, z, dt, mass, inertia, gravity,
+                     device, out)
+
+
+def _noise_em(who, stats_fn, extra, imu, p, dp, contact, f, x0, P0, Q, R, iters, tol, shared, n_traj, dtype, stream_index,
+              stream_offset, z, dt, mass, inertia, gravity, device, out) -> KfNoiseEmResult:
+    """The EM loop of kf_noise_em / kf_noise_em_full around the E-step stats_fn (extra: its further keyword arguments)."""
     if iters < 1:
         raise ValueError("iters must be >= 1")
     nv.require_cuda()
@@ -497,14 +561,14 @@ def kf_noise_em(
         t = _as_device(default if a is None else a, dtype, device)
         if t.shape == (n, n):
             if not _is_diagonal(t):
-                raise ValueError("kf_noise_em estimates diagonal noise: Q and R must be diagonal")
+                raise ValueError(f"{who} estimates diagonal noise: Q and R must be diagonal")
             t = torch.diagonal(t)
         if t.shape == (n,):
             return t.clone() if shared else t[:, None].expand(n, N).contiguous()
         if t.shape != (n, N):
-            raise ValueError(f"kf_noise_em: a noise start of shape {tuple(t.shape)} is not [{n}], [{n}, {n}] or [{n}, {N}]")
+            raise ValueError(f"{who}: a noise start of shape {tuple(t.shape)} is not [{n}], [{n}, {n}] or [{n}, {N}]")
         if shared:
-            raise ValueError("kf_noise_em: shared=True needs a shared start ([n] or a diagonal matrix)")
+            raise ValueError(f"{who}: shared=True needs a shared start ([n] or a diagonal matrix)")
         return t.clone()
 
     q = diag_start(Q, INITIAL_PARAMS.Q, 12)
@@ -514,9 +578,9 @@ def kf_noise_em(
     status = torch.zeros(N, dtype=torch.int32, device=device)
     lls, converged, prev = [], False, None
     for it in range(iters):
-        res = kf_noise_stats(imu, p, dp, contact, f, x0, p0, q, r, n_traj=N, dtype=dtype, stream_index=stream_index,
-                    stream_offset=stream_offset, z=z, q_kind=kind, r_kind=kind, p0_kind=p0_kind, dt=dt, mass=mass, inertia=inertia,
-                    gravity=gravity, device=device, out=out)
+        res = stats_fn(imu, p, dp, contact, f, x0, p0, q, r, n_traj=N, dtype=dtype, stream_index=stream_index,
+                       stream_offset=stream_offset, z=z, q_kind=kind, r_kind=kind, p0_kind=p0_kind, dt=dt, mass=mass, inertia=inertia,
+                       gravity=gravity, device=device, out=out, **extra)
         st = res.noise_stats
         status |= res.status
         ll = st[EM_STATS_ROWS - 1].clone()

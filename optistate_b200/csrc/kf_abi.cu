@@ -404,12 +404,13 @@ int smooth_full(const OptiKfSmoothDesc *s, cudaStream_t stream) {
     return cudaGetLastError() == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
 }
 
-// Scratch of the EM statistics: the smoother's, then z [T][10][S] (padded to 256 bytes) when the filter forms the measurements.
+// Scratch of the EM statistics: the smoother's (np as for SmoothStorage), then z [T][10][S] (padded to 256 bytes) when the filter
+// forms the measurements.
 struct EmStorage {
     size_t z, total;
-    explicit EmStorage(const OptiKfDesc *d) {
+    explicit EmStorage(const OptiKfDesc *d, int np = okf::NPB) {
         const size_t esz = d->dtype == OPTI_KF_F64 ? 8 : 4, ts = (size_t)d->n_steps * (size_t)d->n_streams;
-        z = SmoothStorage(d).total;
+        z = SmoothStorage(d, np).total;
         total = z + ((d->phases & OPTI_KF_PHASE_MEASURE) ? ((ts * okf::NZ * esz + 255) & ~(size_t)255) : 0);
     }
 };
@@ -447,6 +448,47 @@ int noise_em_stats(const OptiKfNoiseEmDesc *s, cudaStream_t stream) {
     p.P0 = (const Real *)f->P0; p.p0_kind = f->p0_kind;
     p.stats = (Real *)s->stats;
     rc = okf::launch_em_stats<Real>(p, stream);
+    if (rc < 0) return rc;
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return cudaGetLastError() == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
+}
+
+// The E-step on the full covariance: the forward pass of smooth_full(), then kf_rts_full_kernel<Real, mpc, true>.
+template <typename Real>
+int noise_em_full_stats(const OptiKfNoiseEmDesc *s, cudaStream_t stream) {
+    const OptiKfDesc *f = s->filter;
+    const SmoothStorage ss(f, okf::NP);
+    const EmStorage es(f, okf::NP);
+    unsigned char *base = (unsigned char *)s->storage;
+    OptiKfDesc fw = *f;
+    fw.flags |= OPTI_KF_FLAG_FULL_COVARIANCE;
+    if (!fw.x_steps && base) fw.x_steps = base + ss.x_post;
+    if (!fw.x_model_steps && base) fw.x_model_steps = base + ss.x_prior;
+    int rc = launch<Real>(&fw, OPTI_KF_ALGO_SEQUENTIAL, stream, base);
+    if (rc != OPTI_KF_OK) return rc;
+    const long long N = f->n_traj, T = f->n_steps;
+    if (N == 0) return OPTI_KF_OK;
+    if (T == 0)
+        return cudaMemsetAsync(s->stats, 0, (size_t)okf::EM_STATS_ROWS * N * sizeof(Real), stream) == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
+    const Real *z = (const Real *)f->z_in;
+    if (f->phases & OPTI_KF_PHASE_MEASURE) {
+        z = (const Real *)(base + es.z);
+        launch_measure<Real>(T, f->n_streams, (const Real *)f->imu, (const Real *)f->p, (const Real *)f->dp, (const Real *)f->contact,
+                             nullptr, (Real *)z, nullptr, nullptr, nullptr, stream);
+    }
+    okf::SmoothFullParams<Real> p;
+    std::memset(&p, 0, sizeof p);
+    p.N = N; p.T = T; p.dt = (Real)f->dt; p.cov_model = f->cov_model;
+    p.Q = (const Real *)f->Q; p.q_kind = f->q_kind;
+    p.x_post = (const Real *)fw.x_steps; p.x_prior = (const Real *)fw.x_model_steps; p.P_post = (const Real *)base;
+    p.body_ref = (const Real *)f->body_ref; p.S = f->n_streams; p.stream_offset = f->stream_offset; p.stream_index = f->stream_index;
+    p.x_smooth = (Real *)s->x_smooth; p.var_smooth = (Real *)s->var_smooth; p.status = f->status;
+    p.z = z;
+    p.R = (const Real *)f->R; p.r_kind = f->r_kind;
+    p.x0 = (const Real *)f->x0; p.x0_ld = f->x0_per_traj ? N : 1; p.x0_inc = f->x0_per_traj ? 1 : 0;
+    p.P0 = (const Real *)f->P0; p.p0_kind = f->p0_kind;
+    p.stats = (Real *)s->stats;
+    rc = okf::launch_em_stats_full<Real>(p, stream);
     if (rc < 0) return rc;
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError() == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
@@ -562,6 +604,28 @@ int optistate_kf_noise_em_stats(const OptiKfNoiseEmDesc *desc, void *cuda_stream
     if (f->n_traj > 0 && f->n_steps > 0 && !desc->storage) return OPTI_KF_E_NULL;
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     return f->dtype == OPTI_KF_F64 ? noise_em_stats<double>(desc, stream) : noise_em_stats<float>(desc, stream);
+}
+
+int optistate_kf_noise_em_full_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out) {
+    const int rc = smooth_full_check(filter);
+    if (rc != OPTI_KF_OK) return rc;
+    if (!bytes_out) return OPTI_KF_E_NULL;
+    *bytes_out = EmStorage(filter, okf::NP).total;
+    return OPTI_KF_OK;
+}
+
+int optistate_kf_noise_em_full_stats(const OptiKfNoiseEmDesc *desc, void *cuda_stream) {
+    if (!desc) return OPTI_KF_E_NULL;
+    if (desc->struct_size != sizeof(OptiKfNoiseEmDesc) || desc->abi_version != OPTISTATE_KF_ABI_VERSION) return OPTI_KF_E_VERSION;
+    if (!desc->filter) return OPTI_KF_E_NULL;
+    const int rc = smooth_full_check(desc->filter);
+    if (rc != OPTI_KF_OK) return rc;
+    const OptiKfDesc *f = desc->filter;
+    if (f->n_traj > 0 && !desc->stats) return OPTI_KF_E_NULL;
+    if (desc->storage_bytes < EmStorage(f, okf::NP).total) return OPTI_KF_E_SHAPE;
+    if (f->n_traj > 0 && f->n_steps > 0 && !desc->storage) return OPTI_KF_E_NULL;
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    return f->dtype == OPTI_KF_F64 ? noise_em_full_stats<double>(desc, stream) : noise_em_full_stats<float>(desc, stream);
 }
 
 int optistate_kf_batch(const OptiKfDesc *desc, void *cuda_stream) {

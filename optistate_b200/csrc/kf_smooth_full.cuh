@@ -17,6 +17,15 @@
 //   * The next (earlier) step's inputs are copied to shared memory with cp.async while the current one computes (two stages),
 //     each warp copying a quarter of the rows; three block barriers per step.
 //   * Pivots use rcp_.  One that is not positive and finite sets OPTI_KF_ST_SMOOTH_NOT_PD; the recursion carries on.
+//
+// kStats: the E-step of EM on the same recursion (DESIGN.md section 0.3), as kf_rts_kernel<Real, true> does for the decoupled
+// groups: one more step, t = -1, from x+ = x0 and all 78 entries of P+ = P0, and per trajectory the 23 sums of OptiKfNoiseEmDesc.
+//   * Sw: warp q owns the rows rtsf_row(q, .).  It solves those columns of M = (P-)^-1 on the factor it holds, parks them in its
+//     own slots of W (dead until W is written), and once dPs is complete adds q + q^2 ((M dPs M)_uu + (M d)_u^2).
+//   * Sv: row k goes to the warp that owns the diagonal entry of dPs it reads (tri(sel(k), sel(k)) mod 4), before it subtracts P-.
+//   * log-likelihood: warp RTSF_LL_WARP, after its rows of Ps_t, recomputes P- and factors S = H P- H^T + R (10x10) on the
+//     innovation; determinants are multiplied into a mantissa with the exponent split off (det_renorm).
+//   * The accumulators are registers of the warp that owns them; z is read from global memory (shared by a stream's members).
 #pragma once
 
 #include "kf_smooth.cuh"
@@ -38,6 +47,12 @@ struct SmoothFullParams {
     Real *x_smooth;             // [T][12][N]
     Real *var_smooth;           // [T][12][N] or NULL
     uint32_t *status;           // [N] or NULL: OPTI_KF_ST_SMOOTH_NOT_PD is OR-ed in
+    // E-step of EM (kf_rts_full_kernel<Real, kMpc, true> only; last, so that every field above keeps its constant-bank offset)
+    const Real *z;              // [T][10][S] measurements of the stream (S, stream_offset, stream_index as for body_ref)
+    const Real *R; int r_kind;  // OPTI_KF_MAT_DIAG [10] or OPTI_KF_MAT_DIAG_PER [10][N]
+    const Real *x0; long long x0_ld; int x0_inc;
+    const Real *P0; int p0_kind;  // any kind of Params: NONE = Q
+    Real *stats;                // [23][N]: Sw (0-11), Sv (12-21), log-likelihood (22)
 };
 
 constexpr int RTSF_TRAJ = 32;                      // trajectories per block
@@ -63,7 +78,29 @@ __host__ __device__ constexpr bool rtsf_rows_ok() {
 }
 static_assert(rtsf_rows_ok(), "the row sets partition the 12 rows with 19-20 triangle entries per warp");
 
-template <typename Real, bool kMpc>
+// E-step roles.  Sv row k: the warp that owns dPs entry tri(sel(k), sel(k)) (3 3 2 2 rows for warps 0-3), in accumulator slot
+// rtsf_sv_slot(k); the log-likelihood: warp 2 (19 triangle entries, 2 Sv rows).
+__host__ __device__ constexpr int rtsf_sv_warp(int k) { return tri(sel(k), sel(k)) & 3; }
+__host__ __device__ constexpr int rtsf_sv_slot(int k) {
+    int n = 0;
+    for (int j = 0; j < k; ++j) n += rtsf_sv_warp(j) == rtsf_sv_warp(k);
+    return n;
+}
+__host__ __device__ constexpr int rtsf_sv_of(int k) {  // measurement row whose Sv reads dPs entry k, or -1
+    for (int j = 0; j < NZ; ++j)
+        if (tri(sel(j), sel(j)) == k) return j;
+    return -1;
+}
+constexpr int RTSF_SV_SLOTS = 3;
+constexpr int RTSF_LL_WARP = 2;
+__host__ __device__ constexpr bool rtsf_sv_ok() {
+    for (int k = 0; k < NZ; ++k)
+        if (rtsf_sv_slot(k) >= RTSF_SV_SLOTS) return false;
+    return true;
+}
+static_assert(rtsf_sv_ok(), "no warp owns more than three Sv rows");
+
+template <typename Real, bool kMpc, bool kStats = false>
 __global__ void __launch_bounds__(RTSF_THREADS, 2) kf_rts_full_kernel(const __grid_constant__ SmoothFullParams<Real> prm) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int nt = RTSF_TRAJ;
@@ -77,18 +114,37 @@ __global__ void __launch_bounds__(RTSF_THREADS, 2) kf_rts_full_kernel(const __gr
     const long long i = (long long)blockIdx.x * nt + lane;
     const bool active = i < N;
     const long long ic = active ? i : N - 1;  // the last block's spare lanes recompute a real trajectory and store nothing
-    const long long s = kMpc ? (prm.stream_index ? (long long)prm.stream_index[ic] : (ic + prm.stream_offset) % prm.S) : 0;
+    const long long s = (kMpc || kStats) ? (prm.stream_index ? (long long)prm.stream_index[ic] : (ic + prm.stream_offset) % prm.S) : 0;
     const Real *qg = prm.Q + (prm.q_kind == OPTI_KF_MAT_DIAG ? 0 : ic);
     const int qs = prm.q_kind == OPTI_KF_MAT_DIAG ? 1 : (int)N;
     int rows[3];
 #pragma unroll
     for (int c = 0; c < 3; ++c) rows[c] = rtsf_row(q, c);
 
+    // entry k (tri order) of P0 for the step t = -1
+    const auto prior_P0 = [&](int k) -> Real {
+        int a = 0;
+        while (tri(a, a) < k) ++a;
+        const int b = k - tri(a, 0);
+        switch (prm.p0_kind) {
+            case OPTI_KF_MAT_NONE: return a == b ? qg[a * qs] : Real(0);
+            case OPTI_KF_MAT_DIAG: return a == b ? prm.P0[a] : Real(0);
+            case OPTI_KF_MAT_DIAG_PER: return a == b ? prm.P0[a * N + ic] : Real(0);
+            case OPTI_KF_MAT_DENSE: return prm.P0[a * NX + b];
+            default: return prm.P0[(long long)(a * NX + b) * N + ic];
+        }
+    };
     // step t's stage: x+_t, P+_t and (t + 1 < T) x-_{t+1} and the reference angles of step t + 1; warp q copies rows q mod 4
     const auto issue = [&](long long t, Real *st) {
 #pragma unroll 1
         for (int r = q; r < RTSF_STAGE_ROWS; r += RTSF_WARPS) {
             const Real *src;
+            if constexpr (kStats) {
+                if (t < 0 && r < NX + NP) {  // the step t = -1: x+ = x0, P+ = P0 (Q when absent), every entry
+                    st[r * nt] = r < NX ? prm.x0[r * prm.x0_ld + ic * prm.x0_inc] : prior_P0(r - NX);
+                    continue;
+                }
+            }
             if (r < NX) src = prm.x_post + (t * NX + r) * N + ic;
             else if (r < NX + NP) src = prm.P_post + (t * NP + (r - NX)) * N + ic;
             else if (t + 1 >= T) continue;
@@ -101,7 +157,12 @@ __global__ void __launch_bounds__(RTSF_THREADS, 2) kf_rts_full_kernel(const __gr
     };
     const auto store = [&](long long t, int row, Real x, Real var) {
         if (!active) return;
-        st_stream(prm.x_smooth + (t * NX + row) * N + i, x);
+        if constexpr (kStats) {
+            if (t < 0) return;  // the step t = -1 stores nothing; x_smooth is optional
+            if (prm.x_smooth) st_stream(prm.x_smooth + (t * NX + row) * N + i, x);
+        } else {
+            st_stream(prm.x_smooth + (t * NX + row) * N + i, x);
+        }
         if (prm.var_smooth) st_stream(prm.var_smooth + (t * NX + row) * N + i, var);
     };
 
@@ -117,21 +178,16 @@ __global__ void __launch_bounds__(RTSF_THREADS, 2) kf_rts_full_kernel(const __gr
 #pragma unroll
         for (int c = 0; c < 3; ++c) store(T - 1, rows[c], st[rows[c] * nt], st[(NX + tri(rows[c], rows[c])) * nt]);
         if (T >= 2) issue(T - 2, ((T - 2) & 1) ? stage1 : stage0);
+        else if constexpr (kStats) issue(-1, stage1);
     }
 
     uint32_t status[1] = {0};
     const Real e1 = kMpc ? exp_minus_one(prm.dt) : Real(0);
-    for (long long t = T - 2; t >= 0; --t) {
-        cp_async_wait_all();
-        __syncthreads();  // stage t has landed; xs_{t+1}, Ps_{t+1} are written and the previous step's W has been read
-        const Real *st = (t & 1) ? stage1 : stage0;
-        if (t > 0) issue(t - 1, (t & 1) ? stage0 : stage1);  // that stage was step t + 1's, read before the barrier
-
-        // P-_{t+1}, as the forward pass's predict of step t + 1 formed it
-        Real Pm[NP];
+    // P-_{t+1}, as the forward pass's predict of step t + 1 formed it, from stage t; B: the blocks of F - 1 1^T (mpc: E) or F - I
+    // (predict: dt R^T) on the attitude rows
+    const auto prior = [&](const Real *st, Real (&Pm)[NP], Real (&B)[9]) {
 #pragma unroll
         for (int k = 0; k < NP; ++k) Pm[k] = st[(NX + k) * nt];
-        Real B[9];  // the blocks of F - 1 1^T (mpc: E) or F - I (predict: dt R^T) on the attitude rows
         if constexpr (kMpc) {
             const Real *ref = st + (2 * NX + NP) * nt;
             Real Rb[9];
@@ -150,10 +206,39 @@ __global__ void __launch_bounds__(RTSF_THREADS, 2) kf_rts_full_kernel(const __gr
                 for (int k = 0; k < 3; ++k) B[3 * a + k] = prm.dt * R[3 * k + a];
             cov_predict_sym<false>(Pm, R, prm.dt, qg, qs);
         }
+    };
+    const Real *zs = kStats ? prm.z + s : nullptr;  // z of this trajectory's stream
+    Real accw[3], accv[RTSF_SV_SLOTS], ll_quad = Real(0), det_m = Real(1);  // E-step accumulators of this warp's rows
+    int det_e = 0;
+    uint32_t ll_bad[1] = {0};
+#pragma unroll
+    for (int c = 0; c < 3; ++c) accw[c] = Real(0);
+#pragma unroll
+    for (int c = 0; c < RTSF_SV_SLOTS; ++c) accv[c] = Real(0);
+    for (long long t = T - 2; t >= (kStats ? -1 : 0); --t) {
+        cp_async_wait_all();
+        __syncthreads();  // stage t has landed; xs_{t+1}, Ps_{t+1} are written and the previous step's W has been read
+        const Real *st = (t & 1) ? stage1 : stage0;
+        if (t > 0) issue(t - 1, (t & 1) ? stage0 : stage1);  // that stage was step t + 1's, read before the barrier
+        else if constexpr (kStats) {
+            if (t == 0) issue(-1, stage1);
+        }
+
+        Real Pm[NP], B[9];
+        prior(st, Pm, B);
         // dPs = Ps_{t+1} - P-_{t+1}: warp q owns the entries k = q mod 4
 #pragma unroll
         for (int k = 0; k < NP; ++k)
-            if ((k & 3) == q) ps[k * nt] -= Pm[k];
+            if ((k & 3) == q) {
+                if constexpr (kStats) {
+                    const int j = rtsf_sv_of(k);  // Sv of measurement row j: (z_{t+1,j} - xs_{t+1,sel(j)})^2 + Ps_{t+1,sel(j)sel(j)}
+                    if (j >= 0) {
+                        const Real e = ld_stream(zs + ((t + 1) * NZ + j) * prm.S) - xsm[sel(j) * nt];
+                        accv[rtsf_sv_slot(j)] += fma_(e, e, ps[k * nt]);
+                    }
+                }
+                ps[k * nt] -= Pm[k];
+            }
 
         // P- = L D L^T in place: L[i][j] (i > j) at tri(i, j), D[j] at tri(j, j)
         Real dinv[NX];
@@ -177,6 +262,28 @@ __global__ void __launch_bounds__(RTSF_THREADS, 2) kf_rts_full_kernel(const __gr
             }
         }
 
+        if constexpr (kStats) {
+            // columns rows[c] of M = (P-)^-1 = L^-T D^-1 L^-1, parked in this warp's slots of W until dPs is complete
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                Real m[NX];
+#pragma unroll
+                for (int u = 0; u < NX; ++u) {
+                    Real v = u == rows[c] ? Real(1) : Real(0);
+#pragma unroll
+                    for (int k = 0; k < u; ++k) v = fnma_(Pm[tri(u, k)], m[k], v);
+                    m[u] = v;
+                }
+#pragma unroll
+                for (int u = 0; u < NX; ++u) m[u] *= dinv[u];
+#pragma unroll
+                for (int u = NX - 2; u >= 0; --u)
+#pragma unroll
+                    for (int k = u + 1; k < NX; ++k) m[u] = fnma_(Pm[tri(k, u)], m[k], m[u]);
+#pragma unroll
+                for (int u = 0; u < NX; ++u) W[(u * NX + rows[c]) * nt] = m[u];
+            }
+        }
         // this warp's columns of C = F P+, then G^T = (P-)^-1 C on them
         Real Gt[NX][3];
 #pragma unroll
@@ -226,6 +333,15 @@ __global__ void __launch_bounds__(RTSF_THREADS, 2) kf_rts_full_kernel(const __gr
             }
         }
         __syncthreads();  // dPs complete
+        Real m[kStats ? 3 : 1][NX], quad[3];  // E-step: this warp's columns of M and m^T dPs m
+        if constexpr (kStats) {
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                quad[c] = Real(0);
+#pragma unroll
+                for (int u = 0; u < NX; ++u) m[c][u] = W[(u * NX + rows[c]) * nt];
+            }
+        }
 #pragma unroll
         for (int k = 0; k < NX; ++k) {
             Real dk[NX];
@@ -236,7 +352,24 @@ __global__ void __launch_bounds__(RTSF_THREADS, 2) kf_rts_full_kernel(const __gr
                 Real v = dk[0] * Gt[0][c];
 #pragma unroll
                 for (int l = 1; l < NX; ++l) v = fma_(dk[l], Gt[l][c], v);
+                if constexpr (kStats) {
+                    Real h = dk[0] * m[c][0];
+#pragma unroll
+                    for (int l = 1; l < NX; ++l) h = fma_(dk[l], m[c][l], h);
+                    quad[c] = fma_(m[c][k], h, quad[c]);
+                }
                 W[(k * NX + rows[c]) * nt] = v;
+            }
+        }
+        if constexpr (kStats) {
+            // Sw: E[w_u^2 | Z] = q_u + q_u^2 ((M dPs M)_uu + (M d)_u^2), d = xs_{t+1} - x-_{t+1}
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                Real md = Real(0);
+#pragma unroll
+                for (int u = 0; u < NX; ++u) md = fma_(m[c][u], xsm[u * nt] - st[(NX + NP + u) * nt], md);
+                const Real qc = qg[rows[c] * qs];
+                accw[c] += fma_(qc * qc, fma_(md, md, quad[c]), qc);
             }
         }
         __syncthreads();  // W complete, dPs read
@@ -256,12 +389,68 @@ __global__ void __launch_bounds__(RTSF_THREADS, 2) kf_rts_full_kernel(const __gr
             xsm[r * nt] = xn[c];
             store(t, r, xn[c], diag);
         }
+        if constexpr (kStats) {
+            if (q == RTSF_LL_WARP) {
+                // log N(z_{t+1}; H x-_{t+1}, S), S = H P-_{t+1} H^T + R: P- once more, then L D L^T of S solved on the innovation
+                Real y[NZ];
+#pragma unroll
+                for (int j = 0; j < NZ; ++j) y[j] = ld_stream(zs + ((t + 1) * NZ + j) * prm.S) - st[(NX + NP + sel(j)) * nt];
+                Real Sm[NP], Bl[9];
+                prior(st, Sm, Bl);
+                Real yq = Real(0);
+#pragma unroll
+                for (int j = 0; j < NZ; ++j) {
+                    const int sj = sel(j);
+                    Real e[NZ];  // e[k] = L[j][k] D[k]
+#pragma unroll
+                    for (int k = 0; k < j; ++k) e[k] = Sm[tri(sj, sel(k))] * Sm[tri(sel(k), sel(k))];
+                    Real dj = Sm[tri(sj, sj)] + __ldg(prm.r_kind == OPTI_KF_MAT_DIAG ? prm.R + j : prm.R + j * N + ic);
+#pragma unroll
+                    for (int k = 0; k < j; ++k) dj = fnma_(e[k], Sm[tri(sj, sel(k))], dj);
+                    note_bad_pivot(dj, ll_bad, EM_BAD_PIVOT);
+                    Sm[tri(sj, sj)] = dj;
+                    const Real inv = rcp_(dj);
+#pragma unroll
+                    for (int r = j + 1; r < NZ; ++r) {
+                        Real v = Sm[tri(sel(r), sj)];
+#pragma unroll
+                        for (int k = 0; k < j; ++k) v = fnma_(Sm[tri(sel(r), sel(k))], e[k], v);
+                        Sm[tri(sel(r), sj)] = v * inv;
+                    }
+                    Real yj = y[j];
+#pragma unroll
+                    for (int k = 0; k < j; ++k) yj = fnma_(Sm[tri(sj, sel(k))], y[k], yj);
+                    y[j] = yj;
+                    yq = fma_(yj * inv, yj, yq);
+                    det_m *= dj;
+                    det_renorm(det_m, det_e);
+                }
+                ll_quad = fma_(Real(-0.5), yq, ll_quad);
+            }
+        }
+    }
+    if constexpr (kStats) {
+        if (active) {
+#pragma unroll
+            for (int c = 0; c < 3; ++c) prm.stats[rows[c] * N + i] = accw[c];
+#pragma unroll
+            for (int k = 0; k < NZ; ++k)
+                if (rtsf_sv_warp(k) == q) prm.stats[(NX + k) * N + i] = accv[rtsf_sv_slot(k)];
+            if (q == RTSF_LL_WARP) {
+                // -0.5 (10 T log 2 pi + log det) + the accumulated -0.5 y^T S^-1 y; a bad pivot of S makes it NaN
+                const double log_det = log((double)det_m) + (double)det_e * 0.69314718055994530942;
+                const double ll = (double)ll_quad - 0.5 * (log_det + (double)(NZ * T) * 1.83787706640934548356);
+                prm.stats[(EM_STATS_ROWS - 1) * N + i] = ll_bad[0] ? Real(NAN) : (Real)ll;
+            }
+        }
     }
     if (q == 0 && active && status[0] && prm.status) prm.status[i] |= status[0];
 }
 
-// Launch of kf_rts_full_kernel<Real, mpc> (instantiated in kf_smooth_full.cu for double and float).
+// Launches of kf_rts_full_kernel<Real, mpc> and <Real, mpc, true> (instantiated in kf_smooth_full.cu for double and float).
 template <typename Real>
 int launch_rts_full(const SmoothFullParams<Real> &p, cudaStream_t stream);
+template <typename Real>
+int launch_em_stats_full(const SmoothFullParams<Real> &p, cudaStream_t stream);
 
 }  // namespace okf

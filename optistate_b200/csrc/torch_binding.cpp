@@ -212,14 +212,17 @@ int64_t kf_smooth_full(const std::map<std::string, int64_t> &cfg, const std::map
 }
 
 // E-step of EM: the filter's tensors as for kf_batch, plus stats [23][N], optional x_smooth / var_smooth [T][12][N] and em_storage
-// (uint8, optistate_kf_noise_em_storage_bytes; cfg query_storage = 1 returns that size instead of running).
-int64_t kf_noise_em_stats(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
+// (uint8, the entry's storage query; cfg query_storage = 1 returns that size instead of running).  kf_noise_em_stats and
+// kf_noise_em_full_stats differ only in the two entry points.
+using EmStatsFn = int (*)(const OptiKfNoiseEmDesc *, void *);
+int64_t run_noise_em_stats(SmoothStorageFn storage_bytes, EmStatsFn em_stats, const std::map<std::string, int64_t> &cfg,
+                           const std::map<std::string, double> &consts, const TensorMap &tensors) {
     OptiKfDesc d;
     const c10::Device dev = filter_desc(cfg, consts, tensors, d);
     const c10::cuda::CUDAGuard guard(dev);
     if (geti(cfg, "query_storage", 0)) {
         size_t bytes = 0;
-        const int rc = optistate_kf_noise_em_storage_bytes(&d, &bytes);
+        const int rc = storage_bytes(&d, &bytes);
         return rc < 0 ? rc : (int64_t)bytes;
     }
     const Checker ck{d.dtype == OPTI_KF_F64 ? at::kDouble : at::kFloat, dev};
@@ -239,7 +242,17 @@ int64_t kf_noise_em_stats(const std::map<std::string, int64_t> &cfg, const std::
                 "optistate_b200: 'em_storage' must be a contiguous uint8 CUDA tensor");
     s.storage = t.data_ptr();
     s.storage_bytes = (size_t)t.numel();
-    return optistate_kf_noise_em_stats(&s, at::cuda::getCurrentCUDAStream().stream());
+    return em_stats(&s, at::cuda::getCurrentCUDAStream().stream());
+}
+
+int64_t kf_noise_em_stats(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
+    return run_noise_em_stats(optistate_kf_noise_em_storage_bytes, optistate_kf_noise_em_stats, cfg, consts, tensors);
+}
+
+// The E-step on the full covariance (optistate_kf_noise_em_full_stats): arguments as for kf_noise_em_stats.
+int64_t kf_noise_em_full_stats(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts,
+                               const TensorMap &tensors) {
+    return run_noise_em_stats(optistate_kf_noise_em_full_storage_bytes, optistate_kf_noise_em_full_stats, cfg, consts, tensors);
 }
 
 int kf_resolve_algo(const std::map<std::string, int64_t> &cfg) {
@@ -653,6 +666,7 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
     m.def("kf_smooth", &kf_smooth);
     m.def("kf_smooth_full", &kf_smooth_full);
     m.def("kf_noise_em_stats", &kf_noise_em_stats);
+    m.def("kf_noise_em_full_stats", &kf_noise_em_full_stats);
     m.def("kf_measure", &kf_measure);
     m.def("kf_class_step", &kf_class_step);
     m.def("kf_resolve_algo", &kf_resolve_algo);
