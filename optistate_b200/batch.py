@@ -13,6 +13,7 @@ can share a few input streams.
 """
 from __future__ import annotations
 
+import inspect
 from dataclasses import dataclass, field
 from typing import Dict, Iterable, Optional
 
@@ -191,18 +192,33 @@ class _FilterCall:
         return KfBatchResult(algo=_ALGO_NAMES[self.cfg["algo"]], n_traj=self.n_traj, n_steps=self.n_steps, tensors=res, status=self.status)
 
 
+def _out_tensor(out, name, shape, dtype, device) -> torch.Tensor:
+    """The caller's out[name], which must be `shape` `dtype`, or a new tensor."""
+    if out is not None and name in out:
+        if tuple(out[name].shape) != shape or out[name].dtype != dtype:
+            raise ValueError(f"out['{name}'] must be {shape} {dtype}")
+        return out[name]
+    return torch.empty(shape, dtype=dtype, device=device)
+
+
+def _scratch(out, key, nbytes: int, device) -> torch.Tensor:
+    """uint8 device scratch of at least nbytes (and at least 1): out[key] when large enough, else a new one kept in out[key] for
+    the caller's next call with the same shapes."""
+    t = out.get(key) if out is not None else None
+    if t is None or t.numel() < nbytes:
+        t = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=device)
+        if out is not None:
+            out[key] = t
+    return t
+
+
 def _attach_workspace(call: _FilterCall, out):
     """Scratch for the streamed SEQUENTIAL path (measurement pre-pass + TMA-fed kernel); 0 bytes when unused."""
     ws_bytes = call.ext.kf_batch(dict(call.cfg, query_workspace=1), call.consts, call.tensors)
     if ws_bytes < 0:
         nv.check(int(ws_bytes), "optistate_kf_workspace_bytes")
     if ws_bytes > 0:
-        ws = out.get("workspace") if out is not None else None
-        if ws is None or ws.numel() < ws_bytes:
-            ws = torch.empty(int(ws_bytes), dtype=torch.uint8, device=call.device)
-            if out is not None:
-                out["workspace"] = ws  # kept for the caller's next call with the same shapes
-        call.tensors["workspace"] = ws
+        call.tensors["workspace"] = _scratch(out, "workspace", int(ws_bytes), call.device)
 
 
 def _filter_call(imu, p, dp, contact, f, x0, P0, Q, R, *, n_traj, dtype, stream_index, stream_offset, outputs, ckpt_every, truth,
@@ -269,12 +285,8 @@ def _filter_call(imu, p, dp, contact, f, x0, P0, Q, R, *, n_traj, dtype, stream_
             if summary_peers.dtype != dtype or summary_peers.n_local != N or summary_peers.device != device:
                 raise ValueError("summary_peers was set up for another dtype, device or shard size")
             tensors[o] = summary_peers.tensor
-        elif out is not None and o in out:
-            if tuple(out[o].shape) != shape or out[o].dtype != dtype:
-                raise ValueError(f"out['{o}'] must be {shape} {dtype}")
-            tensors[o] = out[o]
         else:
-            tensors[o] = torch.empty(shape, dtype=dtype, device=device)
+            tensors[o] = _out_tensor(out, o, shape, dtype, device)
     status = out["status"] if out is not None and "status" in out else torch.zeros(N, dtype=torch.int32, device=device)
     tensors["status"] = status
 
@@ -297,43 +309,43 @@ def _filter_call(imu, p, dp, contact, f, x0, P0, Q, R, *, n_traj, dtype, stream_
 
 
 _SMOOTH_OUTPUTS = ("x_smooth", "var_smooth")
+EM_STATS_ROWS = 23
+EM_FIELDS = {"Sw": slice(0, 12), "Sv": slice(12, 22), "loglik": 22}
+_FILTER_SIGNATURE = inspect.signature(kf_batch)
 
 
-def kf_smooth(
-    imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *,
-    n_traj: Optional[int] = None, dtype: torch.dtype = torch.float64, stream_index=None, stream_offset: int = 0,
-    outputs: Iterable[str] = ("x_smooth",), ckpt_every: int = 0, truth=None, nominal=None, body_ref=None, z=None,
-    algo: str = "auto", cov_model: str = "predict", q_kind=None, r_kind=None, p0_kind=None,
-    dt: float = INITIAL_PARAMS.DT_mpc, mass: float = INITIAL_PARAMS.ROBOT_MASS, inertia=None,
-    gravity: float = INITIAL_PARAMS.GRAVITY, device=None, out: Optional[Dict[str, torch.Tensor]] = None,
-    summary_peers=None, p0_is_symmetric: Optional[bool] = None, structure: str = "auto", packed: bool = True,
-) -> KfBatchResult:
-    """Fixed-interval Rauch-Tung-Striebel smoother: runs the filter exactly as kf_batch runs it with the same arguments, then a
-    backward kernel that conditions every step's estimate on ALL measurements of the recording (offline use).
-
-    outputs: x_smooth [T,12,N] (smoothed state, the default), var_smooth [T,12,N] (diagonal of the smoothed covariance), and any
-    kf_batch output - those come from the same forward pass.  out: as for kf_batch, plus "smooth_storage" (uint8 scratch of
-    optistate_kf_smooth_storage_bytes: the packed posterior covariance of every step, 240 B per trajectory-step in FP64, and the
-    filter's x_steps / x_model_steps when they are not outputs), replaced in `out` when missing or too small.
-    Supported: the sequential algo with the predict() covariance model, diagonal Q and R and a P0 without entries across the
-    groups {th, w}, {x, vx}, {y, vy}, {z, vz}; anything else raises ValueError.  status gains OPTI_KF_ST_SMOOTH_NOT_PD (32).
-    """
-    call, smooth_want = _backward_call("kf_smooth", imu, p, dp, contact, f, x0, P0, Q, R, outputs, True, dict(
-        n_traj=n_traj, dtype=dtype, stream_index=stream_index, stream_offset=stream_offset, ckpt_every=ckpt_every, truth=truth,
-        nominal=nominal, body_ref=body_ref, z=z, algo=algo, cov_model=cov_model, q_kind=q_kind, r_kind=r_kind, p0_kind=p0_kind, dt=dt,
-        mass=mass, inertia=inertia, gravity=gravity, device=device, out=out, summary_peers=summary_peers,
-        p0_is_symmetric=p0_is_symmetric, structure=structure, packed=packed))
-    with torch.cuda.device(call.device):
-        _attach_workspace(call, out)
-        _attach_storage(call, out, call.ext.kf_smooth, "smooth_storage", "optistate_kf_smooth_storage_bytes")
-        nv.check(int(call.ext.kf_smooth(call.cfg, call.consts, call.tensors)), "optistate_kf_smooth")
-    return call.result(summary_peers, extra=smooth_want)
+@dataclass(frozen=True)
+class _Backward:
+    """One of the four backward passes over the sequential filter (include/optistate_kf.h)."""
+    who: str        # public name, in ValueErrors
+    entry: str      # binding; with cfg query_storage = 1 it returns the storage size instead of running
+    storage: str    # key of the library's scratch in `out`
+    c_run: str      # C entry and storage query, in nv.check messages
+    c_storage: str
+    full: bool      # the full-covariance kernel: either covariance model, any symmetric P0 (_filter_call refuses others)
+    stats: bool     # the E-step: noise_stats out, x_smooth optional
 
 
-def _backward_call(who, imu, p, dp, contact, f, x0, P0, Q, R, outputs, need_x_smooth, kw, full=False):
-    """The forward pass of kf_smooth / kf_noise_stats / kf_smooth_full / kf_noise_stats_full (_filter_call) with what the backward kernel refuses refused
-    here, and the smoothed outputs allocated: returns (call, smoothed output names).  full: the dense backward kernel, which takes
-    either covariance model and any symmetric P0 (a non-symmetric one is refused by _filter_call for algo='sequential')."""
+_KF_SMOOTH = _Backward("kf_smooth", "kf_smooth", "smooth_storage", "optistate_kf_smooth",
+                       "optistate_kf_smooth_storage_bytes", False, False)
+_KF_SMOOTH_FULL = _Backward("kf_smooth_full", "kf_smooth_full", "smooth_storage", "optistate_kf_smooth_full",
+                            "optistate_kf_smooth_full_storage_bytes", True, False)
+_KF_NOISE_STATS = _Backward("kf_noise_stats", "kf_noise_em_stats", "em_storage", "optistate_kf_noise_em_stats",
+                            "optistate_kf_noise_em_storage_bytes", False, True)
+_KF_NOISE_STATS_FULL = _Backward("kf_noise_stats_full", "kf_noise_em_full_stats", "em_storage", "optistate_kf_noise_em_full_stats",
+                                 "optistate_kf_noise_em_full_storage_bytes", True, True)
+
+
+def _run_backward(v: _Backward, args, outputs, kw) -> KfBatchResult:
+    """The forward pass (_filter_call, with kf_batch's keywords and defaults) with what the backward kernel refuses refused here,
+    the smoothed outputs, noise_stats and the library's storage attached, then the backward entry."""
+    try:
+        bound = _FILTER_SIGNATURE.bind(*args, **kw)
+    except TypeError as e:  # a keyword kf_batch does not take
+        raise TypeError(f"{v.who}() {e}") from None
+    bound.apply_defaults()
+    kw = bound.arguments
+    who, full = v.who, v.full
     if not full and kw["cov_model"] != "predict":
         raise ValueError(f"{who} supports the predict() covariance model only (predict_mpc makes F_d dense)")
     if not full and kw["structure"] != "auto":
@@ -342,10 +354,10 @@ def _backward_call(who, imu, p, dp, contact, f, x0, P0, Q, R, outputs, need_x_sm
         raise ValueError(f"{who} runs on the sequential filter; algo='joint' is not supported")
     outputs = list(outputs)
     smooth_want = [o for o in outputs if o in _SMOOTH_OUTPUTS]
-    if need_x_smooth and "x_smooth" not in smooth_want:
+    if not v.stats and "x_smooth" not in smooth_want:
         smooth_want.insert(0, "x_smooth")
-    kw = dict(kw, algo="sequential" if kw["algo"] == "auto" else kw["algo"])
-    call = _filter_call(imu, p, dp, contact, f, x0, P0, Q, R, outputs=[o for o in outputs if o not in _SMOOTH_OUTPUTS], **kw)
+    kw.update(outputs=[o for o in outputs if o not in _SMOOTH_OUTPUTS], algo="sequential" if kw["algo"] == "auto" else kw["algo"])
+    call = _filter_call(**kw)
     cfg = call.cfg
     if cfg["q_kind"] not in (nv.MAT_DIAG, nv.MAT_DIAG_PER) or cfg["r_kind"] not in (nv.MAT_DIAG, nv.MAT_DIAG_PER):
         raise ValueError(f"{who} needs diagonal Q and R " + ("(the sequential filter takes no dense noise)" if full else
@@ -354,30 +366,45 @@ def _backward_call(who, imu, p, dp, contact, f, x0, P0, Q, R, outputs, need_x_sm
         raise ValueError(f"{who} needs a P0 without entries across the groups {{th, w}}, {{x, vx}}, {{y, vy}}, {{z, vz}}")
     T, N, out, dtype = call.n_steps, call.n_traj, kw["out"], kw["dtype"]
     for o in smooth_want:
-        shape = (T, 12, N)
-        if out is not None and o in out:
-            if tuple(out[o].shape) != shape or out[o].dtype != dtype:
-                raise ValueError(f"out['{o}'] must be {shape} {dtype}")
-            call.tensors[o] = out[o]
-        else:
-            call.tensors[o] = torch.empty(shape, dtype=dtype, device=call.device)
-    return call, smooth_want
+        call.tensors[o] = _out_tensor(out, o, (T, 12, N), dtype, call.device)
+    extra = smooth_want
+    if v.stats:
+        call.tensors["noise_stats"] = _out_tensor(out, "noise_stats", (EM_STATS_ROWS, N), dtype, call.device)
+        extra = ["noise_stats", *smooth_want]
+    entry = getattr(call.ext, v.entry)
+    with torch.cuda.device(call.device):
+        _attach_workspace(call, out)
+        st_bytes = entry(dict(cfg, query_storage=1), call.consts, call.tensors)
+        nv.check(int(min(st_bytes, 0)), v.c_storage)
+        call.tensors[v.storage] = _scratch(out, v.storage, int(st_bytes), call.device)
+        nv.check(int(entry(cfg, call.consts, call.tensors)), v.c_run)
+    return call.result(kw["summary_peers"], extra=extra)
 
 
-def kf_smooth_full(
-    imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *,
-    n_traj: Optional[int] = None, dtype: torch.dtype = torch.float64, stream_index=None, stream_offset: int = 0,
-    outputs: Iterable[str] = ("x_smooth",), ckpt_every: int = 0, truth=None, nominal=None, body_ref=None, z=None,
-    algo: str = "auto", cov_model: str = "predict", q_kind=None, r_kind=None, p0_kind=None,
-    dt: float = INITIAL_PARAMS.DT_mpc, mass: float = INITIAL_PARAMS.ROBOT_MASS, inertia=None,
-    gravity: float = INITIAL_PARAMS.GRAVITY, device=None, out: Optional[Dict[str, torch.Tensor]] = None,
-    summary_peers=None, p0_is_symmetric: Optional[bool] = None, structure: str = "auto", packed: bool = True,
-) -> KfBatchResult:
+def kf_smooth(imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *, outputs: Iterable[str] = ("x_smooth",),
+              **kw) -> KfBatchResult:
+    """Fixed-interval Rauch-Tung-Striebel smoother: runs the filter exactly as kf_batch runs it with the same arguments, then a
+    backward kernel that conditions every step's estimate on ALL measurements of the recording (offline use).  The keywords
+    other than outputs are kf_batch's, with its defaults.
+
+    outputs: x_smooth [T,12,N] (smoothed state, the default), var_smooth [T,12,N] (diagonal of the smoothed covariance), and any
+    kf_batch output - those come from the same forward pass.  out: as for kf_batch, plus "smooth_storage" (uint8 scratch of
+    optistate_kf_smooth_storage_bytes: the packed posterior covariance of every step, 240 B per trajectory-step in FP64, and the
+    filter's x_steps / x_model_steps when they are not outputs), replaced in `out` when missing or too small.
+    Supported: the sequential algo with the predict() covariance model, diagonal Q and R and a P0 without entries across the
+    groups {th, w}, {x, vx}, {y, vy}, {z, vz}; anything else raises ValueError.  status gains OPTI_KF_ST_SMOOTH_NOT_PD (32).
+    """
+    return _run_backward(_KF_SMOOTH, (imu, p, dp, contact, f, x0, P0, Q, R), outputs, kw)
+
+
+def kf_smooth_full(imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *, outputs: Iterable[str] = ("x_smooth",),
+                   **kw) -> KfBatchResult:
     """The fixed-interval smoother of kf_smooth on the FULL 12x12 covariance (DESIGN.md section 0.2): for the predict_mpc
     covariance model (cov_model="mpc", whose element-wise F_d = exp(dt F) makes P dense) and for a P0 with entries across the
-    groups, which kf_smooth refuses.  Arguments, outputs (x_smooth, var_smooth and any kf_batch output) and out["smooth_storage"]
-    as for kf_smooth; the storage holds all 78 entries of P+ per step (624 B per trajectory-step in FP64).  The forward pass runs
-    the sequential filter's full-covariance kernels, whose outputs equal kf_batch's with the same arguments.
+    groups, which kf_smooth refuses.  Arguments (the keywords other than outputs are kf_batch's), outputs (x_smooth, var_smooth
+    and any kf_batch output) and out["smooth_storage"] as for kf_smooth; the storage holds all 78 entries of P+ per step (624 B
+    per trajectory-step in FP64).  The forward pass runs the sequential filter's full-covariance kernels, whose outputs equal
+    kf_batch's with the same arguments.
 
     The closed loop's output, smoothed offline:
 
@@ -388,99 +415,34 @@ def kf_smooth_full(
     predict_mpc model with identified noise P- reaches condition numbers near 1e8, which FP32 cannot resolve.
     status gains OPTI_KF_ST_SMOOTH_NOT_PD (32).
     """
-    call, smooth_want = _backward_call("kf_smooth_full", imu, p, dp, contact, f, x0, P0, Q, R, outputs, True, dict(
-        n_traj=n_traj, dtype=dtype, stream_index=stream_index, stream_offset=stream_offset, ckpt_every=ckpt_every, truth=truth,
-        nominal=nominal, body_ref=body_ref, z=z, algo=algo, cov_model=cov_model, q_kind=q_kind, r_kind=r_kind, p0_kind=p0_kind, dt=dt,
-        mass=mass, inertia=inertia, gravity=gravity, device=device, out=out, summary_peers=summary_peers,
-        p0_is_symmetric=p0_is_symmetric, structure=structure, packed=packed), full=True)
-    with torch.cuda.device(call.device):
-        _attach_workspace(call, out)
-        _attach_storage(call, out, call.ext.kf_smooth_full, "smooth_storage", "optistate_kf_smooth_full_storage_bytes")
-        nv.check(int(call.ext.kf_smooth_full(call.cfg, call.consts, call.tensors)), "optistate_kf_smooth_full")
-    return call.result(summary_peers, extra=smooth_want)
+    return _run_backward(_KF_SMOOTH_FULL, (imu, p, dp, contact, f, x0, P0, Q, R), outputs, kw)
 
 
-def _attach_storage(call: _FilterCall, out, entry, key, what):
-    """The backward pass's device scratch (size from the library), reused from / kept in `out[key]`."""
-    st_bytes = entry(dict(call.cfg, query_storage=1), call.consts, call.tensors)
-    nv.check(int(min(st_bytes, 0)), what)
-    st = out.get(key) if out is not None else None
-    if st is None or st.numel() < st_bytes:
-        st = torch.empty(max(int(st_bytes), 1), dtype=torch.uint8, device=call.device)
-        if out is not None:
-            out[key] = st  # kept for the caller's next call with the same shapes
-    call.tensors[key] = st
-
-
-EM_STATS_ROWS = 23
-EM_FIELDS = {"Sw": slice(0, 12), "Sv": slice(12, 22), "loglik": 22}
-
-
-def kf_noise_stats(
-    imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *,
-    n_traj: Optional[int] = None, dtype: torch.dtype = torch.float64, stream_index=None, stream_offset: int = 0,
-    outputs: Iterable[str] = (), ckpt_every: int = 0, truth=None, nominal=None, body_ref=None, z=None,
-    algo: str = "auto", cov_model: str = "predict", q_kind=None, r_kind=None, p0_kind=None,
-    dt: float = INITIAL_PARAMS.DT_mpc, mass: float = INITIAL_PARAMS.ROBOT_MASS, inertia=None,
-    gravity: float = INITIAL_PARAMS.GRAVITY, device=None, out: Optional[Dict[str, torch.Tensor]] = None,
-    summary_peers=None, p0_is_symmetric: Optional[bool] = None, structure: str = "auto", packed: bool = True,
-) -> KfBatchResult:
+def kf_noise_stats(imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *, outputs: Iterable[str] = (),
+                   **kw) -> KfBatchResult:
     """E-step of expectation-maximisation for diagonal Q and R (DESIGN.md section 0): runs the filter and the smoother's backward
     kernel exactly as kf_smooth does with the same arguments, and returns `noise_stats` [23, N] per trajectory:
         rows 0-11   Sw = sum_t E[w_t^2 | Z]   over the T transitions t = -1 .. T-2 (x_{-1} ~ N(x0, P0), P0 = Q when None)
         rows 12-21  Sv = sum_t E[v_t^2 | Z]   over the T measurements
         row 22      the prediction-error log-likelihood sum_t log N(z_t; H x-_t, H P-_t H^T + R) of the filter that ran
-    The M-step is Q = diag(Sw) / T, R = diag(Sv) / T (kf_noise_em).  outputs: x_smooth, var_smooth and any kf_batch output, all
-    optional.  out: as for kf_smooth, with "noise_stats" and "em_storage" (uint8 scratch of optistate_kf_noise_em_storage_bytes).
-    Refuses what kf_smooth refuses, with the same ValueErrors.
+    The M-step is Q = diag(Sw) / T, R = diag(Sv) / T (kf_noise_em).  The keywords other than outputs are kf_batch's, with its
+    defaults.  outputs: x_smooth, var_smooth and any kf_batch output, all optional.  out: as for kf_smooth, with "noise_stats" and
+    "em_storage" (uint8 scratch of optistate_kf_noise_em_storage_bytes).  Refuses what kf_smooth refuses, with the same ValueErrors.
     """
-    call, smooth_want = _backward_call("kf_noise_stats", imu, p, dp, contact, f, x0, P0, Q, R, outputs, False, dict(
-        n_traj=n_traj, dtype=dtype, stream_index=stream_index, stream_offset=stream_offset, ckpt_every=ckpt_every, truth=truth,
-        nominal=nominal, body_ref=body_ref, z=z, algo=algo, cov_model=cov_model, q_kind=q_kind, r_kind=r_kind, p0_kind=p0_kind, dt=dt,
-        mass=mass, inertia=inertia, gravity=gravity, device=device, out=out, summary_peers=summary_peers,
-        p0_is_symmetric=p0_is_symmetric, structure=structure, packed=packed))
-    return _noise_stats_run(call, smooth_want, out, dtype, summary_peers, "kf_noise_em_stats", "optistate_kf_noise_em_stats")
+    return _run_backward(_KF_NOISE_STATS, (imu, p, dp, contact, f, x0, P0, Q, R), outputs, kw)
 
 
-def kf_noise_stats_full(
-    imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *,
-    n_traj: Optional[int] = None, dtype: torch.dtype = torch.float64, stream_index=None, stream_offset: int = 0,
-    outputs: Iterable[str] = (), ckpt_every: int = 0, truth=None, nominal=None, body_ref=None, z=None,
-    algo: str = "auto", cov_model: str = "predict", q_kind=None, r_kind=None, p0_kind=None,
-    dt: float = INITIAL_PARAMS.DT_mpc, mass: float = INITIAL_PARAMS.ROBOT_MASS, inertia=None,
-    gravity: float = INITIAL_PARAMS.GRAVITY, device=None, out: Optional[Dict[str, torch.Tensor]] = None,
-    summary_peers=None, p0_is_symmetric: Optional[bool] = None, structure: str = "auto", packed: bool = True,
-) -> KfBatchResult:
+def kf_noise_stats_full(imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *, outputs: Iterable[str] = (),
+                        **kw) -> KfBatchResult:
     """The E-step of kf_noise_stats on the FULL covariance (DESIGN.md section 0.3): the forward pass and backward kernel of
     kf_smooth_full, so the predict_mpc covariance model (cov_model="mpc", with body_ref) and a coupled or dense symmetric P0 are
-    taken.  Returns `noise_stats` [23, N] with the rows of kf_noise_stats (the innovation covariance of the log-likelihood is the
-    dense H P- H^T + R), and x_smooth / var_smooth or any kf_batch output when asked for.  out: as for kf_smooth_full, with
-    "noise_stats" and "em_storage" (optistate_kf_noise_em_full_storage_bytes).  Refuses what kf_smooth_full refuses: algo="joint",
-    dense Q or R and a non-symmetric P0 raise ValueError.
+    taken.  The keywords other than outputs are kf_batch's, with its defaults.  Returns `noise_stats` [23, N] with the rows of
+    kf_noise_stats (the innovation covariance of the log-likelihood is the dense H P- H^T + R), and x_smooth / var_smooth or any
+    kf_batch output when asked for.  out: as for kf_smooth_full, with "noise_stats" and "em_storage"
+    (optistate_kf_noise_em_full_storage_bytes).  Refuses what kf_smooth_full refuses: algo="joint", dense Q or R and a
+    non-symmetric P0 raise ValueError.
     """
-    call, smooth_want = _backward_call("kf_noise_stats_full", imu, p, dp, contact, f, x0, P0, Q, R, outputs, False, dict(
-        n_traj=n_traj, dtype=dtype, stream_index=stream_index, stream_offset=stream_offset, ckpt_every=ckpt_every, truth=truth,
-        nominal=nominal, body_ref=body_ref, z=z, algo=algo, cov_model=cov_model, q_kind=q_kind, r_kind=r_kind, p0_kind=p0_kind, dt=dt,
-        mass=mass, inertia=inertia, gravity=gravity, device=device, out=out, summary_peers=summary_peers,
-        p0_is_symmetric=p0_is_symmetric, structure=structure, packed=packed), full=True)
-    return _noise_stats_run(call, smooth_want, out, dtype, summary_peers, "kf_noise_em_full_stats", "optistate_kf_noise_em_full_stats")
-
-
-def _noise_stats_run(call, smooth_want, out, dtype, summary_peers, entry, what):
-    """The stats output and the E-step's storage attached to `call`, then the library's entry `what` (binding `entry`)."""
-    shape = (EM_STATS_ROWS, call.n_traj)
-    if out is not None and "noise_stats" in out:
-        if tuple(out["noise_stats"].shape) != shape or out["noise_stats"].dtype != dtype:
-            raise ValueError(f"out['noise_stats'] must be {shape} {dtype}")
-        call.tensors["noise_stats"] = out["noise_stats"]
-    else:
-        call.tensors["noise_stats"] = torch.empty(shape, dtype=dtype, device=call.device)
-    with torch.cuda.device(call.device):
-        _attach_workspace(call, out)
-        fn = getattr(call.ext, entry)
-        _attach_storage(call, out, fn, "em_storage", what.replace("_stats", "_storage_bytes"))
-        nv.check(int(fn(call.cfg, call.consts, call.tensors)), what)
-    return call.result(summary_peers, extra=("noise_stats", *smooth_want))
+    return _run_backward(_KF_NOISE_STATS_FULL, (imu, p, dp, contact, f, x0, P0, Q, R), outputs, kw)
 
 
 @dataclass
@@ -514,8 +476,9 @@ def kf_noise_em(
     tol: stop once the largest relative increase of the log-likelihood (per trajectory; pooled with shared=True) falls below
     it - one host synchronisation per iteration, only when tol is given.  Storage and workspace are reused across iterations.
     """
-    return _noise_em("kf_noise_em", kf_noise_stats, {}, imu, p, dp, contact, f, x0, P0, Q, R, iters, tol, shared, n_traj, dtype,
-                     stream_index, stream_offset, z, dt, mass, inertia, gravity, device, out)
+    return _noise_em("kf_noise_em", kf_noise_stats, (imu, p, dp, contact, f, x0, P0, Q, R), dict(
+        n_traj=n_traj, dtype=dtype, stream_index=stream_index, stream_offset=stream_offset, z=z, dt=dt, mass=mass, inertia=inertia,
+        gravity=gravity, device=device, out=out), iters, tol, shared)
 
 
 def kf_noise_em_full(
@@ -540,19 +503,21 @@ def kf_noise_em_full(
     under predict_mpc that model is further from the mean model: F_d = 1 1^T + D is not the mean model's Jacobian, so Q absorbs
     the difference and is not the process noise of the robot.  FP64 is the dtype for real data (kf_smooth_full).
     """
-    return _noise_em("kf_noise_em_full", kf_noise_stats_full, dict(cov_model=cov_model, body_ref=body_ref), imu, p, dp, contact, f,
-                     x0, P0, Q, R, iters, tol, shared, n_traj, dtype, stream_index, stream_offset, z, dt, mass, inertia, gravity,
-                     device, out)
+    return _noise_em("kf_noise_em_full", kf_noise_stats_full, (imu, p, dp, contact, f, x0, P0, Q, R), dict(
+        n_traj=n_traj, dtype=dtype, stream_index=stream_index, stream_offset=stream_offset, z=z, cov_model=cov_model,
+        body_ref=body_ref, dt=dt, mass=mass, inertia=inertia, gravity=gravity, device=device, out=out), iters, tol, shared)
 
 
-def _noise_em(who, stats_fn, extra, imu, p, dp, contact, f, x0, P0, Q, R, iters, tol, shared, n_traj, dtype, stream_index,
-              stream_offset, z, dt, mass, inertia, gravity, device, out) -> KfNoiseEmResult:
-    """The EM loop of kf_noise_em / kf_noise_em_full around the E-step stats_fn (extra: its further keyword arguments)."""
+def _noise_em(who, stats_fn, args, filter_kw, iters, tol, shared) -> KfNoiseEmResult:
+    """The EM loop of kf_noise_em / kf_noise_em_full around the E-step stats_fn, which gets the filter's arguments args
+    (imu .. R) and keywords filter_kw with the current Q, R and P0."""
     if iters < 1:
         raise ValueError("iters must be >= 1")
     nv.require_cuda()
-    out = {} if out is None else out  # storage and workspace of the first E-step, reused by the others
-    device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    imu, p, dp, contact, f, x0, P0, Q, R = args
+    n_traj, dtype, z = filter_kw["n_traj"], filter_kw["dtype"], filter_kw["z"]
+    out = {} if filter_kw["out"] is None else filter_kw["out"]  # storage and workspace of the first E-step, reused by the others
+    device = torch.device("cuda", torch.cuda.current_device()) if filter_kw["device"] is None else torch.device(filter_kw["device"])
     base = z if z is not None else imu
     T, S = int(base.shape[0]), int(base.shape[2]) if base.ndim == 3 else 1
     N = int(S if n_traj is None else n_traj)
@@ -576,11 +541,10 @@ def _noise_em(who, stats_fn, extra, imu, p, dp, contact, f, x0, P0, Q, R, iters,
     kind = nv.MAT_DIAG if shared else nv.MAT_DIAG_PER
     p0, p0_kind = (q.clone(), kind) if P0 is None else (P0, None)
     status = torch.zeros(N, dtype=torch.int32, device=device)
+    kw = dict(filter_kw, n_traj=N, device=device, out=out, q_kind=kind, r_kind=kind, p0_kind=p0_kind)
     lls, converged, prev = [], False, None
     for it in range(iters):
-        res = stats_fn(imu, p, dp, contact, f, x0, p0, q, r, n_traj=N, dtype=dtype, stream_index=stream_index,
-                       stream_offset=stream_offset, z=z, q_kind=kind, r_kind=kind, p0_kind=p0_kind, dt=dt, mass=mass, inertia=inertia,
-                       gravity=gravity, device=device, out=out, **extra)
+        res = stats_fn(imu, p, dp, contact, f, x0, p0, q, r, **kw)
         st = res.noise_stats
         status |= res.status
         ll = st[EM_STATS_ROWS - 1].clone()

@@ -4,6 +4,7 @@
 #include <atomic>
 #include <cstdlib>
 #include <cstring>
+#include <type_traits>
 
 #include "kf_features.cuh"
 #include "kf_identify.cuh"
@@ -318,11 +319,20 @@ int fma_peak(long long fma_per_thread, double *flops_out, double *seconds_out, c
     return OPTI_KF_OK;
 }
 
-// ---- fixed-interval smoother ------------------------------------------------------------------------------------
-// What the backward kernel can take: the decoupled-group form of the SEQUENTIAL filter (kf_smooth.cuh).
-int smooth_check(const OptiKfDesc *d) {
+// ---- the backward passes over the SEQUENTIAL filter: smoother and EM E-step ------------------------------------------
+// full: the full-covariance kernel (all 78 entries of P+, SmoothFullParams, kf_rts_full_kernel) instead of the decoupled one
+// (30 packed entries, SmoothParams, kf_rts_kernel); stats: the E-step of EM, which accepts exactly what its smoother accepts.
+struct Backward {
+    bool full, stats;
+};
+
+// What the backward kernels can take.  Decoupled: the decoupled-group form of the SEQUENTIAL filter (kf_smooth.cuh).  Full:
+// whatever the SEQUENTIAL filter runs (AUTO means SEQUENTIAL here, as the symmetric P0 this entry requires permits), in either
+// covariance model and with any P0 kind.
+int backward_check(const OptiKfDesc *d, bool full) {
     const int rc = validate(d);
     if (rc != OPTI_KF_OK) return rc;
+    if (full) return d->algo != OPTI_KF_ALGO_JOINT && sequential_ok(d) ? OPTI_KF_OK : OPTI_KF_E_UNSUPPORTED;
     if (d->cov_model != OPTI_KF_COV_PREDICT || (d->flags & OPTI_KF_FLAG_FULL_COVARIANCE)) return OPTI_KF_E_UNSUPPORTED;
     if (!is_diag_kind(d->q_kind) || !is_diag_kind(d->r_kind)) return OPTI_KF_E_UNSUPPORTED;
     const bool p0_groups = d->p0_kind == OPTI_KF_MAT_NONE || is_diag_kind(d->p0_kind) || (d->flags & OPTI_KF_FLAG_P0_DECOUPLED);
@@ -332,166 +342,110 @@ int smooth_check(const OptiKfDesc *d) {
     return algo == OPTI_KF_ALGO_SEQUENTIAL ? OPTI_KF_OK : OPTI_KF_E_UNSUPPORTED;
 }
 
-// Scratch of the smoother, each part padded to 256 bytes: P+ [T][np][N] at 0 (np = 30 packed decoupled entries, or all 78 for
-// optistate_kf_smooth_full), then x+ and x- [T][12][N] unless the filter descriptor has x_steps / x_model_steps (the smoother
-// reads those).  Byte offsets.
-struct SmoothStorage {
-    size_t x_post, x_prior, total;
-    explicit SmoothStorage(const OptiKfDesc *d, int np = okf::NPB) {
+// Scratch of the backward passes, each part padded to 256 bytes: P+ [T][np][N] at 0 (np = 30 packed decoupled entries, or all
+// 78 when full), then x+ and x- [T][12][N] unless the filter descriptor has x_steps / x_model_steps (the backward kernel reads
+// those), then for the E-step z [T][10][S] when the filter forms the measurements.  Byte offsets.
+struct BackwardStorage {
+    size_t x_post, x_prior, z, total;
+    BackwardStorage(const OptiKfDesc *d, Backward v) {
         const auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
         const size_t esz = d->dtype == OPTI_KF_F64 ? 8 : 4, tn = (size_t)d->n_steps * (size_t)d->n_traj;
-        x_post = up(tn * (size_t)np * esz);
+        const size_t ts = (size_t)d->n_steps * (size_t)d->n_streams;
+        x_post = up(tn * (size_t)(v.full ? okf::NP : okf::NPB) * esz);
         x_prior = x_post + (d->x_steps ? 0 : up(tn * okf::NX * esz));
-        total = x_prior + (d->x_model_steps ? 0 : up(tn * okf::NX * esz));
+        z = x_prior + (d->x_model_steps ? 0 : up(tn * okf::NX * esz));
+        total = z + (v.stats && (d->phases & OPTI_KF_PHASE_MEASURE) ? up(ts * okf::NZ * esz) : 0);
     }
 };
 
+// The forward pass, with x+ / x- in the storage where the caller did not ask for them, then the backward kernel.  A full pass runs
+// the full-covariance filter kernels whatever the caller's flags, so P+ is [T][78][N] (on decoupled inputs they are bit-identical
+// to the kBlock ones, kf_seq_core.cuh).
 template <typename Real>
-int smooth(const OptiKfSmoothDesc *s, cudaStream_t stream) {
-    const OptiKfDesc *f = s->filter;
-    const SmoothStorage ss(f);
-    unsigned char *base = (unsigned char *)s->storage;
-    OptiKfDesc fw = *f;  // the forward pass, with x+ / x- in the storage where the caller did not ask for them
-    if (!fw.x_steps && base) fw.x_steps = base + ss.x_post;
-    if (!fw.x_model_steps && base) fw.x_model_steps = base + ss.x_prior;
-    int rc = launch<Real>(&fw, OPTI_KF_ALGO_SEQUENTIAL, stream, base);
-    if (rc != OPTI_KF_OK) return rc;
-    if (f->n_traj == 0 || f->n_steps == 0) return OPTI_KF_OK;
-    okf::SmoothParams<Real> p;
-    std::memset(&p, 0, sizeof p);
-    p.N = f->n_traj; p.T = f->n_steps; p.dt = (Real)f->dt;
-    p.Q = (const Real *)f->Q; p.q_kind = f->q_kind;
-    p.x_post = (const Real *)fw.x_steps; p.x_prior = (const Real *)fw.x_model_steps; p.P_post = (const Real *)base;
-    p.x_smooth = (Real *)s->x_smooth; p.var_smooth = (Real *)s->var_smooth; p.status = f->status;
-    rc = okf::launch_rts<Real>(p, stream);
-    if (rc < 0) return rc;
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return cudaGetLastError() == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
-}
-
-// What the full-covariance smoother can take: whatever the SEQUENTIAL filter runs (AUTO means SEQUENTIAL here, as the symmetric
-// P0 this entry requires permits), in either covariance model and with any P0 kind.
-int smooth_full_check(const OptiKfDesc *d) {
-    const int rc = validate(d);
-    if (rc != OPTI_KF_OK) return rc;
-    return d->algo != OPTI_KF_ALGO_JOINT && sequential_ok(d) ? OPTI_KF_OK : OPTI_KF_E_UNSUPPORTED;
-}
-
-// The forward pass always runs the full-covariance kernels, so P+ is [T][78][N] whatever the caller's flags (on decoupled inputs
-// they are bit-identical to the kBlock ones, kf_seq_core.cuh).
-template <typename Real>
-int smooth_full(const OptiKfSmoothDesc *s, cudaStream_t stream) {
-    const OptiKfDesc *f = s->filter;
-    const SmoothStorage ss(f, okf::NP);
-    unsigned char *base = (unsigned char *)s->storage;
+int run_backward(Backward v, const OptiKfDesc *f, void *storage, void *x_smooth, void *var_smooth, void *stats, cudaStream_t stream) {
+    const BackwardStorage st(f, v);
+    unsigned char *base = (unsigned char *)storage;
     OptiKfDesc fw = *f;
-    fw.flags |= OPTI_KF_FLAG_FULL_COVARIANCE;
-    if (!fw.x_steps && base) fw.x_steps = base + ss.x_post;
-    if (!fw.x_model_steps && base) fw.x_model_steps = base + ss.x_prior;
-    int rc = launch<Real>(&fw, OPTI_KF_ALGO_SEQUENTIAL, stream, base);
-    if (rc != OPTI_KF_OK) return rc;
-    if (f->n_traj == 0 || f->n_steps == 0) return OPTI_KF_OK;
-    okf::SmoothFullParams<Real> p;
-    std::memset(&p, 0, sizeof p);
-    p.N = f->n_traj; p.T = f->n_steps; p.dt = (Real)f->dt; p.cov_model = f->cov_model;
-    p.Q = (const Real *)f->Q; p.q_kind = f->q_kind;
-    p.x_post = (const Real *)fw.x_steps; p.x_prior = (const Real *)fw.x_model_steps; p.P_post = (const Real *)base;
-    p.body_ref = (const Real *)f->body_ref; p.S = f->n_streams; p.stream_offset = f->stream_offset; p.stream_index = f->stream_index;
-    p.x_smooth = (Real *)s->x_smooth; p.var_smooth = (Real *)s->var_smooth; p.status = f->status;
-    rc = okf::launch_rts_full<Real>(p, stream);
-    if (rc < 0) return rc;
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return cudaGetLastError() == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
-}
-
-// Scratch of the EM statistics: the smoother's (np as for SmoothStorage), then z [T][10][S] (padded to 256 bytes) when the filter
-// forms the measurements.
-struct EmStorage {
-    size_t z, total;
-    explicit EmStorage(const OptiKfDesc *d, int np = okf::NPB) {
-        const size_t esz = d->dtype == OPTI_KF_F64 ? 8 : 4, ts = (size_t)d->n_steps * (size_t)d->n_streams;
-        z = SmoothStorage(d, np).total;
-        total = z + ((d->phases & OPTI_KF_PHASE_MEASURE) ? ((ts * okf::NZ * esz + 255) & ~(size_t)255) : 0);
-    }
-};
-
-template <typename Real>
-int noise_em_stats(const OptiKfNoiseEmDesc *s, cudaStream_t stream) {
-    const OptiKfDesc *f = s->filter;
-    const SmoothStorage ss(f);
-    const EmStorage es(f);
-    unsigned char *base = (unsigned char *)s->storage;
-    OptiKfDesc fw = *f;  // the forward pass, as in smooth()
-    if (!fw.x_steps && base) fw.x_steps = base + ss.x_post;
-    if (!fw.x_model_steps && base) fw.x_model_steps = base + ss.x_prior;
+    if (v.full) fw.flags |= OPTI_KF_FLAG_FULL_COVARIANCE;
+    if (!fw.x_steps && base) fw.x_steps = base + st.x_post;
+    if (!fw.x_model_steps && base) fw.x_model_steps = base + st.x_prior;
     int rc = launch<Real>(&fw, OPTI_KF_ALGO_SEQUENTIAL, stream, base);
     if (rc != OPTI_KF_OK) return rc;
     const long long N = f->n_traj, T = f->n_steps;
-    if (N == 0) return OPTI_KF_OK;
+    if (N == 0 || (T == 0 && !v.stats)) return OPTI_KF_OK;
     if (T == 0)  // no transition and no measurement: every sum is empty
-        return cudaMemsetAsync(s->stats, 0, (size_t)okf::EM_STATS_ROWS * N * sizeof(Real), stream) == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
+        return cudaMemsetAsync(stats, 0, (size_t)okf::EM_STATS_ROWS * N * sizeof(Real), stream) == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
     const Real *z = (const Real *)f->z_in;
-    if (f->phases & OPTI_KF_PHASE_MEASURE) {  // the filter formed z in-kernel: form it once more, per stream, with the same function
-        z = (const Real *)(base + es.z);
+    if (v.stats && (f->phases & OPTI_KF_PHASE_MEASURE)) {  // the filter formed z in-kernel: form it once more, per stream, with the same function
+        z = (const Real *)(base + st.z);
         launch_measure<Real>(T, f->n_streams, (const Real *)f->imu, (const Real *)f->p, (const Real *)f->dp, (const Real *)f->contact,
                              nullptr, (Real *)z, nullptr, nullptr, nullptr, stream);
     }
-    okf::SmoothParams<Real> p;
-    std::memset(&p, 0, sizeof p);
-    p.N = N; p.T = T; p.dt = (Real)f->dt;
-    p.Q = (const Real *)f->Q; p.q_kind = f->q_kind;
-    p.x_post = (const Real *)fw.x_steps; p.x_prior = (const Real *)fw.x_model_steps; p.P_post = (const Real *)base;
-    p.x_smooth = (Real *)s->x_smooth; p.var_smooth = (Real *)s->var_smooth; p.status = f->status;
-    p.z = z; p.S = f->n_streams; p.stream_offset = f->stream_offset; p.stream_index = f->stream_index;
-    p.R = (const Real *)f->R; p.r_kind = f->r_kind;
-    p.x0 = (const Real *)f->x0; p.x0_ld = f->x0_per_traj ? N : 1; p.x0_inc = f->x0_per_traj ? 1 : 0;
-    p.P0 = (const Real *)f->P0; p.p0_kind = f->p0_kind;
-    p.stats = (Real *)s->stats;
-    rc = okf::launch_em_stats<Real>(p, stream);
+    const auto fill = [&](auto &p) {  // the fields SmoothParams and SmoothFullParams share; the E-step's stay zero for the smoother
+        std::memset(&p, 0, sizeof p);
+        p.N = N; p.T = T; p.dt = (Real)f->dt;
+        p.Q = (const Real *)f->Q; p.q_kind = f->q_kind;
+        p.x_post = (const Real *)fw.x_steps; p.x_prior = (const Real *)fw.x_model_steps; p.P_post = (const Real *)base;
+        p.x_smooth = (Real *)x_smooth; p.var_smooth = (Real *)var_smooth; p.status = f->status;
+        if (v.full || v.stats) {  // the stream a trajectory reads z (E-step) and body_ref (full) from
+            p.S = f->n_streams; p.stream_offset = f->stream_offset; p.stream_index = f->stream_index;
+        }
+        if (v.stats) {
+            p.z = z;
+            p.R = (const Real *)f->R; p.r_kind = f->r_kind;
+            p.x0 = (const Real *)f->x0; p.x0_ld = f->x0_per_traj ? N : 1; p.x0_inc = f->x0_per_traj ? 1 : 0;
+            p.P0 = (const Real *)f->P0; p.p0_kind = f->p0_kind;
+            p.stats = (Real *)stats;
+        }
+    };
+    if (v.full) {
+        okf::SmoothFullParams<Real> p;
+        fill(p);
+        p.cov_model = f->cov_model; p.body_ref = (const Real *)f->body_ref;
+        rc = v.stats ? okf::launch_rts_full<Real, true>(p, stream) : okf::launch_rts_full<Real, false>(p, stream);
+    } else {
+        okf::SmoothParams<Real> p;
+        fill(p);
+        rc = v.stats ? okf::launch_rts<Real, true>(p, stream) : okf::launch_rts<Real, false>(p, stream);
+    }
     if (rc < 0) return rc;
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError() == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
 }
 
-// The E-step on the full covariance: the forward pass of smooth_full(), then kf_rts_full_kernel<Real, mpc, true>.
-template <typename Real>
-int noise_em_full_stats(const OptiKfNoiseEmDesc *s, cudaStream_t stream) {
-    const OptiKfDesc *f = s->filter;
-    const SmoothStorage ss(f, okf::NP);
-    const EmStorage es(f, okf::NP);
-    unsigned char *base = (unsigned char *)s->storage;
-    OptiKfDesc fw = *f;
-    fw.flags |= OPTI_KF_FLAG_FULL_COVARIANCE;
-    if (!fw.x_steps && base) fw.x_steps = base + ss.x_post;
-    if (!fw.x_model_steps && base) fw.x_model_steps = base + ss.x_prior;
-    int rc = launch<Real>(&fw, OPTI_KF_ALGO_SEQUENTIAL, stream, base);
+int backward_storage_bytes(const OptiKfDesc *filter, Backward v, size_t *bytes_out) {
+    const int rc = backward_check(filter, v.full);
     if (rc != OPTI_KF_OK) return rc;
-    const long long N = f->n_traj, T = f->n_steps;
-    if (N == 0) return OPTI_KF_OK;
-    if (T == 0)
-        return cudaMemsetAsync(s->stats, 0, (size_t)okf::EM_STATS_ROWS * N * sizeof(Real), stream) == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
-    const Real *z = (const Real *)f->z_in;
-    if (f->phases & OPTI_KF_PHASE_MEASURE) {
-        z = (const Real *)(base + es.z);
-        launch_measure<Real>(T, f->n_streams, (const Real *)f->imu, (const Real *)f->p, (const Real *)f->dp, (const Real *)f->contact,
-                             nullptr, (Real *)z, nullptr, nullptr, nullptr, stream);
+    if (!bytes_out) return OPTI_KF_E_NULL;
+    *bytes_out = BackwardStorage(filter, v).total;
+    return OPTI_KF_OK;
+}
+
+// The entries' envelope, codes in the order the header documents: the descriptor, the filter, the required output (the smoother's
+// x_smooth, the E-step's stats), then the storage.
+template <typename Desc>
+int backward_entry(const Desc *desc, bool full, void *cuda_stream) {
+    constexpr bool stats = std::is_same<Desc, OptiKfNoiseEmDesc>::value;
+    if (!desc) return OPTI_KF_E_NULL;
+    if (desc->struct_size != sizeof(Desc) || desc->abi_version != OPTISTATE_KF_ABI_VERSION) return OPTI_KF_E_VERSION;
+    if (!desc->filter) return OPTI_KF_E_NULL;
+    const OptiKfDesc *f = desc->filter;
+    const int rc = backward_check(f, full);
+    if (rc != OPTI_KF_OK) return rc;
+    const bool steps = f->n_traj > 0 && f->n_steps > 0;  // empty batches carry empty (NULL) arrays
+    void *out_stats = nullptr;
+    if constexpr (stats) {
+        out_stats = desc->stats;
+        if (f->n_traj > 0 && !out_stats) return OPTI_KF_E_NULL;
+    } else {
+        if (steps && !desc->x_smooth) return OPTI_KF_E_NULL;
     }
-    okf::SmoothFullParams<Real> p;
-    std::memset(&p, 0, sizeof p);
-    p.N = N; p.T = T; p.dt = (Real)f->dt; p.cov_model = f->cov_model;
-    p.Q = (const Real *)f->Q; p.q_kind = f->q_kind;
-    p.x_post = (const Real *)fw.x_steps; p.x_prior = (const Real *)fw.x_model_steps; p.P_post = (const Real *)base;
-    p.body_ref = (const Real *)f->body_ref; p.S = f->n_streams; p.stream_offset = f->stream_offset; p.stream_index = f->stream_index;
-    p.x_smooth = (Real *)s->x_smooth; p.var_smooth = (Real *)s->var_smooth; p.status = f->status;
-    p.z = z;
-    p.R = (const Real *)f->R; p.r_kind = f->r_kind;
-    p.x0 = (const Real *)f->x0; p.x0_ld = f->x0_per_traj ? N : 1; p.x0_inc = f->x0_per_traj ? 1 : 0;
-    p.P0 = (const Real *)f->P0; p.p0_kind = f->p0_kind;
-    p.stats = (Real *)s->stats;
-    rc = okf::launch_em_stats_full<Real>(p, stream);
-    if (rc < 0) return rc;
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return cudaGetLastError() == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
+    const Backward v{full, stats};
+    if (desc->storage_bytes < BackwardStorage(f, v).total) return OPTI_KF_E_SHAPE;
+    if (steps && !desc->storage) return OPTI_KF_E_NULL;
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    return f->dtype == OPTI_KF_F64 ? run_backward<double>(v, f, desc->storage, desc->x_smooth, desc->var_smooth, out_stats, stream)
+                                   : run_backward<float>(v, f, desc->storage, desc->x_smooth, desc->var_smooth, out_stats, stream);
 }
 
 template <typename Real>
@@ -539,94 +493,24 @@ int optistate_kf_workspace_bytes(const OptiKfDesc *desc, size_t *bytes_out) {
 }
 
 int optistate_kf_smooth_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out) {
-    const int rc = smooth_check(filter);
-    if (rc != OPTI_KF_OK) return rc;
-    if (!bytes_out) return OPTI_KF_E_NULL;
-    *bytes_out = SmoothStorage(filter).total;
-    return OPTI_KF_OK;
+    return backward_storage_bytes(filter, {false, false}, bytes_out);
 }
-
-int optistate_kf_smooth(const OptiKfSmoothDesc *desc, void *cuda_stream) {
-    if (!desc) return OPTI_KF_E_NULL;
-    if (desc->struct_size != sizeof(OptiKfSmoothDesc) || desc->abi_version != OPTISTATE_KF_ABI_VERSION) return OPTI_KF_E_VERSION;
-    if (!desc->filter) return OPTI_KF_E_NULL;
-    const int rc = smooth_check(desc->filter);
-    if (rc != OPTI_KF_OK) return rc;
-    const OptiKfDesc *f = desc->filter;
-    const bool steps = f->n_traj > 0 && f->n_steps > 0;  // empty batches carry empty (NULL) arrays
-    if (steps && !desc->x_smooth) return OPTI_KF_E_NULL;
-    if (desc->storage_bytes < SmoothStorage(f).total) return OPTI_KF_E_SHAPE;
-    if (steps && !desc->storage) return OPTI_KF_E_NULL;
-    cudaStream_t stream = (cudaStream_t)cuda_stream;
-    return f->dtype == OPTI_KF_F64 ? smooth<double>(desc, stream) : smooth<float>(desc, stream);
-}
+int optistate_kf_smooth(const OptiKfSmoothDesc *desc, void *cuda_stream) { return backward_entry(desc, false, cuda_stream); }
 
 int optistate_kf_smooth_full_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out) {
-    const int rc = smooth_full_check(filter);
-    if (rc != OPTI_KF_OK) return rc;
-    if (!bytes_out) return OPTI_KF_E_NULL;
-    *bytes_out = SmoothStorage(filter, okf::NP).total;
-    return OPTI_KF_OK;
+    return backward_storage_bytes(filter, {true, false}, bytes_out);
 }
-
-int optistate_kf_smooth_full(const OptiKfSmoothDesc *desc, void *cuda_stream) {
-    if (!desc) return OPTI_KF_E_NULL;
-    if (desc->struct_size != sizeof(OptiKfSmoothDesc) || desc->abi_version != OPTISTATE_KF_ABI_VERSION) return OPTI_KF_E_VERSION;
-    if (!desc->filter) return OPTI_KF_E_NULL;
-    const int rc = smooth_full_check(desc->filter);
-    if (rc != OPTI_KF_OK) return rc;
-    const OptiKfDesc *f = desc->filter;
-    const bool steps = f->n_traj > 0 && f->n_steps > 0;
-    if (steps && !desc->x_smooth) return OPTI_KF_E_NULL;
-    if (desc->storage_bytes < SmoothStorage(f, okf::NP).total) return OPTI_KF_E_SHAPE;
-    if (steps && !desc->storage) return OPTI_KF_E_NULL;
-    cudaStream_t stream = (cudaStream_t)cuda_stream;
-    return f->dtype == OPTI_KF_F64 ? smooth_full<double>(desc, stream) : smooth_full<float>(desc, stream);
-}
+int optistate_kf_smooth_full(const OptiKfSmoothDesc *desc, void *cuda_stream) { return backward_entry(desc, true, cuda_stream); }
 
 int optistate_kf_noise_em_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out) {
-    const int rc = smooth_check(filter);
-    if (rc != OPTI_KF_OK) return rc;
-    if (!bytes_out) return OPTI_KF_E_NULL;
-    *bytes_out = EmStorage(filter).total;
-    return OPTI_KF_OK;
+    return backward_storage_bytes(filter, {false, true}, bytes_out);
 }
-
-int optistate_kf_noise_em_stats(const OptiKfNoiseEmDesc *desc, void *cuda_stream) {
-    if (!desc) return OPTI_KF_E_NULL;
-    if (desc->struct_size != sizeof(OptiKfNoiseEmDesc) || desc->abi_version != OPTISTATE_KF_ABI_VERSION) return OPTI_KF_E_VERSION;
-    if (!desc->filter) return OPTI_KF_E_NULL;
-    const int rc = smooth_check(desc->filter);
-    if (rc != OPTI_KF_OK) return rc;
-    const OptiKfDesc *f = desc->filter;
-    if (f->n_traj > 0 && !desc->stats) return OPTI_KF_E_NULL;
-    if (desc->storage_bytes < EmStorage(f).total) return OPTI_KF_E_SHAPE;
-    if (f->n_traj > 0 && f->n_steps > 0 && !desc->storage) return OPTI_KF_E_NULL;
-    cudaStream_t stream = (cudaStream_t)cuda_stream;
-    return f->dtype == OPTI_KF_F64 ? noise_em_stats<double>(desc, stream) : noise_em_stats<float>(desc, stream);
-}
+int optistate_kf_noise_em_stats(const OptiKfNoiseEmDesc *desc, void *cuda_stream) { return backward_entry(desc, false, cuda_stream); }
 
 int optistate_kf_noise_em_full_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out) {
-    const int rc = smooth_full_check(filter);
-    if (rc != OPTI_KF_OK) return rc;
-    if (!bytes_out) return OPTI_KF_E_NULL;
-    *bytes_out = EmStorage(filter, okf::NP).total;
-    return OPTI_KF_OK;
+    return backward_storage_bytes(filter, {true, true}, bytes_out);
 }
-
-int optistate_kf_noise_em_full_stats(const OptiKfNoiseEmDesc *desc, void *cuda_stream) {
-    if (!desc) return OPTI_KF_E_NULL;
-    if (desc->struct_size != sizeof(OptiKfNoiseEmDesc) || desc->abi_version != OPTISTATE_KF_ABI_VERSION) return OPTI_KF_E_VERSION;
-    if (!desc->filter) return OPTI_KF_E_NULL;
-    const int rc = smooth_full_check(desc->filter);
-    if (rc != OPTI_KF_OK) return rc;
-    const OptiKfDesc *f = desc->filter;
-    if (f->n_traj > 0 && !desc->stats) return OPTI_KF_E_NULL;
-    if (desc->storage_bytes < EmStorage(f, okf::NP).total) return OPTI_KF_E_SHAPE;
-    if (f->n_traj > 0 && f->n_steps > 0 && !desc->storage) return OPTI_KF_E_NULL;
-    cudaStream_t stream = (cudaStream_t)cuda_stream;
-    return f->dtype == OPTI_KF_F64 ? noise_em_full_stats<double>(desc, stream) : noise_em_full_stats<float>(desc, stream);
-}
+int optistate_kf_noise_em_full_stats(const OptiKfNoiseEmDesc *desc, void *cuda_stream) { return backward_entry(desc, true, cuda_stream); }
 
 int optistate_kf_batch(const OptiKfDesc *desc, void *cuda_stream) {
     const int rc = validate(desc);

@@ -430,10 +430,8 @@ __global__ void __launch_bounds__(RTS_THREADS) kf_rts_kernel(const __grid_consta
     if (status[0] && prm.status) prm.status[i] |= status[0];
 }
 
-// Launches of kf_rts_kernel<Real, false> and <Real, true> (instantiated in kf_smooth.cu for double and float).
-template <typename Real>
+// Launch of kf_rts_kernel<Real, kStats> (instantiated in kf_smooth.cu for double and float).
+template <typename Real, bool kStats>
 int launch_rts(const SmoothParams<Real> &p, cudaStream_t stream);
-template <typename Real>
-int launch_em_stats(const SmoothParams<Real> &p, cudaStream_t stream);
 
 }  // namespace okf

@@ -447,10 +447,8 @@ __global__ void __launch_bounds__(RTSF_THREADS, 2) kf_rts_full_kernel(const __gr
     if (q == 0 && active && status[0] && prm.status) prm.status[i] |= status[0];
 }
 
-// Launches of kf_rts_full_kernel<Real, mpc> and <Real, mpc, true> (instantiated in kf_smooth_full.cu for double and float).
-template <typename Real>
+// Launch of kf_rts_full_kernel<Real, mpc, kStats> (instantiated in kf_smooth_full.cu for double and float).
+template <typename Real, bool kStats>
 int launch_rts_full(const SmoothFullParams<Real> &p, cudaStream_t stream);
-template <typename Real>
-int launch_em_stats_full(const SmoothFullParams<Real> &p, cudaStream_t stream);
 
 }  // namespace okf

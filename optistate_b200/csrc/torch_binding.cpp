@@ -8,6 +8,7 @@
 #include <map>
 #include <optional>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/optistate_kf.h"
@@ -168,13 +169,14 @@ int64_t kf_batch(const std::map<std::string, int64_t> &cfg, const std::map<std::
     return optistate_kf_batch(&d, at::cuda::getCurrentCUDAStream().stream());
 }
 
-// Fixed-interval smoother: the filter's tensors as for kf_batch, plus x_smooth [T][12][N], optional var_smooth [T][12][N] and
-// smooth_storage (uint8, the entry's storage query; cfg query_storage = 1 returns that size instead of running).  kf_smooth and
-// kf_smooth_full differ only in the two entry points.
-using SmoothStorageFn = int (*)(const OptiKfDesc *, size_t *);
-using SmoothFn = int (*)(const OptiKfSmoothDesc *, void *);
-int64_t run_smooth(SmoothStorageFn storage_bytes, SmoothFn smooth, const std::map<std::string, int64_t> &cfg,
-                   const std::map<std::string, double> &consts, const TensorMap &tensors) {
+// The backward passes: the filter's tensors as for kf_batch, plus the smoother's x_smooth [T][12][N] (required) or the E-step's
+// noise_stats [23][N] (required; x_smooth optional), optional var_smooth [T][12][N], and the uint8 storage of the entry's
+// storage query, smooth_storage or em_storage (cfg query_storage = 1 returns that size instead of running).  Desc:
+// OptiKfSmoothDesc or OptiKfNoiseEmDesc.
+template <typename Desc>
+int64_t run_backward(int (*storage_bytes)(const OptiKfDesc *, size_t *), int (*entry)(const Desc *, void *),
+                     const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
+    constexpr bool stats = std::is_same<Desc, OptiKfNoiseEmDesc>::value;
     OptiKfDesc d;
     const c10::Device dev = filter_desc(cfg, consts, tensors, d);
     const c10::cuda::CUDAGuard guard(dev);
@@ -185,74 +187,37 @@ int64_t run_smooth(SmoothStorageFn storage_bytes, SmoothFn smooth, const std::ma
     }
     const Checker ck{d.dtype == OPTI_KF_F64 ? at::kDouble : at::kFloat, dev};
     const int64_t N = d.n_traj, T = d.n_steps;
-    OptiKfSmoothDesc s;
+    Desc s;
     std::memset(&s, 0, sizeof s);
     s.struct_size = sizeof s;
     s.abi_version = OPTISTATE_KF_ABI_VERSION;
     s.filter = &d;
-    s.x_smooth = const_cast<void *>(ck.get(tensors, "x_smooth", T * 12 * N, true));
+    if constexpr (stats) s.stats = const_cast<void *>(ck.get(tensors, "noise_stats", OPTI_KF_EM_STATS_ROWS * N, true));
+    s.x_smooth = const_cast<void *>(ck.get(tensors, "x_smooth", T * 12 * N, !stats));
     s.var_smooth = const_cast<void *>(ck.get(tensors, "var_smooth", T * 12 * N, false));
-    auto is = tensors.find("smooth_storage");
-    TORCH_CHECK(is != tensors.end(), "optistate_b200: missing tensor 'smooth_storage'");
+    const std::string key = stats ? "em_storage" : "smooth_storage";
+    auto is = tensors.find(key);
+    TORCH_CHECK(is != tensors.end(), "optistate_b200: missing tensor '", key, "'");
     const at::Tensor &t = is->second;
     TORCH_CHECK(t.is_cuda() && t.device() == dev && t.scalar_type() == at::kByte && t.is_contiguous(),
-                "optistate_b200: 'smooth_storage' must be a contiguous uint8 CUDA tensor");
+                "optistate_b200: '", key, "' must be a contiguous uint8 CUDA tensor");
     s.storage = t.data_ptr();
     s.storage_bytes = (size_t)t.numel();
-    return smooth(&s, at::cuda::getCurrentCUDAStream().stream());
+    return entry(&s, at::cuda::getCurrentCUDAStream().stream());
 }
 
 int64_t kf_smooth(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
-    return run_smooth(optistate_kf_smooth_storage_bytes, optistate_kf_smooth, cfg, consts, tensors);
+    return run_backward(optistate_kf_smooth_storage_bytes, optistate_kf_smooth, cfg, consts, tensors);
 }
-
-// The full-covariance smoother (optistate_kf_smooth_full): arguments as for kf_smooth.
 int64_t kf_smooth_full(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
-    return run_smooth(optistate_kf_smooth_full_storage_bytes, optistate_kf_smooth_full, cfg, consts, tensors);
+    return run_backward(optistate_kf_smooth_full_storage_bytes, optistate_kf_smooth_full, cfg, consts, tensors);
 }
-
-// E-step of EM: the filter's tensors as for kf_batch, plus stats [23][N], optional x_smooth / var_smooth [T][12][N] and em_storage
-// (uint8, the entry's storage query; cfg query_storage = 1 returns that size instead of running).  kf_noise_em_stats and
-// kf_noise_em_full_stats differ only in the two entry points.
-using EmStatsFn = int (*)(const OptiKfNoiseEmDesc *, void *);
-int64_t run_noise_em_stats(SmoothStorageFn storage_bytes, EmStatsFn em_stats, const std::map<std::string, int64_t> &cfg,
-                           const std::map<std::string, double> &consts, const TensorMap &tensors) {
-    OptiKfDesc d;
-    const c10::Device dev = filter_desc(cfg, consts, tensors, d);
-    const c10::cuda::CUDAGuard guard(dev);
-    if (geti(cfg, "query_storage", 0)) {
-        size_t bytes = 0;
-        const int rc = storage_bytes(&d, &bytes);
-        return rc < 0 ? rc : (int64_t)bytes;
-    }
-    const Checker ck{d.dtype == OPTI_KF_F64 ? at::kDouble : at::kFloat, dev};
-    const int64_t N = d.n_traj, T = d.n_steps;
-    OptiKfNoiseEmDesc s;
-    std::memset(&s, 0, sizeof s);
-    s.struct_size = sizeof s;
-    s.abi_version = OPTISTATE_KF_ABI_VERSION;
-    s.filter = &d;
-    s.stats = const_cast<void *>(ck.get(tensors, "noise_stats", OPTI_KF_EM_STATS_ROWS * N, true));
-    s.x_smooth = const_cast<void *>(ck.get(tensors, "x_smooth", T * 12 * N, false));
-    s.var_smooth = const_cast<void *>(ck.get(tensors, "var_smooth", T * 12 * N, false));
-    auto is = tensors.find("em_storage");
-    TORCH_CHECK(is != tensors.end(), "optistate_b200: missing tensor 'em_storage'");
-    const at::Tensor &t = is->second;
-    TORCH_CHECK(t.is_cuda() && t.device() == dev && t.scalar_type() == at::kByte && t.is_contiguous(),
-                "optistate_b200: 'em_storage' must be a contiguous uint8 CUDA tensor");
-    s.storage = t.data_ptr();
-    s.storage_bytes = (size_t)t.numel();
-    return em_stats(&s, at::cuda::getCurrentCUDAStream().stream());
-}
-
 int64_t kf_noise_em_stats(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
-    return run_noise_em_stats(optistate_kf_noise_em_storage_bytes, optistate_kf_noise_em_stats, cfg, consts, tensors);
+    return run_backward(optistate_kf_noise_em_storage_bytes, optistate_kf_noise_em_stats, cfg, consts, tensors);
 }
-
-// The E-step on the full covariance (optistate_kf_noise_em_full_stats): arguments as for kf_noise_em_stats.
 int64_t kf_noise_em_full_stats(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts,
                                const TensorMap &tensors) {
-    return run_noise_em_stats(optistate_kf_noise_em_full_storage_bytes, optistate_kf_noise_em_full_stats, cfg, consts, tensors);
+    return run_backward(optistate_kf_noise_em_full_storage_bytes, optistate_kf_noise_em_full_stats, cfg, consts, tensors);
 }
 
 int kf_resolve_algo(const std::map<std::string, int64_t> &cfg) {
