@@ -49,17 +49,17 @@ def skew(v):
     return np.array([[0, -v[2], v[1]], [v[2], 0, -v[0]], [-v[1], v[0], 0]])
 
 
-def dynamics(th, p):
+def dynamics(th, p, *, mass=MASS, inertia=INERTIA):
     """A (force_controller.py:179-192) and B (:194-224) for reference angles th (3) and body-frame feet p (12)."""
     R = rot_zyx(*th)
     A = np.zeros((12, 12))
     A[0:3, 6:9] = R.T
     A[3:6, 9:12] = np.eye(3)
-    I_hat_inv = np.linalg.inv(R @ np.diag(INERTIA) @ R.T)
+    I_hat_inv = np.linalg.inv(R @ np.diag(np.asarray(inertia, float)) @ R.T)
     B = np.zeros((12, 12))
     for leg in range(4):
         B[6:9, 3 * leg:3 * leg + 3] = I_hat_inv @ skew(R @ p[3 * leg:3 * leg + 3])
-        B[9:12, 3 * leg:3 * leg + 3] = np.eye(3) / MASS
+        B[9:12, 3 * leg:3 * leg + 3] = np.eye(3) / mass
     return A, B
 
 
@@ -70,33 +70,43 @@ def horizon(x, body_ref, p):
     return body, feet
 
 
-def rollout_cost(u, x, body_ref, p, dt=0.01):
+def _grav(gravity):
+    """The gravity vector of the dynamics: `gravity` on the z velocity (force_controller.py:28)."""
+    g = np.zeros(12)
+    g[11] = gravity
+    return g
+
+
+def rollout_cost(u, x, body_ref, p, dt=0.01, *, mass=MASS, inertia=INERTIA, gravity=GRAV[11], w_state=Q_W, w_force=R_W):
     """The reference's objective loop, literally (force_controller.py:70-104).  u: (12, NH) forces per stage."""
     body, feet = horizon(x, body_ref, p)
     u = np.asarray(u, float).reshape(12, NH)
-    Q, R, P = np.diag(Q_W), R_W * np.eye(12), np.diag(Q_W)
+    w = np.asarray(w_state, float)
+    Q, R, P = np.diag(w), w_force * np.eye(12), np.diag(w)
+    grav = _grav(gravity)
     state, cost = body[:, 0].copy(), 0.0
     for i in range(NH):
-        A, B = dynamics(body[0:3, i], feet[:, i])
-        state = (np.eye(12) + A * dt) @ state + (B * dt) @ u[:, i] + dt * GRAV
+        A, B = dynamics(body[0:3, i], feet[:, i], mass=mass, inertia=inertia)
+        state = (np.eye(12) + A * dt) @ state + (B * dt) @ u[:, i] + dt * grav
         e = state - body[:, i + 1]
         cost += e @ (P if i == NH - 1 else Q) @ e + u[:, i] @ R @ u[:, i]
     return cost
 
 
-def build_qp(x, body_ref, p, dt=0.01):
+def build_qp(x, body_ref, p, dt=0.01, *, mass=MASS, inertia=INERTIA, gravity=GRAV[11], w_state=Q_W, w_force=R_W):
     """Condensed form: cost(u) = 1/2 u^T H u + g^T u + c0 with u = vec of the (12, NH) forces, stage-major (u[12 i + k])."""
     body, feet = horizon(x, body_ref, p)
     n = 12 * NH
     Su, sc = np.zeros((12, n)), body[:, 0].copy()
-    H, g, c0 = 2.0 * R_W * np.eye(n), np.zeros(n), 0.0
+    H, g, c0 = 2.0 * w_force * np.eye(n), np.zeros(n), 0.0
+    grav = _grav(gravity)
     for i in range(NH):
-        A, B = dynamics(body[0:3, i], feet[:, i])
+        A, B = dynamics(body[0:3, i], feet[:, i], mass=mass, inertia=inertia)
         Ad = np.eye(12) + A * dt
         Su = Ad @ Su
         Su[:, 12 * i:12 * i + 12] += B * dt
-        sc = Ad @ sc + dt * GRAV
-        W = np.diag(Q_W)  # P = Q
+        sc = Ad @ sc + dt * grav
+        W = np.diag(np.asarray(w_state, float))  # P = Q
         e = sc - body[:, i + 1]
         H += 2.0 * Su.T @ W @ Su
         g += 2.0 * Su.T @ W @ e
@@ -104,9 +114,9 @@ def build_qp(x, body_ref, p, dt=0.01):
     return H, g, c0
 
 
-def constraints(contact):
+def constraints(contact, *, mu=MU, fz_max=FZ_MAX):
     """A u <= b rows (and the index set of variables pinned to zero) for the contact pattern of all NH stages.
-    contact == 0: f = 0 (force_controller.py:110-123);  contact == 1: friction pyramid + 0 <= fz <= 150 (:125-156);
+    contact == 0: f = 0 (force_controller.py:110-123);  contact == 1: friction pyramid + 0 <= fz <= fz_max (:125-156);
     any other value: the reference's if_else selects neither, the leg is unconstrained."""
     contact = np.asarray(contact, float).reshape(4)
     rows, rhs, pinned = [], [], []
@@ -116,8 +126,8 @@ def constraints(contact):
             if contact[leg] == 0:
                 pinned += [k, k + 1, k + 2]
             elif contact[leg] == 1:
-                for coef, b in (((0, 0, -1.0), 0.0), ((0, 0, 1.0), FZ_MAX), ((1.0, 0, -MU), 0.0), ((-1.0, 0, -MU), 0.0),
-                                ((0, 1.0, -MU), 0.0), ((0, -1.0, -MU), 0.0)):
+                for coef, b in (((0, 0, -1.0), 0.0), ((0, 0, 1.0), fz_max), ((1.0, 0, -mu), 0.0), ((-1.0, 0, -mu), 0.0),
+                                ((0, 1.0, -mu), 0.0), ((0, -1.0, -mu), 0.0)):
                     r = np.zeros(12 * NH)
                     r[k:k + 3] = coef
                     rows.append(r)
@@ -177,8 +187,10 @@ def kkt_certificate(u, H, g, A, b, pinned, act_tol=1e-7):
     return viol, float(np.abs(grad + A[np.ix_(act, free)].T @ lam).max() / scale)
 
 
-def solve(x, body_ref, p, contact, dt=0.01):
-    """Forces (12, NH) of the reference's MPC for one problem."""
-    H, g, _ = build_qp(x, body_ref, p, dt)
-    A, b, pinned = constraints(contact)
+def solve(x, body_ref, p, contact, dt=0.01, *, mass=MASS, inertia=INERTIA, gravity=GRAV[11], mu=MU, fz_max=FZ_MAX, w_state=Q_W,
+          w_force=R_W):
+    """Forces (12, NH) of the reference's MPC for one problem.  The keyword constants default to the reference's (module
+    constants above); they are the call arguments of optistate_b200.mpc.mpc_forces of the same names."""
+    H, g, _ = build_qp(x, body_ref, p, dt, mass=mass, inertia=inertia, gravity=gravity, w_state=w_state, w_force=w_force)
+    A, b, pinned = constraints(contact, mu=mu, fz_max=fz_max)
     return solve_ldp(H, g, A, b, pinned).reshape(NH, 12).T
