@@ -9,8 +9,8 @@
 //     streams, so one copy feeds all of them and a block of four needs 12 KB of FP64 input tiles instead of 47 KB.
 //     That is what decides occupancy: with a tile per warp the decoupled-group kernels (168 registers, three blocks per
 //     SM by registers) were held to two blocks by 108 KB of shared memory; with the shared tile three blocks fit
-//     (ncu: launch__occupancy_limit_shared_mem).  The warp that is LAST to finish reading a group (a shared-memory
-//     counter) issues the refill, so nobody waits on a designated producer.
+//     (ncu: launch__occupancy_limit_shared_mem).  The warp that is LAST to finish reading a group (a ticket drawn from a
+//     shared-memory counter) issues the refill, so nobody waits on a designated producer.
 //   * Three channel groups, each single-buffered and refilled for step t+1 the moment the block has consumed
 //     step t's copy, so the copy has most of a filter step (several microseconds) to land:
 //         G0 = M[12]            read at the top of the step (mean model)        -> refilled after the covariance predict (kBlock), else right away
@@ -97,11 +97,12 @@ __device__ __forceinline__ void tma_tile_g2s(void *dst, const CUtensorMap *map, 
 
 template <typename Real, int kThreads, int kNoiseRows = TMA_NOISE_ROWS, int kStages = 1>
 struct TmaSmem {
-    // dynamic shared memory: [mbarriers + counters 128 B][G0 [g0_rows][32] | G1 [10][32] | G2 [12*n_lab][32]] (kStages tile sets per
-    //                        block)  [noise [22 | 32][128]][acc [25][128] (8-byte sums; double and F2 kernels only)]   (elements: Real)
+    // dynamic shared memory: [mbarriers 128 B][election line 128 B][G0 [g0_rows][32] | G1 [10][32] | G2 [12*n_lab][32]] (kStages tile
+    //                        sets per block)  [noise [22 | 32][128]][acc [25][128] (8-byte sums; double and F2 kernels only)]   (elements: Real)
     static __host__ __device__ constexpr size_t warp_rows(int n_lab, int g0_rows) { return g0_rows + TMA_CH_G1 + 12 * n_lab; }
     static __host__ __device__ constexpr size_t warp_bytes(int n_lab, int g0_rows) { return warp_rows(n_lab, g0_rows) * 32 * sizeof(Real); }
-    static __host__ __device__ constexpr size_t off_in() { return 128; }
+    static __host__ __device__ constexpr size_t off_elect() { return 128; }
+    static __host__ __device__ constexpr size_t off_in() { return 256; }
     static __host__ __device__ constexpr size_t off_noise(int n_lab, int g0_rows) { return off_in() + kStages * warp_bytes(n_lab, g0_rows); }
     static __host__ __device__ constexpr size_t off_acc(int n_lab, int g0_rows) { return off_noise(n_lab, g0_rows) + (size_t)kNoiseRows * kThreads * sizeof(Real); }
     static __host__ __device__ constexpr size_t total(int n_lab, int g0_rows, bool acc_in_smem) {
@@ -159,6 +160,31 @@ __host__ __device__ constexpr bool tma_acc_in_smem() {
     return kSummary && sizeof(Real) == 8;
 }
 
+#ifdef OKF_ELECT_STAMPS
+// Diagnostic build (tools/probes/elect_stamps.py compiles ONE translation unit with it): lane 0 of every warp of the first
+// kStampBlocks blocks of a throughput-geometry launch writes clock64() at the top of each of steps [kStampT0, kStampT0 + kStampSteps),
+// before and after each of the three refill elections (election and copy issue) and at the end of the step, and each of those
+// blocks its SM, to the arrays below; okf_elect_stamps_read copies them out.  The stores change the schedule of the loop a little,
+// so its numbers are for the election, not for the kernel's rate.
+constexpr int kStampBlocks = 1024, kStampWarps = 4, kStampT0 = 400, kStampSteps = 16, kStampEvents = 8;
+enum StampEvent { kStTop, kStElect0, kStElect0End, kStElect1, kStElect1End, kStElect2, kStElect2End, kStEnd };
+__device__ long long okf_elect_stamps[kStampBlocks * kStampWarps * kStampSteps * kStampEvents];
+__device__ unsigned okf_elect_smid[kStampBlocks];
+extern "C" int okf_elect_stamps_read(long long *stamps, unsigned *smid) {
+    if (cudaMemcpyFromSymbol(stamps, okf_elect_stamps, sizeof(okf_elect_stamps)) != cudaSuccess) return 1;
+    return cudaMemcpyFromSymbol(smid, okf_elect_smid, sizeof(okf_elect_smid)) != cudaSuccess ? 1 : 0;
+}
+#define OKF_STAMP(ev)                                                                                                                 \
+    do {                                                                                                                              \
+        if (stamp_on && t >= kStampT0 && t < kStampT0 + kStampSteps)                                                                  \
+            okf_elect_stamps[((blockIdx.x * kStampWarps + warp) * kStampSteps + (t - kStampT0)) * kStampEvents + (ev)] = clock64(); \
+    } while (0)
+#else
+#define OKF_STAMP(ev) \
+    do {              \
+    } while (0)
+#endif
+
 // kW: warps per block; 0 = the throughput geometry above (tma_warps).  kW = 1 is the LATENCY variant, chosen by the host when there are
 // no more trajectories than streams (every block of the throughput geometry would hold one working warp - BASELINE configs[1],
 // 1,024 trajectories x 10,000 steps, is the case): a block is its one warp, so nobody counts readers (no shared-memory atomic, whose
@@ -199,7 +225,9 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
     const int n_lab = kSummary ? (prm.truth ? 1 : 0) + (prm.nominal ? 1 : 0) : 0;
 
     uint64_t *bars = reinterpret_cast<uint64_t *>(smem_raw);  // full[G0], full[G1], full[G2]
-    int *consumed = reinterpret_cast<int *>(smem_raw + 64);   // warps that have finished reading the current copy of G0, G1, G2
+    // election line: words 0-2 count the warps that have finished reading G0, G1, G2 (see last_reader); the rest is padding that
+    // the other lanes of an election touch
+    uint32_t *tickets = reinterpret_cast<uint32_t *>(smem_raw + Smem::off_elect());
     constexpr int kG0Rows = tma_g0_rows<kOut, kMpc>();
     Real *g0w = reinterpret_cast<Real *>(smem_raw + Smem::off_in());
     Real *g1w = g0w + kG0Rows * 32, *g2w = g1w + TMA_CH_G1 * 32;  // the block's [C][32] tiles (of Real)
@@ -211,9 +239,14 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
     if (tid == 0) {
 #pragma unroll
         for (int b = 0; b < 3 * kStages; ++b) mbar_init(&bars[b], 1);  // full[G0], full[G1], full[G2] of every tile set
-        consumed[0] = consumed[1] = consumed[2] = 0;
+        if constexpr (!kBlock) tickets[0] = tickets[1] = tickets[2] = 0;
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
+    if (kBlock && tid < 32) tickets[tid] = 0;
+#ifdef OKF_ELECT_STAMPS
+    const bool stamp_on = TMA_WARPS == kStampWarps && lane == 0 && blockIdx.x < kStampBlocks;
+    if (stamp_on && warp == 0) asm volatile("mov.u32 %0, %%smid;" : "=r"(okf_elect_smid[blockIdx.x]));
+#endif
     __syncthreads();
     if (!warp_active) return;  // fewer members than warps in the last group of a tile
     if (prm.T > 0 && warp == 0) {  // warp 0 of a block always has work
@@ -226,24 +259,49 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
             }
         }
     }
-    // A warp is done with group g of this step; the LAST warp of the block to get here refills the group for the next step.
-    // (The counter is reset before the copy is issued, and nobody can count for the next step before that copy has landed.)
-    const auto last_reader = [&](int g) -> int {
+    // A warp is done with group g of step t; the LAST warp of the block to get here refills the group for the next step.
+    //   * Who is last (decoupled-group kernels): lane 0 draws a ticket, word g of the election line incremented by one; the last
+    //     ticket of step t is (t + 1) n_active - 1.  The counter is never reset: no warp can draw for step t + 1 before that refill
+    //     has landed, so the tickets of a step are the n_active values after those of the step before.  Every lane executes the
+    //     atomic, on its own word of the 32-word line (lane 0 on word g, the others adding 0 to the rest of the line, the other
+    //     groups' counters included): one conflict-free pass.  An add that only lane 0 executes is expanded by ptxas into a
+    //     warp-aggregated sequence (vote, popc, shuffle, a second branch) whose dependent chain stalls the warp.
+    //   * Ordering.  The hazard is the reads of the tile (ld.shared, generic proxy) by every warp against the TMA engine's
+    //     overwrite with step t + 1 (async proxy).  __syncwarp orders the warp's reads before lane 0's ticket; the ticket is an
+    //     acq_rel atomic on one location, so the last ticket acquires every earlier warp's release of its reads (the
+    //     read-modify-writes form one release sequence), and the copy is issued after it by the thread that drew it.  No proxy
+    //     fence: fence.proxy.async makes generic-proxy WRITES visible to the async proxy, and only the copies write the tiles.  The
+    //     release is one MEMBAR.ALL.CTA ahead of the ticket; the form it replaces fenced with __threadfence_block (MEMBAR.SC.CTA)
+    //     twice on the last reader's path and reset the counter in between.  Stamped at the bench shape (tools/probes/elect_stamps.py),
+    //     election and copy issue take 577 cycles per warp-step against 934; FP64 bench 2.19e10 -> 2.28e10 trajectory-steps/s on one
+    //     B200 at 1,000 W (profiles/r7_elect_ab.txt).  The warps of a scheduler are not in lockstep, so their windows do not stack.
+    //   * The full-covariance kernels (!kBlock) keep that form: lane 0 adds 1 between two block-scope fences, and the last reader
+    //     resets the counter before it issues the copy.  They run at the 255-register cap, where the ticket spills.
+    const auto last_reader = [&](int g, long long t) -> int {
         __syncwarp();  // every lane of this warp has read its values
-        int last = 0;
         if constexpr (TMA_WARPS == 1) {  // the block's only warp is always the last reader
             if (lane == 0) __threadfence_block();
             return lane == 0 ? 0 : 1;
         }
-        if (lane == 0) {
-            __threadfence_block();
-            last = atomicAdd(&consumed[g], 1) == n_active - 1;
-            if (last) {
-                consumed[g] = 0;
+        if constexpr (!kBlock) {
+            int last = 0;
+            if (lane == 0) {
                 __threadfence_block();
+                int *consumed = reinterpret_cast<int *>(tickets);
+                last = atomicAdd(&consumed[g], 1) == n_active - 1;
+                if (last) {
+                    consumed[g] = 0;
+                    __threadfence_block();
+                }
             }
+            return last ? 0 : 1;
         }
-        return last ? 0 : 1;  // 0 = "this lane issues the copy" in the issue_* helpers
+        uint32_t ticket;
+        asm volatile("atom.acq_rel.cta.shared::cta.add.u32 %0, [%1], %2;"
+                     : "=r"(ticket)
+                     : "r"(smem_u32(tickets + ((g + lane) & 31))), "r"(lane == 0 ? 1u : 0u)
+                     : "memory");
+        return lane == 0 && ticket == (uint32_t)(t + 1) * (uint32_t)n_active - 1u ? 0 : 1;  // 0 = "this lane issues the copy"
     };
 
     Real *q = noise + tid, *r = noise + 12 * nt + tid;
@@ -341,6 +399,7 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
         Real *g0 = g0w + stg, *g1 = g1w + stg, *g2 = g2w + stg;
 
         // ---- G0: leg moments -> mean model ------------------------------------------------------------------
+        OKF_STAMP(kStTop);
         mbar_wait(&bar[0], par);
         if constexpr (kOut == 2) {
             if (active && prm.p_world_steps) store_world_feet<32>(g0 + NM * 32 + lane, Rm, prm.p_world_steps, (t * 12) * N + i, N);
@@ -363,8 +422,10 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
             inv = rcp_(s);
         };
         const auto refill_g0 = [&] {  // this warp has consumed the step's moments: the last one refills G0 for step t + 1
-            const int elect = last_reader(0);
+            OKF_STAMP(kStElect0);
+            const int elect = last_reader(0, t);
             if (more) issue_g0<kOut, kMpc>(maps, t + kStages, s_warp, g0, &bar[0], elect);
+            OKF_STAMP(kStElect0End);
         };
         // kBlock: the first pivot's reciprocal and the G0 refill come after the predict, so that the mean model's dependent chain,
         // the predict's independent FMAs and the reciprocal form one basic block the scheduler can interleave (the copy still has
@@ -410,8 +471,10 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
         fold_pipelined<8, kBlock>(P, x, z[8 * 32], r[8 * nt], r[9 * nt], inv, inv_n, nis, status, nothing); inv = inv_n;
         const Real z9 = z[9 * 32], r9 = r[9 * nt];
         {  // this warp has read its last measurement of the step: the last one refills G1 for step t + 1
-            const int elect = last_reader(1);
+            OKF_STAMP(kStElect1);
+            const int elect = last_reader(1, t);
             if (more) issue_g1(maps, t + kStages, s_warp, g1, &bar[1], elect);
+            OKF_STAMP(kStElect1End);
         }
         fold_pipelined<9, kBlock>(P, x, z9, r9, r9, inv, inv_n, nis, status, [&] {
             // the posterior state is final here: start the next step's sin/cos underneath the last rank-1 update
@@ -458,10 +521,13 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
         if constexpr (kSummary) {
             acc_add(24, to_acc(nis));
             if (n_lab) {
-                const int elect = last_reader(2);  // this warp has consumed the step's labels: the last one refills G2 for step t + 1
+                OKF_STAMP(kStElect2);
+                const int elect = last_reader(2, t);  // this warp has consumed the step's labels: the last one refills G2 for step t + 1
                 if (more) issue_g2(maps, t + kStages, s_warp, n_lab, g2, &bar[2], elect);
+                OKF_STAMP(kStElect2End);
             }
         }
+        OKF_STAMP(kStEnd);
     }
 
     // A non-finite state is absorbing (NaN and Inf - Inf propagate through every later predict and update, nothing divides by
