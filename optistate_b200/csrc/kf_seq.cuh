@@ -2,6 +2,8 @@
 // [T][C][S] layout (stream index fastest).  It serves everything the TMA-fed kernel (kf_seq_tma.cuh) cannot take:
 // an arbitrary stream_index gather, stream counts that are not a multiple of 32, unaligned arrays, or no workspace for
 // the measurement pre-pass (the measurement is then formed inside the kernel, kalman_filter.py:79-117).
+// Its own are the per-thread input loads, the measurement and the running sums; set-up, stores and epilogue are kf_seq_core.cuh's.
+// Its trace (sequential) and K gain (gain_trace) round differently from the streamed kernel's (pairwise, precomputed 1 / r).
 #pragma once
 
 #include "kf_seq_core.cuh"
@@ -20,36 +22,17 @@ __global__ void __launch_bounds__(128) kf_seq_kernel(const __grid_constant__ Par
     const long long N = prm.N, S = prm.S;
     const long long s = stream_of(prm, i);
     Real *q = noise + threadIdx.x, *r = noise + 12 * nt + threadIdx.x;
-#pragma unroll
-    for (int c = 0; c < NX; ++c) q[c * nt] = prm.q_kind == OPTI_KF_MAT_DIAG ? prm.Q[c] : prm.Q[c * N + i];
-#pragma unroll
-    for (int c = 0; c < NZ; ++c) r[c * nt] = prm.r_kind == OPTI_KF_MAT_DIAG ? prm.R[c] : prm.R[c * N + i];
-
+    load_noise(prm, N, i, q, r, nt);
     Real x[NX], P[NP];
 #pragma unroll
     for (int c = 0; c < NX; ++c) x[c] = prm.x0[c * prm.x0_ld + i * prm.x0_inc];
-#pragma unroll
-    for (int a = 0; a < NX; ++a)
-#pragma unroll
-        for (int b = 0; b <= a; ++b) {
-            Real v = Real(0);
-            if (cpl<kBlock>(a, b)) switch (prm.p0_kind) {  // structural zeros are never loaded
-                case OPTI_KF_MAT_NONE: v = (a == b) ? q[a * nt] : Real(0); break;
-                case OPTI_KF_MAT_DIAG: v = (a == b) ? prm.P0[a] : Real(0); break;
-                case OPTI_KF_MAT_DIAG_PER: v = (a == b) ? prm.P0[a * N + i] : Real(0); break;
-                case OPTI_KF_MAT_DENSE: v = prm.P0[a * NX + b]; break;
-                default: v = prm.P0[(long long)(a * NX + b) * N + i]; break;
-            }
-            P[tri(a, b)] = v;
-        }
+    load_P0<kBlock>(prm, N, i, q, nt, P);
 
     uint32_t status[1] = {0};
     Real ptrace = Real(0), kgain = Real(0), ymax = Real(0);
-    double acc_truth[kSummary ? NX : 1], acc_nom[kSummary ? NX : 1], acc_nis = 0.0;
-    if (kSummary) {
+    typename Acc<Real>::type acc[kSummary ? ACC_ROWS : 1];
 #pragma unroll
-        for (int c = 0; c < NX; ++c) { acc_truth[c] = 0.0; acc_nom[c] = 0.0; }
-    }
+    for (int c = 0; c < (kSummary ? ACC_ROWS : 1); ++c) acc[c] = 0.0;
 
     Real Rm[9];
     rot_zyx(x[0], x[1], x[2], Rm);
@@ -133,62 +116,25 @@ __global__ void __launch_bounds__(128) kf_seq_kernel(const __grid_constant__ Par
         if (prm.k_gain_steps != nullptr || (last && prm.summary != nullptr)) {
             kgain = gain_trace<kBlock>(P, r, nt);
         }
-        if (prm.x_steps) {
-#pragma unroll
-            for (int c = 0; c < NX; ++c) st_stream(prm.x_steps + (t * NX + c) * N + i, x[c]);
-        }
-        if (prm.p_trace_steps) st_stream(prm.p_trace_steps + t * N + i, ptrace);
-        if (prm.k_gain_steps) st_stream(prm.k_gain_steps + t * N + i, kgain);
-        if (prm.nis_steps) st_stream(prm.nis_steps + t * N + i, nis);
-        if (kSummary) {
-            acc_nis += (double)nis;
+        store_step<kBlock, true>(prm, t, N, i, x, P, ptrace, kgain, nis);
+        if constexpr (kSummary) {
+            acc[24] += to_acc(nis);
             if (prm.truth) {
 #pragma unroll
-                for (int c = 0; c < NX; ++c) acc_truth[c] = err_acc(acc_truth[c], x[c], ld_stream(prm.truth + (t * NX + c) * S + s));
+                for (int c = 0; c < NX; ++c) acc[c] = err_acc(acc[c], x[c], ld_stream(prm.truth + (t * NX + c) * S + s));
             }
             if (prm.nominal) {
 #pragma unroll
-                for (int c = 0; c < NX; ++c) acc_nom[c] = err_acc(acc_nom[c], x[c], ld_stream(prm.nominal + (t * NX + c) * S + s));
+                for (int c = 0; c < NX; ++c) acc[12 + c] = err_acc(acc[12 + c], x[c], ld_stream(prm.nominal + (t * NX + c) * S + s));
             }
-        }
-        if (prm.P_ckpt && prm.ckpt_every > 0 && (t + 1) % prm.ckpt_every == 0) {
-            Real *dst = prm.P_ckpt + ((t + 1) / prm.ckpt_every - 1) * (long long)(NX * NX) * N + i;
-#pragma unroll
-            for (int a = 0; a < NX; ++a)
-#pragma unroll
-                for (int b = 0; b < NX; ++b) dst[(long long)(a * NX + b) * N] = cpl<kBlock>(a, b) ? P[tri(a, b)] : Real(0);
-        }
-        if (prm.P_steps) {
-            if constexpr (kBlock) store_packed_P(prm.P_steps, t, N, i, P);
-            else store_full_P(prm.P_steps, t, N, i, P);
         }
     }
 
 #pragma unroll
     for (int c = 0; c < NX; ++c) note_nonfinite(x[c], status, OPTI_KF_ST_NONFINITE);  // absorbing: see kf_seq_tma.cuh
-    if (prm.x_final) {
-#pragma unroll
-        for (int c = 0; c < NX; ++c) prm.x_final[c * N + i] = x[c];
-    }
-    if (prm.P_final) {
-#pragma unroll
-        for (int a = 0; a < NX; ++a)
-#pragma unroll
-            for (int b = 0; b < NX; ++b) prm.P_final[(long long)(a * NX + b) * N + i] = cpl<kBlock>(a, b) ? P[tri(a, b)] : Real(0);
-    }
-    if (kSummary && prm.summary) {
-        const double invT = prm.T > 0 ? 1.0 / (double)prm.T : 0.0;
-#pragma unroll
-        for (int c = 0; c < NX; ++c) {
-            st_summary(prm, c, i, x[c]);
-            st_summary(prm, 12 + c, i, P[tri(c, c)]);
-            st_summary(prm, 24 + c, i, (Real)sqrt(acc_truth[c] * invT));
-            st_summary(prm, 36 + c, i, (Real)sqrt(acc_nom[c] * invT));
-        }
-        st_summary(prm, 48, i, (Real)(acc_nis * invT));
-        st_summary(prm, 49, i, ptrace);
-        st_summary(prm, 50, i, kgain);
-        st_summary(prm, 51, i, (Real)sqrt((double)ymax));
+    store_final<kBlock>(prm, N, i, x, P);
+    if constexpr (kSummary) {
+        if (prm.summary) store_summary(prm, i, x, P, [&](int k) { return acc[k]; }, ptrace, kgain, ymax);
     }
     if (prm.status) prm.status[i] = status[0] | (prm.stream_status ? prm.stream_status[s] : 0u);  // pre-pass flags (ALL_SWING) of this stream
 }

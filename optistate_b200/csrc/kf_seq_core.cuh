@@ -1,5 +1,5 @@
 // Arithmetic core of the SEQUENTIAL path, shared by the TMA-fed kernel (kf_seq_tma.cuh) and the direct-load kernel
-// (kf_seq.cuh); generic over Real = double | float | F2 (kf_arith.cuh).
+// (kf_seq.cuh), with their set-up, per-step stores and epilogue; generic over Real = double | float | F2 (kf_arith.cuh).
 //
 //   * P is a packed symmetric matrix (78 scalars) that lives in registers for the whole time loop; x (12) too.
 //   * The covariance transition F_d P F_d^T + Q (kalman_filter.py:125-135) is evaluated block-wise on the packed form in
@@ -288,6 +288,107 @@ __device__ __forceinline__ Real gain_trace_rinv(const Real (&P)[NP], const Real 
     }
     return g0 + g1;
 }
+
+// trace of P, pairwise: a chain of four additions instead of twelve
+template <typename Real>
+__device__ __forceinline__ Real trace_of(const Real (&P)[NP]) {
+    Real h[6];
+#pragma unroll
+    for (int c = 0; c < 6; ++c) h[c] = P[tri(2 * c, 2 * c)] + P[tri(2 * c + 1, 2 * c + 1)];
+    return ((h[0] + h[1]) + (h[2] + h[3])) + (h[4] + h[5]);
+}
+
+// Set-up and outputs of the two kernels.  Loads take `idx` (the streamed kernel's clamped index), stores the thread's first
+// trajectory `i`.  N is the caller's prm.N: loaded again here, it changes the kernels' index arithmetic.
+
+// q[12] and r[10] to the caller's shared-memory columns q[c * nt], r[c * nt]
+template <typename Real, typename Scalar>
+__device__ __forceinline__ void load_noise(const Params<Scalar> &prm, long long N, long long idx, Real *q, Real *r, int nt) {
+#pragma unroll
+    for (int c = 0; c < NX; ++c) q[c * nt] = prm.q_kind == OPTI_KF_MAT_DIAG ? Real(prm.Q[c]) : ld_traj(prm.Q, c * N + idx, Real());
+#pragma unroll
+    for (int c = 0; c < NZ; ++c) r[c * nt] = prm.r_kind == OPTI_KF_MAT_DIAG ? Real(prm.R[c]) : ld_traj(prm.R, c * N + idx, Real());
+}
+
+// P0; NONE is diag(q).  x0 stays in the kernels: F2 needs a select on x0_inc, which costs the FP64 direct kernels spills.
+template <bool kBlock, typename Real, typename Scalar>
+__device__ __forceinline__ void load_P0(const Params<Scalar> &prm, long long N, long long idx, const Real *q, int nt, Real (&P)[NP]) {
+#pragma unroll
+    for (int a = 0; a < NX; ++a)
+#pragma unroll
+        for (int b = 0; b <= a; ++b) {
+            Real v = Real(0);
+            if (cpl<kBlock>(a, b)) switch (prm.p0_kind) {  // structural zeros are never loaded
+                case OPTI_KF_MAT_NONE: v = (a == b) ? q[a * nt] : Real(0); break;
+                case OPTI_KF_MAT_DIAG: v = (a == b) ? Real(prm.P0[a]) : Real(0); break;
+                case OPTI_KF_MAT_DIAG_PER: v = (a == b) ? ld_traj(prm.P0, a * N + idx, Real()) : Real(0); break;
+                case OPTI_KF_MAT_DENSE: v = Real(prm.P0[a * NX + b]); break;
+                default: v = ld_traj(prm.P0, (long long)(a * NX + b) * N + idx, Real()); break;
+            }
+            P[tri(a, b)] = v;
+        }
+}
+
+// Outputs of step t after the update; kRare adds P_ckpt (dense 144) and P_steps (packed or full, by kBlock)
+template <bool kBlock, bool kRare, typename Real, typename Scalar>
+__device__ __forceinline__ void store_step(const Params<Scalar> &prm, long long t, long long N, long long i, const Real (&x)[NX],
+                                           const Real (&P)[NP], Real ptrace, Real kgain, Real nis) {
+    if (prm.x_steps) {
+#pragma unroll
+        for (int c = 0; c < NX; ++c) st_traj(prm.x_steps, (t * NX + c) * N + i, x[c]);
+    }
+    if (prm.p_trace_steps) st_traj(prm.p_trace_steps, t * N + i, ptrace);
+    if (prm.k_gain_steps) st_traj(prm.k_gain_steps, t * N + i, kgain);
+    if (prm.nis_steps) st_traj(prm.nis_steps, t * N + i, nis);
+    if constexpr (kRare) {
+        if (prm.P_ckpt && prm.ckpt_every > 0 && (t + 1) % prm.ckpt_every == 0) {
+            const long long base = ((t + 1) / prm.ckpt_every - 1) * (long long)(NX * NX) * N + i;
+#pragma unroll
+            for (int a = 0; a < NX; ++a)
+#pragma unroll
+                for (int b = 0; b < NX; ++b) st_traj(prm.P_ckpt, base + (long long)(a * NX + b) * N, cpl<kBlock>(a, b) ? P[tri(a, b)] : Real(0));
+        }
+        if (prm.P_steps) {
+            if constexpr (kBlock) store_packed_P(prm.P_steps, t, N, i, P);
+            else store_full_P(prm.P_steps, t, N, i, P);
+        }
+    }
+}
+
+// x_final and P_final (dense 144, structural zeros written as zeros)
+template <bool kBlock, typename Real, typename Scalar>
+__device__ __forceinline__ void store_final(const Params<Scalar> &prm, long long N, long long i, const Real (&x)[NX], const Real (&P)[NP]) {
+    if (prm.x_final) {
+#pragma unroll
+        for (int c = 0; c < NX; ++c) st_traj(prm.x_final, c * N + i, x[c]);
+    }
+    if (prm.P_final) {
+#pragma unroll
+        for (int a = 0; a < NX; ++a)
+#pragma unroll
+            for (int b = 0; b < NX; ++b) st_traj(prm.P_final, (long long)(a * NX + b) * N + i, cpl<kBlock>(a, b) ? P[tri(a, b)] : Real(0));
+    }
+}
+
+// Summary rows 0-51 from x, P, the running sums acc(k), ptrace, kgain and ymax; an absent label stream gives zeros
+constexpr int ACC_ROWS = 25;  // running sums of the summary: 0-11 truth, 12-23 nominal, 24 NIS
+template <typename Real, typename Scalar, typename AccGet>
+__device__ __forceinline__ void store_summary(const Params<Scalar> &prm, long long i, const Real (&x)[NX], const Real (&P)[NP], AccGet acc,
+                                              Real ptrace, Real kgain, Real ymax) {
+    const double invT = prm.T > 0 ? 1.0 / (double)prm.T : 0.0;
+#pragma unroll
+    for (int c = 0; c < NX; ++c) {
+        st_summary(prm, c, i, x[c]);
+        st_summary(prm, 12 + c, i, P[tri(c, c)]);
+        st_summary(prm, 24 + c, i, prm.truth ? rms_out(acc(c), invT, Real()) : Real(0));
+        st_summary(prm, 36 + c, i, prm.nominal ? rms_out(acc(12 + c), invT, Real()) : Real(0));
+    }
+    st_summary(prm, 48, i, mean_out(acc(24), invT, Real()));
+    st_summary(prm, 49, i, ptrace);
+    st_summary(prm, 50, i, kgain);
+    st_summary(prm, 51, i, sqrt_(ymax));
+}
+
 
 // cheap test whether trunc(R^T) can have a non-zero entry in any lane (then the exact decision is taken per lane)
 template <typename Real>

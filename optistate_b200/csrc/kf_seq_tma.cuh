@@ -29,6 +29,7 @@
 //     the recursion on FFMA2 / FADD2 / FMUL2, halving the issue slots per trajectory-step; its tiles are [C] x 64.
 //   * z and the leg moments M of the mean model (leg_moments, kf_seq_core.cuh) come from the measurement pre-pass: they are
 //     state-independent and, with shared base streams, identical for every Monte-Carlo member of a stream.
+//   * Its own are the tiles, their refill elections and the schedule around them; the rest is kf_seq_core.cuh's.
 #pragma once
 
 #include <cuda.h>  // CUtensorMap (types only; the encoder is fetched through cudaGetDriverEntryPoint)
@@ -58,7 +59,6 @@ template <int kW>
 __host__ __device__ constexpr int tma_stages() { return kW == 1 ? 2 : 1; }
 template <int kOut>
 __host__ __device__ constexpr int tma_noise_rows() { return kOut != 0 ? TMA_NOISE_ROWS_OUT : TMA_NOISE_ROWS; }
-constexpr int TMA_ACC_ROWS = 25;    // running sums of the summary: 0-11 truth, 12-23 nominal, 24 NIS
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
@@ -106,7 +106,7 @@ struct TmaSmem {
     static __host__ __device__ constexpr size_t off_noise(int n_lab, int g0_rows) { return off_in() + kStages * warp_bytes(n_lab, g0_rows); }
     static __host__ __device__ constexpr size_t off_acc(int n_lab, int g0_rows) { return off_noise(n_lab, g0_rows) + (size_t)kNoiseRows * kThreads * sizeof(Real); }
     static __host__ __device__ constexpr size_t total(int n_lab, int g0_rows, bool acc_in_smem) {
-        return off_acc(n_lab, g0_rows) + (acc_in_smem ? (size_t)TMA_ACC_ROWS * kThreads * 8 : 0);
+        return off_acc(n_lab, g0_rows) + (acc_in_smem ? (size_t)ACC_ROWS * kThreads * 8 : 0);
     }
 };
 
@@ -305,10 +305,7 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
     };
 
     Real *q = noise + tid, *r = noise + 12 * nt + tid;
-#pragma unroll
-    for (int c = 0; c < NX; ++c) q[c * nt] = prm.q_kind == OPTI_KF_MAT_DIAG ? Real(prm.Q[c]) : ld_traj(prm.Q, c * N + ic, Real());
-#pragma unroll
-    for (int c = 0; c < NZ; ++c) r[c * nt] = prm.r_kind == OPTI_KF_MAT_DIAG ? Real(prm.R[c]) : ld_traj(prm.R, c * N + ic, Real());
+    load_noise(prm, N, ic, q, r, nt);
     if constexpr (kOut != 0) {  // K_gain = sum_j P[j][sel j] / r[j] is wanted every step: the ten reciprocals are taken once
 #pragma unroll
         for (int c = 0; c < NZ; ++c) r[(NZ + c) * nt] = rcp_(r[c * nt]);
@@ -316,26 +313,13 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
     Real x[NX], P[NP];
 #pragma unroll
     for (int c = 0; c < NX; ++c) x[c] = prm.x0_inc ? ld_traj(prm.x0, c * prm.x0_ld + ic, Real()) : Real(prm.x0[c]);
-#pragma unroll
-    for (int a = 0; a < NX; ++a)
-#pragma unroll
-        for (int b = 0; b <= a; ++b) {
-            Real v = Real(0);
-            if (cpl<kBlock>(a, b)) switch (prm.p0_kind) {  // structural zeros are never loaded
-                case OPTI_KF_MAT_NONE: v = (a == b) ? q[a * nt] : Real(0); break;
-                case OPTI_KF_MAT_DIAG: v = (a == b) ? Real(prm.P0[a]) : Real(0); break;
-                case OPTI_KF_MAT_DIAG_PER: v = (a == b) ? ld_traj(prm.P0, a * N + ic, Real()) : Real(0); break;
-                case OPTI_KF_MAT_DENSE: v = Real(prm.P0[a * NX + b]); break;
-                default: v = ld_traj(prm.P0, (long long)(a * NX + b) * N + ic, Real()); break;
-            }
-            P[tri(a, b)] = v;
-        }
+    load_P0<kBlock>(prm, N, ic, q, nt, P);
 
     uint32_t status[L];
 #pragma unroll
     for (int ln = 0; ln < L; ++ln) status[ln] = 0;
     Real ptrace = Real(0), kgain = Real(0), ymax = Real(0);
-    constexpr int kAccRegs = (kSummary && !kAccSmem) ? TMA_ACC_ROWS : 1;
+    constexpr int kAccRegs = (kSummary && !kAccSmem) ? ACC_ROWS : 1;
     AccT acc_r[kAccRegs];
 #pragma unroll
     for (int c = 0; c < kAccRegs; ++c) acc_r[c] = acc_zero(AccT());
@@ -350,7 +334,7 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
     };
     if constexpr (kSummary) {
 #pragma unroll
-        for (int c = 0; c < TMA_ACC_ROWS; ++c) {
+        for (int c = 0; c < ACC_ROWS; ++c) {
             if constexpr (kAccSmem) acc_s[c * nt] = acc_zero(AccT()); else acc_r[c] = acc_zero(AccT());
         }
     }
@@ -377,12 +361,6 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
                 for (int c = 0; c < 6; ++c) acc_r[acc0 + c0 + c] = err_acc(acc_r[acc0 + c0 + c], x[c0 + c], lv[c]);
             }
         }
-    };
-    auto trace_of = [](const Real (&Pm)[NP]) {  // pairwise: a chain of four additions instead of twelve
-        Real h[6];
-#pragma unroll
-        for (int c = 0; c < 6; ++c) h[c] = Pm[tri(2 * c, 2 * c)] + Pm[tri(2 * c + 1, 2 * c + 1)];
-        return ((h[0] + h[1]) + (h[2] + h[3])) + (h[4] + h[5]);
     };
 
     const Real e1_mpc = kMpc ? exp_minus_one(Real(prm.dt)) : Real(0);
@@ -494,28 +472,7 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
         if constexpr (kOut != 0) {
             ptrace = trace_of(P);
             if (prm.k_gain_steps != nullptr) kgain = gain_trace_rinv<kBlock>(P, r + NZ * nt, nt);
-            if (active) {
-                if (prm.x_steps) {
-#pragma unroll
-                    for (int c = 0; c < NX; ++c) st_traj(prm.x_steps, (t * NX + c) * N + i, x[c]);
-                }
-                if (prm.p_trace_steps) st_traj(prm.p_trace_steps, t * N + i, ptrace);
-                if (prm.k_gain_steps) st_traj(prm.k_gain_steps, t * N + i, kgain);
-                if (prm.nis_steps) st_traj(prm.nis_steps, t * N + i, nis);
-                if constexpr (kOut == 2) {
-                    if (prm.P_ckpt && prm.ckpt_every > 0 && (t + 1) % prm.ckpt_every == 0) {
-                        const long long base = ((t + 1) / prm.ckpt_every - 1) * (long long)(NX * NX) * N + i;
-#pragma unroll
-                        for (int a = 0; a < NX; ++a)
-#pragma unroll
-                            for (int b = 0; b < NX; ++b) st_traj(prm.P_ckpt, base + (long long)(a * NX + b) * N, cpl<kBlock>(a, b) ? P[tri(a, b)] : Real(0));
-                    }
-                    if (prm.P_steps) {
-                        if constexpr (kBlock) store_packed_P(prm.P_steps, t, N, i, P);
-                        else store_full_P(prm.P_steps, t, N, i, P);
-                    }
-                }
-            }
+            if (active) store_step<kBlock, kOut == 2>(prm, t, N, i, x, P, ptrace, kgain, nis);
         }
 
         if constexpr (kSummary) {
@@ -535,35 +492,15 @@ __global__ void __launch_bounds__(kW ? 32 * kW : tma_threads<kBlock>(), kW == 1 
 #pragma unroll
     for (int c = 0; c < NX; ++c) note_nonfinite(x[c], status, OPTI_KF_ST_NONFINITE);
     if (!active) return;
-    if (prm.x_final) {
-#pragma unroll
-        for (int c = 0; c < NX; ++c) st_traj(prm.x_final, c * N + i, x[c]);
-    }
-    if (prm.P_final) {
-#pragma unroll
-        for (int a = 0; a < NX; ++a)
-#pragma unroll
-            for (int b = 0; b < NX; ++b) st_traj(prm.P_final, (long long)(a * NX + b) * N + i, cpl<kBlock>(a, b) ? P[tri(a, b)] : Real(0));
-    }
+    store_final<kBlock>(prm, N, i, x, P);
     if (kSummary && prm.summary) {
         if (prm.T > 0) {  // of the last step: the posterior P is still in registers
             ptrace = trace_of(P);
             kgain = gain_trace<kBlock>(P, r, nt);
         }
-        const double invT = prm.T > 0 ? 1.0 / (double)prm.T : 0.0;
-#pragma unroll
-        for (int c = 0; c < NX; ++c) {
-            st_summary(prm, c, i, x[c]);
-            st_summary(prm, 12 + c, i, P[tri(c, c)]);
-            st_summary(prm, 24 + c, i, prm.truth ? rms_out(acc_get(c), invT, Real()) : Real(0));
-            st_summary(prm, 36 + c, i, prm.nominal ? rms_out(acc_get(12 + c), invT, Real()) : Real(0));
-        }
-        st_summary(prm, 48, i, mean_out(acc_get(24), invT, Real()));
-        st_summary(prm, 49, i, ptrace);
-        st_summary(prm, 50, i, kgain);
-        st_summary(prm, 51, i, sqrt_(ymax));
+        store_summary(prm, i, x, P, acc_get, ptrace, kgain, ymax);
     }
-    if (prm.status) {
+    if (prm.status) {  // with the pre-pass flags (ALL_SWING) of each trajectory's stream
 #pragma unroll
         for (int ln = 0; ln < L; ++ln)
             prm.status[i + ln] = status[ln] | (prm.stream_status ? prm.stream_status[s_warp + lane * L + ln] : 0u);

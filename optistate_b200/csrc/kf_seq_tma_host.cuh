@@ -66,13 +66,18 @@ int launch_seq_tma_k(const Params<typename Lanes<Real>::scalar> &p, cudaStream_t
     return OPTI_KF_OK;
 }
 
+// kOut of the instantiation that writes the per-step outputs p asks for (see kf_seq_tma.cuh)
+template <typename Scalar>
+int tma_out_class(const Params<Scalar> &p) {
+    if (p.x_model_steps || p.p_world_steps || p.z_steps || p.P_ckpt || p.P_steps) return 2;
+    return (p.x_steps || p.p_trace_steps || p.k_gain_steps || p.nis_steps) ? 1 : 0;
+}
+
 // per-step outputs, the predict_mpc covariance model and the decoupled-group form are compile-time variants of the kernel
 // (see kf_seq_tma.cuh); kBlock is chosen by the caller from Params.block and never combines with the predict_mpc model
 template <typename Real, bool kSummary, bool kBlock>
 int launch_seq_tma(const Params<typename Lanes<Real>::scalar> &p, cudaStream_t stream) {
-    const bool rare = p.x_model_steps || p.p_world_steps || p.z_steps || p.P_ckpt || p.P_steps;
-    const bool estimates = p.x_steps || p.p_trace_steps || p.k_gain_steps || p.nis_steps;
-    const int out = rare ? 2 : (estimates ? 1 : 0);
+    const int out = tma_out_class(p);
     const bool mpc = p.cov_model == OPTI_KF_COV_MPC;
     if constexpr (kBlock) {
         if (mpc) return OPTI_KF_E_UNSUPPORTED;
@@ -97,11 +102,11 @@ int launch_seq_tma(const Params<typename Lanes<Real>::scalar> &p, cudaStream_t s
 // kf_seq_tma_lone_*.cu for double and float.
 template <typename Real, bool kSummary>
 int launch_seq_tma_lone(const Params<typename Lanes<Real>::scalar> &p, cudaStream_t stream) {
-    const bool rare = p.x_model_steps || p.p_world_steps || p.z_steps || p.P_ckpt || p.P_steps;
-    const bool estimates = p.x_steps || p.p_trace_steps || p.k_gain_steps || p.nis_steps;
-    if (rare) return launch_seq_tma_k<Real, kSummary, 2, false, true, 1>(p, stream);
-    if (estimates) return launch_seq_tma_k<Real, kSummary, 1, false, true, 1>(p, stream);
-    return launch_seq_tma_k<Real, kSummary, 0, false, true, 1>(p, stream);
+    switch (tma_out_class(p)) {
+        case 0: return launch_seq_tma_k<Real, kSummary, 0, false, true, 1>(p, stream);
+        case 1: return launch_seq_tma_k<Real, kSummary, 1, false, true, 1>(p, stream);
+        default: return launch_seq_tma_k<Real, kSummary, 2, false, true, 1>(p, stream);
+    }
 }
 
 }  // namespace okf
