@@ -20,6 +20,8 @@
  *   optistate_kf_smooth_full the same on the full covariance (predict_mpc model, coupled P0).
  *   optistate_kf_noise_em_stats / optistate_kf_noise_em_full_stats
  *                           the E-step of expectation-maximisation for diagonal Q and R on either smoother.
+ *   optistate_kf_adjoint    the gradient of the filter's x_steps with respect to diagonal Q, R, x0 and P0 (an adjoint kernel
+ *                           backwards over the forward pass).
  *
  * Conventions
  *   - plain C, no torch / C++ types; every pointer is a NON-OWNING DEVICE pointer unless stated otherwise;
@@ -384,6 +386,36 @@ int optistate_kf_noise_em_stats(const OptiKfNoiseEmDesc *desc, void *cuda_stream
  * measurements.  Accepts exactly what optistate_kf_smooth_full accepts, with the same return codes. ---- */
 int optistate_kf_noise_em_full_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out);
 int optistate_kf_noise_em_full_stats(const OptiKfNoiseEmDesc *desc, void *cuda_stream);
+
+/* ---- gradient of the filter's x_steps: the vector-Jacobian product of x+_t (t = 0 .. T-1) with respect to the diagonal Q, the
+ * diagonal R, x0 and P0.  Runs the forward pass exactly as optistate_kf_smooth does, then an adjoint kernel, one thread per
+ * trajectory, backwards over the joint form of the update (which the sequential update equals in exact arithmetic):
+ *     a = 0, Pi = 0;  for t = T-1 .. 0:  a += x_bar_t;  b = K_t^T a;  r_bar_k += (K_t^T Pi K_t)_kk - b_k v_k;
+ *     Pb = A_t^T Pi A_t + sym(A_t^T a v_t^T H);  q_bar_i += Pb_ii;  Pi = F_t^T Pb F_t;  a = J_t^T (A_t^T a) + (theta-term of F_t)
+ * with A_t = I - K_t H, v_t = S_t^-1 (z_t - H x-_t) and J_t = dx-_t/dx+_{t-1} the derivative of the mean model (DESIGN.md section
+ * 0.4); at the end x0_bar = a, P0_bar = Pi.  Per trajectory, grad[row][i] holds
+ *     rows 0-11   q_bar = sum_t dL/dQ_ii through P-_t (never through P0 = Q: add rows 34-45 for that when P0 is absent)
+ *     rows 12-21  r_bar = dL/dR_kk
+ *     rows 22-33  x0_bar = dL/dx0
+ *     rows 34-45  the diagonal of dL/dP+_{-1} (dL/dP0 when P0 is given)
+ * for L any loss with dL/dx+_t = x_bar_t.  At an attitude where the mean model's trunc(R^T) changes (exactly axis-aligned, e.g.
+ * the all-zero start) the filter is discontinuous in the attitude; the gradient there is the almost-everywhere one.  Accepts
+ * exactly what optistate_kf_smooth accepts, with the same return codes; with a dense decoupled P0 rows 0-33 are exact and rows
+ * 34-45 the diagonal of dL/dP0.  status[i] gains OPTI_KF_ST_SMOOTH_NOT_PD when a pivot of S_t is not positive and finite. ---- */
+#define OPTI_KF_ADJ_ROWS 46  /* 0-11 q_bar, 12-21 r_bar, 22-33 x0_bar, 34-45 diag P0_bar */
+typedef struct OptiKfAdjointDesc {
+    uint32_t struct_size;       /* sizeof(OptiKfAdjointDesc) */
+    uint32_t abi_version;       /* OPTISTATE_KF_ABI_VERSION */
+    const OptiKfDesc *filter;   /* forward pass, run exactly as optistate_kf_batch runs it */
+    const void *x_bar;          /* [T][12][N] required: dL/dx+_t */
+    void *grad;                 /* [46][N] required */
+    void *storage;              /* device scratch of optistate_kf_adjoint_storage_bytes(filter): the smoother's storage, plus the
+                                   measurements z [T][10][S] when the filter forms them (OPTI_KF_PHASE_MEASURE) and the leg moments
+                                   of the mean model [T][12][S] */
+    size_t storage_bytes;
+} OptiKfAdjointDesc;
+int optistate_kf_adjoint_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out);
+int optistate_kf_adjoint(const OptiKfAdjointDesc *desc, void *cuda_stream);
 
 /* Runs the filter; dtype taken from the descriptor. */
 int optistate_kf_batch(const OptiKfDesc *desc, void *cuda_stream);

@@ -14,11 +14,13 @@ can share a few input streams.
 from __future__ import annotations
 
 import inspect
+import warnings
 from dataclasses import dataclass, field
 from typing import Dict, Iterable, Optional
 
 import numpy as np
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import _native as nv
 from .settings import INITIAL_PARAMS
@@ -316,7 +318,7 @@ _FILTER_SIGNATURE = inspect.signature(kf_batch)
 
 @dataclass(frozen=True)
 class _Backward:
-    """One of the four backward passes over the sequential filter (include/optistate_kf.h)."""
+    """One of the five backward passes over the sequential filter (include/optistate_kf.h)."""
     who: str        # public name, in ValueErrors
     entry: str      # binding; with cfg query_storage = 1 it returns the storage size instead of running
     storage: str    # key of the library's scratch in `out`
@@ -324,6 +326,7 @@ class _Backward:
     c_storage: str
     full: bool      # the full-covariance kernel: either covariance model, any symmetric P0 (_filter_call refuses others)
     stats: bool     # the E-step: noise_stats out, x_smooth optional
+    adj: bool = False  # the adjoint: x_bar in, grad out, no smoothed outputs
 
 
 _KF_SMOOTH = _Backward("kf_smooth", "kf_smooth", "smooth_storage", "optistate_kf_smooth",
@@ -334,11 +337,15 @@ _KF_NOISE_STATS = _Backward("kf_noise_stats", "kf_noise_em_stats", "em_storage",
                             "optistate_kf_noise_em_storage_bytes", False, True)
 _KF_NOISE_STATS_FULL = _Backward("kf_noise_stats_full", "kf_noise_em_full_stats", "em_storage", "optistate_kf_noise_em_full_stats",
                                  "optistate_kf_noise_em_full_storage_bytes", True, True)
+_KF_VJP = _Backward("kf_vjp", "kf_adjoint", "adj_storage", "optistate_kf_adjoint", "optistate_kf_adjoint_storage_bytes", False, False,
+                    adj=True)
+ADJ_ROWS = 46
+ADJ_FIELDS = {"Q": slice(0, 12), "R": slice(12, 22), "x0": slice(22, 34), "P0": slice(34, 46)}
 
 
-def _run_backward(v: _Backward, args, outputs, kw) -> KfBatchResult:
-    """The forward pass (_filter_call, with kf_batch's keywords and defaults) with what the backward kernel refuses refused here,
-    the smoothed outputs, noise_stats and the library's storage attached, then the backward entry."""
+def _backward_call(v: _Backward, args, outputs, kw):
+    """The forward pass's _FilterCall (kf_batch's keywords and defaults) with what the backward kernel refuses refused here, and
+    the remaining outputs; returns (call, kw bound to kf_batch's signature, the backward outputs asked for)."""
     try:
         bound = _FILTER_SIGNATURE.bind(*args, **kw)
     except TypeError as e:  # a keyword kf_batch does not take
@@ -354,7 +361,9 @@ def _run_backward(v: _Backward, args, outputs, kw) -> KfBatchResult:
         raise ValueError(f"{who} runs on the sequential filter; algo='joint' is not supported")
     outputs = list(outputs)
     smooth_want = [o for o in outputs if o in _SMOOTH_OUTPUTS]
-    if not v.stats and "x_smooth" not in smooth_want:
+    if v.adj and smooth_want:
+        raise ValueError(f"{who} has no smoothed outputs")
+    if not v.stats and not v.adj and "x_smooth" not in smooth_want:
         smooth_want.insert(0, "x_smooth")
     kw.update(outputs=[o for o in outputs if o not in _SMOOTH_OUTPUTS], algo="sequential" if kw["algo"] == "auto" else kw["algo"])
     call = _filter_call(**kw)
@@ -364,6 +373,14 @@ def _run_backward(v: _Backward, args, outputs, kw) -> KfBatchResult:
                                                                "(dense noise couples the decoupled groups)"))
     if not full and cfg["p0_kind"] in (nv.MAT_DENSE, nv.MAT_DENSE_PER) and not cfg["flags"] & nv.FLAG_P0_DECOUPLED:
         raise ValueError(f"{who} needs a P0 without entries across the groups {{th, w}}, {{x, vx}}, {{y, vy}}, {{z, vz}}")
+    return call, kw, smooth_want
+
+
+def _run_backward(v: _Backward, args, outputs, kw, x_bar=None) -> KfBatchResult:
+    """The forward pass of _backward_call, the smoothed outputs, noise_stats or the adjoint's x_bar and grad, and the library's
+    storage attached, then the backward entry."""
+    call, kw, smooth_want = _backward_call(v, args, outputs, kw)
+    cfg = call.cfg
     T, N, out, dtype = call.n_steps, call.n_traj, kw["out"], kw["dtype"]
     for o in smooth_want:
         call.tensors[o] = _out_tensor(out, o, (T, 12, N), dtype, call.device)
@@ -371,6 +388,13 @@ def _run_backward(v: _Backward, args, outputs, kw) -> KfBatchResult:
     if v.stats:
         call.tensors["noise_stats"] = _out_tensor(out, "noise_stats", (EM_STATS_ROWS, N), dtype, call.device)
         extra = ["noise_stats", *smooth_want]
+    if v.adj:
+        xb = _as_device(x_bar, dtype, call.device)
+        if tuple(xb.shape) != (T, 12, N):
+            raise ValueError(f"{v.who}: grad_x_steps must have the shape of x_steps, {(T, 12, N)}, got {tuple(xb.shape)}")
+        call.tensors["x_bar"] = xb
+        call.tensors["grad"] = _out_tensor(out, "grad", (ADJ_ROWS, N), dtype, call.device)
+        extra = ["grad"]
     entry = getattr(call.ext, v.entry)
     with torch.cuda.device(call.device):
         _attach_workspace(call, out)
@@ -443,6 +467,116 @@ def kf_noise_stats_full(imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None
     non-symmetric P0 raise ValueError.
     """
     return _run_backward(_KF_NOISE_STATS_FULL, (imu, p, dp, contact, f, x0, P0, Q, R), outputs, kw)
+
+
+def kf_vjp(imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, *, grad_x_steps, outputs: Iterable[str] = (),
+           **kw) -> KfBatchResult:
+    """Gradient of the filter's x_steps (DESIGN.md section 0.4): runs the filter exactly as kf_batch runs it with the same
+    arguments, then an adjoint kernel backwards over it, and returns `grad` [46, N] per trajectory, for any loss L with
+    dL/dx_steps = grad_x_steps [T, 12, N]:
+        rows 0-11   dL/dQ_ii through the predicted covariances (not through P0 = Q: add rows 34-45 when P0 is None)
+        rows 12-21  dL/dR_kk
+        rows 22-33  dL/dx0
+        rows 34-45  the diagonal of dL/dP0 (of the initial covariance, Q when P0 is None)
+    The keywords other than grad_x_steps and outputs are kf_batch's, with its defaults; outputs: any kf_batch output, from the same
+    forward pass.  out: as for kf_batch, plus "grad" and "adj_storage" (uint8 scratch of optistate_kf_adjoint_storage_bytes: the
+    smoother's storage, the measurements and the leg moments of the mean model).  At an exactly axis-aligned attitude (e.g. the
+    all-zero start) the mean model's trunc(R^T) jumps and the gradient is the almost-everywhere one.  Refuses what kf_smooth
+    refuses, with the same ValueErrors; a dense P0 without cross-group entries is taken, rows 34-45 then hold its diagonal only.
+    """
+    return _run_backward(_KF_VJP, (imu, p, dp, contact, f, x0, P0, Q, R), outputs, kw, x_bar=grad_x_steps)
+
+
+def _grad_like(g: torch.Tensor, inp: torch.Tensor, per_traj: bool, n: int) -> torch.Tensor:
+    """A per-trajectory gradient g [n, N] in the shape of the input it belongs to, by the kind the forward pass resolved for it:
+    per trajectory ([n, N]) as it is, shared ([n], or a diagonal [n, n]) summed over the trajectories."""
+    if per_traj:
+        out = g
+    else:
+        out = g.sum(dim=1)
+        if inp.numel() != n:
+            out = torch.diag(out)
+    return out.to(dtype=inp.dtype, device=inp.device).reshape(inp.shape)
+
+
+class _KfStates(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, kw, imu, p, dp, contact, f, x0, P0, Q, R):
+        args = (imu, p, dp, contact, f, x0, P0, Q, R)
+        call, _, _ = _backward_call(_KF_VJP, tuple(a.detach() if isinstance(a, torch.Tensor) else a for a in args), ("x_steps",), kw)
+        cfg = call.cfg
+        if ctx.needs_input_grad[7] and cfg["p0_kind"] in (nv.MAT_DENSE, nv.MAT_DENSE_PER):
+            raise ValueError("kf_states: a dense P0 cannot require grad (the adjoint returns the diagonal of dL/dP0 only)")
+        with torch.cuda.device(call.device):
+            _attach_workspace(call, kw.get("out"))
+            nv.check(int(call.ext.kf_batch(call.cfg, call.consts, call.tensors)), "optistate_kf_batch")
+        # the backward pass re-runs the filter from these inputs: saved through autograd, an input changed in place in between
+        # raises instead of giving the gradient at other values
+        kw_t = sorted(k for k, v in kw.items() if isinstance(v, torch.Tensor))
+        arg_t = [k for k, a in enumerate(args) if isinstance(a, torch.Tensor)]
+        ctx.save_for_backward(*(args[k] for k in arg_t), *(kw[k] for k in kw_t))
+        ctx.layout = arg_t, kw_t
+        ctx.args = tuple(None if isinstance(a, torch.Tensor) else a for a in args)
+        ctx.kw = {k: v for k, v in kw.items() if k not in kw_t}
+        # the kinds the forward pass resolved decide the gradients' shapes (a shape alone is ambiguous when N equals n)
+        ctx.per_traj = dict(Q=cfg["q_kind"] == nv.MAT_DIAG_PER, R=cfg["r_kind"] == nv.MAT_DIAG_PER, P0=cfg["p0_kind"] == nv.MAT_DIAG_PER,
+                            x0=bool(cfg["x0_per_traj"]))
+        return call.tensors["x_steps"]
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        arg_t, kw_t = ctx.layout
+        saved = ctx.saved_tensors
+        args = list(ctx.args)
+        for j, k in enumerate(arg_t):
+            args[k] = saved[j]
+        kw = dict(ctx.kw, **{k: saved[len(arg_t) + j] for j, k in enumerate(kw_t)})
+        x0, P0, Q, R = args[5:]
+        res = kf_vjp(*args, grad_x_steps=g.contiguous(), **kw)
+        bad = res.status[res.status != 0]
+        if bad.numel():
+            bits = int(np.bitwise_or.reduce(np.unique(bad.cpu().numpy())))
+            warnings.warn(f"kf_states: {bad.numel()} trajectories have a non-zero status (bits {bits:#x}, include/optistate_kf.h "
+                          "OPTI_KF_ST_*): their gradients come from a filter or adjoint pivot that was not positive and finite, or "
+                          "from a step without a stance leg", RuntimeWarning, stacklevel=2)
+        grad = res.grad
+        need = ctx.needs_input_grad
+        gq = grad[ADJ_FIELDS["Q"]]
+        if P0 is None:
+            gq = gq + grad[ADJ_FIELDS["P0"]]
+        out = [None] * 10
+        per = ctx.per_traj
+        if need[6]:
+            out[6] = _grad_like(grad[ADJ_FIELDS["x0"]], x0, per["x0"], 12)
+        if need[7]:
+            out[7] = _grad_like(grad[ADJ_FIELDS["P0"]], P0, per["P0"], 12)
+        if need[8]:
+            out[8] = _grad_like(gq, Q, per["Q"], 12)
+        if need[9]:
+            out[9] = _grad_like(grad[ADJ_FIELDS["R"]], R, per["R"], 10)
+        return tuple(out)
+
+
+def kf_states(imu, p, dp, contact, f, x0=None, P0=None, Q=None, R=None, **kw) -> torch.Tensor:
+    """kf_batch's x_steps [T, 12, N] as a differentiable function of Q, R, x0 and P0: gradients of any loss on it reach the
+    filter's parameters through torch autograd, whose backward runs kf_vjp (the forward pass again, then the adjoint kernel; no
+    storage is held between the two).  The keywords are kf_batch's other than outputs.  Gradients come back in each input's own
+    shape: Q, R and P0 diagonal ([n] or a diagonal [n, n] shared - summed over the trajectories - or [n, N]), x0 [12] or [12, N].
+    With P0 None the initial covariance is Q, and its gradient is added to Q's.  Refuses what kf_smooth refuses, and a dense P0
+    that requires grad (the adjoint returns the diagonal of dL/dP0 only), with ValueErrors.  Sensor streams get no gradient.
+    The backward pass re-runs the filter from the saved inputs: one changed in place in between makes autograd raise.  It reads
+    the status words of that filter run and of the adjoint (one host synchronisation) and warns (RuntimeWarning) when a
+    trajectory's is non-zero - a pivot that was not positive and finite, or a step without a stance leg - since its gradient is
+    then not to be trusted; kf_vjp returns the status words themselves.  The result is differentiable once.
+
+        q = torch.log(torch.tensor(Q0, device="cuda")).requires_grad_()
+        loss = ((kf_states(imu, p, dp, contact, f, Q=q.exp(), n_traj=N) - truth_steps) ** 2).mean()
+        loss.backward()  # q.grad
+    """
+    if "outputs" in kw:
+        raise TypeError("kf_states() returns x_steps; it takes no outputs")
+    return _KfStates.apply(dict(kw), imu, p, dp, contact, f, x0, P0, Q, R)
 
 
 @dataclass

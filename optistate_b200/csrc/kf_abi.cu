@@ -6,6 +6,7 @@
 #include <cstring>
 #include <type_traits>
 
+#include "kf_adjoint.cuh"
 #include "kf_features.cuh"
 #include "kf_identify.cuh"
 #include "kf_launch.cuh"
@@ -319,11 +320,12 @@ int fma_peak(long long fma_per_thread, double *flops_out, double *seconds_out, c
     return OPTI_KF_OK;
 }
 
-// ---- the backward passes over the SEQUENTIAL filter: smoother and EM E-step ------------------------------------------
+// ---- the backward passes over the SEQUENTIAL filter: smoother, EM E-step and adjoint ---------------------------------
 // full: the full-covariance kernel (all 78 entries of P+, SmoothFullParams, kf_rts_full_kernel) instead of the decoupled one
-// (30 packed entries, SmoothParams, kf_rts_kernel); stats: the E-step of EM, which accepts exactly what its smoother accepts.
+// (30 packed entries, SmoothParams, kf_rts_kernel); stats: the E-step of EM, which accepts exactly what its smoother accepts;
+// adj: the adjoint of the decoupled filter (AdjointParams, kf_adjoint_kernel), which accepts exactly what the smoother accepts.
 struct Backward {
-    bool full, stats;
+    bool full, stats, adj;
 };
 
 // What the backward kernels can take.  Decoupled: the decoupled-group form of the SEQUENTIAL filter (kf_smooth.cuh).  Full:
@@ -344,9 +346,10 @@ int backward_check(const OptiKfDesc *d, bool full) {
 
 // Scratch of the backward passes, each part padded to 256 bytes: P+ [T][np][N] at 0 (np = 30 packed decoupled entries, or all
 // 78 when full), then x+ and x- [T][12][N] unless the filter descriptor has x_steps / x_model_steps (the backward kernel reads
-// those), then for the E-step z [T][10][S] when the filter forms the measurements.  Byte offsets.
+// those), then for the E-step and the adjoint z [T][10][S] when the filter forms the measurements, then for the adjoint the leg
+// moments of the mean model [T][12][S].  Byte offsets.
 struct BackwardStorage {
-    size_t x_post, x_prior, z, total;
+    size_t x_post, x_prior, z, mom, total;
     BackwardStorage(const OptiKfDesc *d, Backward v) {
         const auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
         const size_t esz = d->dtype == OPTI_KF_F64 ? 8 : 4, tn = (size_t)d->n_steps * (size_t)d->n_traj;
@@ -354,15 +357,18 @@ struct BackwardStorage {
         x_post = up(tn * (size_t)(v.full ? okf::NP : okf::NPB) * esz);
         x_prior = x_post + (d->x_steps ? 0 : up(tn * okf::NX * esz));
         z = x_prior + (d->x_model_steps ? 0 : up(tn * okf::NX * esz));
-        total = z + (v.stats && (d->phases & OPTI_KF_PHASE_MEASURE) ? up(ts * okf::NZ * esz) : 0);
+        mom = z + ((v.stats || v.adj) && (d->phases & OPTI_KF_PHASE_MEASURE) ? up(ts * okf::NZ * esz) : 0);
+        total = mom + (v.adj ? up(ts * okf::NM * esz) : 0);
     }
 };
 
 // The forward pass, with x+ / x- in the storage where the caller did not ask for them, then the backward kernel.  A full pass runs
 // the full-covariance filter kernels whatever the caller's flags, so P+ is [T][78][N] (on decoupled inputs they are bit-identical
 // to the kBlock ones, kf_seq_core.cuh).
+// stats: the E-step's [23][N] or the adjoint's grad [46][N]; x_bar: the adjoint's dL/dx+.
 template <typename Real>
-int run_backward(Backward v, const OptiKfDesc *f, void *storage, void *x_smooth, void *var_smooth, void *stats, cudaStream_t stream) {
+int run_backward(Backward v, const OptiKfDesc *f, void *storage, void *x_smooth, void *var_smooth, void *stats, const void *x_bar,
+                 cudaStream_t stream) {
     const BackwardStorage st(f, v);
     unsigned char *base = (unsigned char *)storage;
     OptiKfDesc fw = *f;
@@ -372,14 +378,17 @@ int run_backward(Backward v, const OptiKfDesc *f, void *storage, void *x_smooth,
     int rc = launch<Real>(&fw, OPTI_KF_ALGO_SEQUENTIAL, stream, base);
     if (rc != OPTI_KF_OK) return rc;
     const long long N = f->n_traj, T = f->n_steps;
-    if (N == 0 || (T == 0 && !v.stats)) return OPTI_KF_OK;
-    if (T == 0)  // no transition and no measurement: every sum is empty
-        return cudaMemsetAsync(stats, 0, (size_t)okf::EM_STATS_ROWS * N * sizeof(Real), stream) == cudaSuccess ? OPTI_KF_OK : OPTI_KF_E_CUDA;
+    if (N == 0 || (T == 0 && !v.stats && !v.adj)) return OPTI_KF_OK;
+    if (T == 0)  // no transition and no measurement: every sum is empty, and x0, P0 do not reach x_steps
+        return cudaMemsetAsync(stats, 0, (size_t)(v.adj ? OPTI_KF_ADJ_ROWS : okf::EM_STATS_ROWS) * N * sizeof(Real), stream) == cudaSuccess
+                   ? OPTI_KF_OK : OPTI_KF_E_CUDA;
     const Real *z = (const Real *)f->z_in;
-    if (v.stats && (f->phases & OPTI_KF_PHASE_MEASURE)) {  // the filter formed z in-kernel: form it once more, per stream, with the same function
-        z = (const Real *)(base + st.z);
+    Real *mom = v.adj ? (Real *)(base + st.mom) : nullptr;
+    const bool form_z = (v.stats || v.adj) && (f->phases & OPTI_KF_PHASE_MEASURE);
+    if (form_z || mom) {  // the filter formed z and the moments in-kernel: form them once more, per stream, with the same functions
+        if (form_z) z = (const Real *)(base + st.z);
         launch_measure<Real>(T, f->n_streams, (const Real *)f->imu, (const Real *)f->p, (const Real *)f->dp, (const Real *)f->contact,
-                             nullptr, (Real *)z, nullptr, nullptr, nullptr, stream);
+                             (const Real *)f->f, form_z ? (Real *)z : nullptr, mom, nullptr, nullptr, stream);
     }
     const auto fill = [&](auto &p) {  // the fields SmoothParams and SmoothFullParams share; the E-step's stay zero for the smoother
         std::memset(&p, 0, sizeof p);
@@ -398,7 +407,21 @@ int run_backward(Backward v, const OptiKfDesc *f, void *storage, void *x_smooth,
             p.stats = (Real *)stats;
         }
     };
-    if (v.full) {
+    if (v.adj) {
+        okf::AdjointParams<Real> p;
+        std::memset(&p, 0, sizeof p);
+        p.N = N; p.T = T; p.dt = (Real)f->dt;
+        for (int k = 0; k < 3; ++k) p.dt_inv_inertia[k] = p.dt * (Real)(1.0 / f->inertia[k]);
+        p.Q = (const Real *)f->Q; p.q_kind = f->q_kind;
+        p.R = (const Real *)f->R; p.r_kind = f->r_kind;
+        p.x0 = (const Real *)f->x0; p.x0_ld = f->x0_per_traj ? N : 1; p.x0_inc = f->x0_per_traj ? 1 : 0;
+        p.P0 = (const Real *)f->P0; p.p0_kind = f->p0_kind;
+        p.x_post = (const Real *)fw.x_steps; p.x_prior = (const Real *)fw.x_model_steps; p.P_post = (const Real *)base;
+        p.x_bar = (const Real *)x_bar; p.z = z; p.mom = mom;
+        p.S = f->n_streams; p.stream_offset = f->stream_offset; p.stream_index = f->stream_index;
+        p.grad = (Real *)stats; p.status = f->status;
+        rc = okf::launch_adjoint<Real>(p, stream);
+    } else if (v.full) {
         okf::SmoothFullParams<Real> p;
         fill(p);
         p.cov_model = f->cov_model; p.body_ref = (const Real *)f->body_ref;
@@ -422,10 +445,10 @@ int backward_storage_bytes(const OptiKfDesc *filter, Backward v, size_t *bytes_o
 }
 
 // The entries' envelope, codes in the order the header documents: the descriptor, the filter, the required output (the smoother's
-// x_smooth, the E-step's stats), then the storage.
+// x_smooth, the E-step's stats, the adjoint's x_bar and grad), then the storage.
 template <typename Desc>
 int backward_entry(const Desc *desc, bool full, void *cuda_stream) {
-    constexpr bool stats = std::is_same<Desc, OptiKfNoiseEmDesc>::value;
+    constexpr bool stats = std::is_same<Desc, OptiKfNoiseEmDesc>::value, adj = std::is_same<Desc, OptiKfAdjointDesc>::value;
     if (!desc) return OPTI_KF_E_NULL;
     if (desc->struct_size != sizeof(Desc) || desc->abi_version != OPTISTATE_KF_ABI_VERSION) return OPTI_KF_E_VERSION;
     if (!desc->filter) return OPTI_KF_E_NULL;
@@ -433,19 +456,28 @@ int backward_entry(const Desc *desc, bool full, void *cuda_stream) {
     const int rc = backward_check(f, full);
     if (rc != OPTI_KF_OK) return rc;
     const bool steps = f->n_traj > 0 && f->n_steps > 0;  // empty batches carry empty (NULL) arrays
-    void *out_stats = nullptr;
-    if constexpr (stats) {
-        out_stats = desc->stats;
-        if (f->n_traj > 0 && !out_stats) return OPTI_KF_E_NULL;
+    void *out_stats = nullptr, *x_smooth = nullptr, *var_smooth = nullptr;
+    const void *x_bar = nullptr;
+    if constexpr (adj) {
+        out_stats = desc->grad;
+        x_bar = desc->x_bar;
+        if ((f->n_traj > 0 && !out_stats) || (steps && !x_bar)) return OPTI_KF_E_NULL;
     } else {
-        if (steps && !desc->x_smooth) return OPTI_KF_E_NULL;
+        x_smooth = desc->x_smooth;
+        var_smooth = desc->var_smooth;
+        if constexpr (stats) {
+            out_stats = desc->stats;
+            if (f->n_traj > 0 && !out_stats) return OPTI_KF_E_NULL;
+        } else {
+            if (steps && !x_smooth) return OPTI_KF_E_NULL;
+        }
     }
-    const Backward v{full, stats};
+    const Backward v{full, stats, adj};
     if (desc->storage_bytes < BackwardStorage(f, v).total) return OPTI_KF_E_SHAPE;
     if (steps && !desc->storage) return OPTI_KF_E_NULL;
     cudaStream_t stream = (cudaStream_t)cuda_stream;
-    return f->dtype == OPTI_KF_F64 ? run_backward<double>(v, f, desc->storage, desc->x_smooth, desc->var_smooth, out_stats, stream)
-                                   : run_backward<float>(v, f, desc->storage, desc->x_smooth, desc->var_smooth, out_stats, stream);
+    return f->dtype == OPTI_KF_F64 ? run_backward<double>(v, f, desc->storage, x_smooth, var_smooth, out_stats, x_bar, stream)
+                                   : run_backward<float>(v, f, desc->storage, x_smooth, var_smooth, out_stats, x_bar, stream);
 }
 
 template <typename Real>
@@ -511,6 +543,11 @@ int optistate_kf_noise_em_full_storage_bytes(const OptiKfDesc *filter, size_t *b
     return backward_storage_bytes(filter, {true, true}, bytes_out);
 }
 int optistate_kf_noise_em_full_stats(const OptiKfNoiseEmDesc *desc, void *cuda_stream) { return backward_entry(desc, true, cuda_stream); }
+
+int optistate_kf_adjoint_storage_bytes(const OptiKfDesc *filter, size_t *bytes_out) {
+    return backward_storage_bytes(filter, {false, false, true}, bytes_out);
+}
+int optistate_kf_adjoint(const OptiKfAdjointDesc *desc, void *cuda_stream) { return backward_entry(desc, false, cuda_stream); }
 
 int optistate_kf_batch(const OptiKfDesc *desc, void *cuda_stream) {
     const int rc = validate(desc);

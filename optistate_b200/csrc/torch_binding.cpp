@@ -170,13 +170,13 @@ int64_t kf_batch(const std::map<std::string, int64_t> &cfg, const std::map<std::
 }
 
 // The backward passes: the filter's tensors as for kf_batch, plus the smoother's x_smooth [T][12][N] (required) or the E-step's
-// noise_stats [23][N] (required; x_smooth optional), optional var_smooth [T][12][N], and the uint8 storage of the entry's
-// storage query, smooth_storage or em_storage (cfg query_storage = 1 returns that size instead of running).  Desc:
-// OptiKfSmoothDesc or OptiKfNoiseEmDesc.
+// noise_stats [23][N] (required; x_smooth optional), optional var_smooth [T][12][N], or the adjoint's x_bar [T][12][N] and grad
+// [46][N] (both required), and the uint8 storage of the entry's storage query, smooth_storage, em_storage or adj_storage (cfg
+// query_storage = 1 returns that size instead of running).  Desc: OptiKfSmoothDesc, OptiKfNoiseEmDesc or OptiKfAdjointDesc.
 template <typename Desc>
 int64_t run_backward(int (*storage_bytes)(const OptiKfDesc *, size_t *), int (*entry)(const Desc *, void *),
                      const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
-    constexpr bool stats = std::is_same<Desc, OptiKfNoiseEmDesc>::value;
+    constexpr bool stats = std::is_same<Desc, OptiKfNoiseEmDesc>::value, adj = std::is_same<Desc, OptiKfAdjointDesc>::value;
     OptiKfDesc d;
     const c10::Device dev = filter_desc(cfg, consts, tensors, d);
     const c10::cuda::CUDAGuard guard(dev);
@@ -192,10 +192,15 @@ int64_t run_backward(int (*storage_bytes)(const OptiKfDesc *, size_t *), int (*e
     s.struct_size = sizeof s;
     s.abi_version = OPTISTATE_KF_ABI_VERSION;
     s.filter = &d;
-    if constexpr (stats) s.stats = const_cast<void *>(ck.get(tensors, "noise_stats", OPTI_KF_EM_STATS_ROWS * N, true));
-    s.x_smooth = const_cast<void *>(ck.get(tensors, "x_smooth", T * 12 * N, !stats));
-    s.var_smooth = const_cast<void *>(ck.get(tensors, "var_smooth", T * 12 * N, false));
-    const std::string key = stats ? "em_storage" : "smooth_storage";
+    if constexpr (adj) {
+        s.x_bar = ck.get(tensors, "x_bar", T * 12 * N, true);
+        s.grad = const_cast<void *>(ck.get(tensors, "grad", OPTI_KF_ADJ_ROWS * N, true));
+    } else {
+        if constexpr (stats) s.stats = const_cast<void *>(ck.get(tensors, "noise_stats", OPTI_KF_EM_STATS_ROWS * N, true));
+        s.x_smooth = const_cast<void *>(ck.get(tensors, "x_smooth", T * 12 * N, !stats));
+        s.var_smooth = const_cast<void *>(ck.get(tensors, "var_smooth", T * 12 * N, false));
+    }
+    const std::string key = adj ? "adj_storage" : stats ? "em_storage" : "smooth_storage";
     auto is = tensors.find(key);
     TORCH_CHECK(is != tensors.end(), "optistate_b200: missing tensor '", key, "'");
     const at::Tensor &t = is->second;
@@ -218,6 +223,10 @@ int64_t kf_noise_em_stats(const std::map<std::string, int64_t> &cfg, const std::
 int64_t kf_noise_em_full_stats(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts,
                                const TensorMap &tensors) {
     return run_backward(optistate_kf_noise_em_full_storage_bytes, optistate_kf_noise_em_full_stats, cfg, consts, tensors);
+}
+
+int64_t kf_adjoint(const std::map<std::string, int64_t> &cfg, const std::map<std::string, double> &consts, const TensorMap &tensors) {
+    return run_backward(optistate_kf_adjoint_storage_bytes, optistate_kf_adjoint, cfg, consts, tensors);
 }
 
 int kf_resolve_algo(const std::map<std::string, int64_t> &cfg) {
@@ -632,6 +641,7 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
     m.def("kf_smooth_full", &kf_smooth_full);
     m.def("kf_noise_em_stats", &kf_noise_em_stats);
     m.def("kf_noise_em_full_stats", &kf_noise_em_full_stats);
+    m.def("kf_adjoint", &kf_adjoint);
     m.def("kf_measure", &kf_measure);
     m.def("kf_class_step", &kf_class_step);
     m.def("kf_resolve_algo", &kf_resolve_algo);
